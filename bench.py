@@ -9,6 +9,7 @@ features with prefix masks, random-init weights with the ReZero gates drawn from
 their 0 init every attention/FFN gradient is exactly zero).
 
     python bench.py --gpus N --steps K --warmup W            # ours
+    python bench.py ... --dump-outputs DIR                   # + what the last timed step computed
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
     torchrun --nproc-per-node N bench.py --gpus N ...        # data parallel, weak scaling
 
@@ -38,6 +39,9 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the benchmark leaves the tree as it found it (which may be read-only): the project modules it
+# imports are compiled in memory, no __pycache__ is written next to them
+sys.dont_write_bytecode = True
 
 import torch  # noqa: E402
 
@@ -52,6 +56,27 @@ def peaks():
         return dict(hbm=d["hbm_gbs"], tf_burst=d["bf16_tflops"], tf_sust=d["bf16_tflops_sustained"],
                     src="measured (MEASURED_PEAKS.json)")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sust=1400.0, src="fallback (B200_PROFILING.md)")
+
+
+# per array: the headline step's gradients (12.6 M values, none above 2^20) are written whole and
+# its 64 x 128 x 512 output is sampled, 52 MiB in all
+DUMP_MAX_ELEMS = 1 << 20
+
+
+def dump_outputs(out_dir: str, arrays) -> None:
+    """Write every (name, tensor) of `arrays` as out_dir/<name>.npy in float32.  A tensor of more
+    than DUMP_MAX_ELEMS elements is written as the same seeded sample of its flattened elements on
+    every run (ascending flat indices), so that the files of two builds compare element for
+    element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays:
+        a = t.detach().float().cpu()
+        if a.numel() > DUMP_MAX_ELEMS:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randperm(a.numel(), generator=g)[:DUMP_MAX_ELEMS].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -757,7 +782,14 @@ def main():
     ap.add_argument("--configs", default="all",
                     help="comma list of the extra BASELINE configs to measure "
                          "(cfg1a,cfg1b,cfg3,cfg3c,cfg4,cfg5), 'all' or 'none'")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (encoder output "
+                         "'out', 'loss', 'grad.<parameter>') to DIR/<name>.npy as float32; arrays "
+                         f"above {DUMP_MAX_ELEMS} elements as a fixed seeded sample of that many "
+                         "(rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -819,6 +851,8 @@ def main():
             symm_sm_reserve=int(os.environ.get("MMEMO_SYMM_SM_RESERVE", "16")),
             reserve_launches=int(os.environ.get("MMEMO_RESERVE_LAUNCHES", "5")))
 
+    last_out = {}
+
     def step():
         model.zero_grad(set_to_none=True)
         out = model(x_dev, m_dev)
@@ -828,6 +862,8 @@ def main():
         else:
             loss.backward()
         loss_dev.copy_(loss.detach())
+        if args.dump_outputs:
+            last_out["out"] = out              # inside the graph: the buffer every replay rewrites
 
     # ---- warm-up (eager) then CUDA-graph capture of the whole step ------------------------------
     side = torch.cuda.Stream()
@@ -881,6 +917,11 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs,
+                     [("out", last_out["out"]), ("loss", loss_dev)] +
+                     [("grad." + n, p.grad) for n, p in model.named_parameters()
+                      if p.grad is not None])
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1068,7 +1109,6 @@ def main():
         dist.all_reduce(t_, op=dist.ReduceOp.MAX)
         return float(t_.item())
 
-    Kc = min(K, 20)
     base = not args.no_cpu_baseline
     for key in want:
         try:
@@ -1078,7 +1118,7 @@ def main():
                 if world > 1:
                     mk = lambda m: mdp.GradReducer(m, world, bucket_bytes=4 << 20)   # noqa: E731
                 configs.append(measure_train_config(
-                    "cfg4", 256, dev, rank, world, Kc, W, barrier, allreduce_max, pk,
+                    "cfg4", 256, dev, rank, world, K, W, barrier, allreduce_max, pk,
                     reducer_factory=mk, shard=(rank, world), baselines=base, scaling="strong"))
             elif world > 1:
                 continue        # single-GPU legs: reported by the N=1 run only
@@ -1086,7 +1126,7 @@ def main():
                 configs.append(measure_robot_ensemble(dev, baselines=base))
             else:
                 bsz = {"cfg1a": 32, "cfg1b": 32, "cfg3": 128, "cfg3c": 64}[key]
-                configs.append(measure_train_config(key, bsz, dev, rank, world, Kc, W, barrier,
+                configs.append(measure_train_config(key, bsz, dev, rank, world, K, W, barrier,
                                                     allreduce_max, pk, baselines=base))
         except Exception as ex:   # a failed leg must not take the headline line down with it
             import traceback
