@@ -166,7 +166,8 @@ int mmemo_resattn_bwd_bf16(const void* d_o, int64_t lddo, const void* q, int64_t
 /* 1 if the tcgen05/TMA attention kernels serve this shape in the _bf16 build */
 int mmemo_resattn_uses_tensor_cores(int64_t Lq, int64_t Lk, int64_t hd, int64_t ld);
 
-/* Grouped residual attention (bf16): n <= 40 independent problems in ONE launch - the nine chains
+/* Grouped residual attention (bf16): n >= 1 independent problems, one launch per 40 (heaviest
+ * problems first within each launch; every problem is checked before the first launch) - the nine chains
  * of a fusion-trunk layer (others/realformer.py:232-257, cmu-mosei/run.py:278-313,
  * Ren-MME/run.py:230-265, robot_demo.py:399-434), both towers of Concat_Trans / Base_model
  * (cmu-mosei/run.py:330-331, Ren-MME/run.py:283-284), the members of an ensemble
@@ -237,7 +238,7 @@ int mmemo_add_ln_bwd_bf16(const void* dy, int64_t lddy, const void* res, int64_t
                           float* dgamma, float* dbeta, float* dxsum, int64_t M, int64_t d,
                           int relu, mmemo_stream_t stream);
 
-/* Grouped variants (n <= 40 problems, ONE launch; HOST arrays of length n; rows contiguous, i.e.
+/* Grouped variants (n >= 1 problems, one launch per 40; HOST arrays of length n; rows contiguous, i.e.
  * every leading dimension = d): the LayerNorms of the nine chains of a fusion-trunk layer.  The
  * backward serves d <= 512 (its single-pass kernel), no ReLU.  MMEMO_ERR_SHAPE when a problem does
  * not meet the vector kernels' alignment (16-byte pointers, d % 8 == 0 (bf16) / d % 4 == 0). */
@@ -272,14 +273,14 @@ int mmemo_rowsum_f32(const void* x, int64_t ldx, float* out, int64_t M, int64_t 
                      mmemo_stream_t stream);
 int mmemo_rowsum_bf16(const void* x, int64_t ldx, float* out, int64_t M, int64_t N, int64_t period,
                       mmemo_stream_t stream);
-/* out[i][c] += sum_m x[i][m, c] for n <= 40 contiguous (M[i], N) bf16 matrices in one launch (the
- * FFN-1 bias gradients of a trunk layer); N % 8 == 0 */
+/* out[i][c] += sum_m x[i][m, c] for n >= 1 contiguous (M[i], N) bf16 matrices, one launch per 40
+ * (the FFN-1 bias gradients of a trunk layer); N % 8 == 0 */
 int mmemo_colsum_grouped_bf16(int n, const void* const* x, float* const* out, const int64_t* M,
                               int64_t N, mmemo_stream_t stream);
 /* dtype conversion of n contiguous elements (bf16 shadow copies of float32 master weights) */
 int mmemo_cast_f32_to_bf16(const float* src, void* dst, int64_t n, mmemo_stream_t stream);
 int mmemo_cast_bf16_to_f32(const void* src, float* dst, int64_t n, mmemo_stream_t stream);
-/* `count` <= 64 tensors in one launch (host arrays): all bf16 weight shadows of a block / of a
+/* `count` tensors, one launch per 64 (host arrays): all bf16 weight shadows of a block / of a
  * whole trunk layer */
 int mmemo_cast_f32_to_bf16_multi(int count, const float* const* src, void* const* dst,
                                  const int64_t* n, mmemo_stream_t stream);
@@ -292,8 +293,8 @@ int mmemo_sqmean_bwd_f32(const void* x, const float* dloss, int64_t n, void* dx,
                          mmemo_stream_t stream);
 int mmemo_sqmean_bwd_bf16(const void* x, const float* dloss, int64_t n, void* dx,
                           mmemo_stream_t stream);
-/* out[i] = sum of n_in[i] (<= 8) equally sized contiguous tensors, for n_out <= 16 outputs in one
- * launch (`in` = the inputs of all outputs, concatenated; out[i] may alias its first input): the
+/* out[i] = sum of n_in[i] (<= 8) equally sized contiguous tensors, for n_out outputs, one launch
+ * per 16 (`in` = the inputs of all outputs, concatenated; out[i] may alias its first input): the
  * gradients reaching one modality stream from the chains that read it (others/realformer.py:232-257),
  * which autograd would add pairwise.  16-byte aligned pointers. */
 int mmemo_sum_grouped_f32(int n_out, void* const* out, const int* n_in, const void* const* in,
@@ -313,7 +314,7 @@ int mmemo_dropout_f32(const void* x, void* y, int64_t n, float p, uint64_t seed,
                       mmemo_stream_t stream);
 int mmemo_dropout_bf16(const void* x, void* y, int64_t n, float p, uint64_t seed,
                        mmemo_stream_t stream);
-/* The same for n <= 64 tensors in ONE launch (the dropout sites of a fusion-trunk layer over all
+/* The same for n >= 1 tensors, one launch per 64 (the dropout sites of a fusion-trunk layer over all
  * of its chains: Ren-MME/run.py:208,212  robot_demo.py:333,368).  x[i] == y[i] is allowed (in
  * place); 16-byte aligned pointers.  x, y, numel, seeds: HOST arrays of length n.  step: nullable
  * DEVICE scalar mixed into every seed when the kernel runs, so that a captured CUDA graph draws
@@ -414,6 +415,21 @@ int mmemo_adam_step_f32(int count, float* const* params, const float* const* gra
                         float lr, float beta1, float beta2, float eps, float weight_decay,
                         int decoupled, int64_t step, const float* sqnorm, float max_norm,
                         mmemo_stream_t stream);
+/* Several optimizers at once (the k folds of a cross-validation, one model each), one launch per
+ * 96 tensors whatever the number of optimizers:
+ *   grad_sqnorm_multi : sqnorm_out[slot[i]] += |g_i|^2 (float32 device array, zero-initialised by
+ *                       the caller): one squared norm per optimizer
+ *   adam_step_multi   : adam_step with per-tensor lr[i], step[i] (1-based), weight_decay[i] and
+ *                       clip coefficient from sqnorm[slot[i]] (sqnorm nullable: no clipping);
+ *                       betas, eps, decoupled and max_norm are shared by the call.
+ * All arrays are HOST arrays of length count. */
+int mmemo_grad_sqnorm_multi_f32(int count, const float* const* grads, const int64_t* numel,
+                                const int* slot, float* sqnorm_out, mmemo_stream_t stream);
+int mmemo_adam_step_multi_f32(int count, float* const* params, const float* const* grads,
+                              float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
+                              const float* lr, const int64_t* step, const float* weight_decay,
+                              const int* slot, float beta1, float beta2, float eps, int decoupled,
+                              const float* sqnorm, float max_norm, mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Device-side batch assembly: ragged float32 sequences (rows of D features, concatenated in

@@ -95,6 +95,8 @@ SIGNATURES = {
     "mmemo_clip_grads_f32": [_i32, _vp, _vp, _vp, _f32, _vp],
     "mmemo_adam_step_f32": [_i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _f32, _i32, _i64,
                             _vp, _f32, _vp],
+    "mmemo_grad_sqnorm_multi_f32": [_i32, _vp, _vp, _vp, _vp, _vp],
+    "mmemo_adam_step_multi_f32": [_i32] + [_vp] * 9 + [_f32, _f32, _f32, _i32, _vp, _f32, _vp],
     "mmemo_assemble_batch_f32": [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _i32, _f32, _vp],
     "mmemo_assemble_stats_batch_f32": [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _i32, _f32,
                                        _vp],

@@ -172,7 +172,8 @@ ln_fwd_vec(const T* __restrict__ res, int64_t ldres, const T* __restrict__ x, in
 
 // Grouped launches: up to LN_MAXP independent problems (the nine chains of a fusion-trunk layer,
 // both towers, ...) share one grid; blockIdx.y selects the problem, the CTAs of a column of the
-// grid stride over its rows.  Rows are contiguous (leading dimension d).
+// grid stride over its rows.  Rows are contiguous (leading dimension d).  A call with more
+// problems checks all of them, then launches consecutive chunks of LN_MAXP.
 constexpr int LN_MAXP = 40;
 struct LnProb {
   const void *res, *x, *dy;
@@ -772,11 +773,12 @@ unsigned ln_share_ctas(LnTable& tb, int n, const int64_t* M, int64_t rows_per_ct
   return (unsigned)at;
 }
 
+// launch == false: check the problems only (every chunk is checked before the first launch)
 template <typename T>
-int fwd_grouped(int n, const void* const* res, const void* const* x, const float* const* gate,
-                const float* const* gamma, const float* const* beta, void* const* y,
-                float* const* mean, float* const* rstd, const int64_t* M, int64_t d, float eps,
-                int relu, cudaStream_t st) {
+int fwd_grouped_chunk(int n, const void* const* res, const void* const* x, const float* const* gate,
+                      const float* const* gamma, const float* const* beta, void* const* y,
+                      float* const* mean, float* const* rstd, const int64_t* M, int64_t d,
+                      float eps, int relu, bool launch, cudaStream_t st) {
   if (n < 1 || n > LN_MAXP) return MMEMO_ERR_ARG;
   constexpr int V = Vec<T>::N;
   if (d <= 0 || d % V || d / V > 256) return MMEMO_ERR_SHAPE;
@@ -794,7 +796,7 @@ int fwd_grouped(int n, const void* const* res, const void* const* x, const float
     a.mean = mean ? mean[i] : nullptr; a.rstd = rstd ? rstd[i] : nullptr; a.M = M[i];
     mmax = M[i] > mmax ? M[i] : mmax;
   }
-  if (mmax == 0) return MMEMO_OK;
+  if (!launch || mmax == 0) return MMEMO_OK;
   // narrow rows share a warp (LPR lanes per row)
   const int nchunk = (int)(d / V);
   const int rpw = nchunk <= 8 ? 4 : (nchunk <= 16 ? 2 : 1);
@@ -821,11 +823,12 @@ int fwd_grouped(int n, const void* const* res, const void* const* x, const float
 }
 
 template <typename T>
-int bwd_grouped(int n, const void* const* dy, const void* const* res, const void* const* x,
-                const float* const* gate, const float* const* gamma, const float* const* mean,
-                const float* const* rstd, void* const* dres, void* const* dx, float* const* dgate,
-                float* const* dgamma, float* const* dbeta, float* const* dxsum, const int64_t* M,
-                int64_t d, cudaStream_t st) {
+int bwd_grouped_chunk(int n, const void* const* dy, const void* const* res, const void* const* x,
+                      const float* const* gate, const float* const* gamma, const float* const* mean,
+                      const float* const* rstd, void* const* dres, void* const* dx,
+                      float* const* dgate, float* const* dgamma, float* const* dbeta,
+                      float* const* dxsum, const int64_t* M, int64_t d, bool launch,
+                      cudaStream_t st) {
   if (n < 1 || n > LN_MAXP) return MMEMO_ERR_ARG;
   constexpr int V = Vec<T>::N;
   if (d <= 0 || d % V || cdiv(d / V, 32) * V > 16) return MMEMO_ERR_SHAPE;   // single-pass kernel only
@@ -847,7 +850,7 @@ int bwd_grouped(int n, const void* const* dy, const void* const* res, const void
     any_dxsum = any_dxsum || a.dxsum;
     mmax = M[i] > mmax ? M[i] : mmax;
   }
-  if (mmax == 0) return MMEMO_OK;
+  if (!launch || mmax == 0) return MMEMO_OK;
   // one persistent 16-warp CTA per SM over the whole group (at least one per problem); narrow rows
   // share a warp (LPR lanes per row)
   const int nchunk = (int)(d / V);
@@ -869,6 +872,44 @@ int bwd_grouped(int n, const void* const* dy, const void* const* res, const void
   if (rpw == 4) MM_G(1, 8); else if (rpw == 2) MM_G(1, 16);
   else if (nch <= 1) MM_G(1, 32); else if (nch <= 2) MM_G(2, 32); else if (V == 4) MM_G(4, 32);
 #undef MM_G
+  return MMEMO_OK;
+}
+
+// an offset into a nullable per-problem host array
+template <typename P>
+P* at(P* a, int i) { return a ? a + i : nullptr; }
+
+template <typename T>
+int fwd_grouped(int n, const void* const* res, const void* const* x, const float* const* gate,
+                const float* const* gamma, const float* const* beta, void* const* y,
+                float* const* mean, float* const* rstd, const int64_t* M, int64_t d, float eps,
+                int relu, cudaStream_t st) {
+  if (n < 1) return MMEMO_ERR_ARG;
+  for (int pass = 0; pass < 2; ++pass)
+    for (int c = 0; c < n; c += LN_MAXP) {
+      const int rc = fwd_grouped_chunk<T>(n - c < LN_MAXP ? n - c : LN_MAXP, at(res, c), x + c,
+                                          at(gate, c), gamma + c, beta + c, y + c, at(mean, c),
+                                          at(rstd, c), M + c, d, eps, relu, pass == 1, st);
+      if (rc) return rc;
+    }
+  return MMEMO_OK;
+}
+
+template <typename T>
+int bwd_grouped(int n, const void* const* dy, const void* const* res, const void* const* x,
+                const float* const* gate, const float* const* gamma, const float* const* mean,
+                const float* const* rstd, void* const* dres, void* const* dx, float* const* dgate,
+                float* const* dgamma, float* const* dbeta, float* const* dxsum, const int64_t* M,
+                int64_t d, cudaStream_t st) {
+  if (n < 1) return MMEMO_ERR_ARG;
+  for (int pass = 0; pass < 2; ++pass)
+    for (int c = 0; c < n; c += LN_MAXP) {
+      const int rc = bwd_grouped_chunk<T>(n - c < LN_MAXP ? n - c : LN_MAXP, dy + c, at(res, c),
+                                          x + c, at(gate, c), gamma + c, mean + c, rstd + c,
+                                          at(dres, c), dx + c, at(dgate, c), at(dgamma, c),
+                                          at(dbeta, c), at(dxsum, c), M + c, d, pass == 1, st);
+      if (rc) return rc;
+    }
   return MMEMO_OK;
 }
 

@@ -15,6 +15,7 @@ constexpr int OPT_MAXT = 96;
 struct NormTable {
   const float* g[OPT_MAXT];
   long long n[OPT_MAXT];
+  int slot[OPT_MAXT];       // output slot of each tensor (one per fold / member; 0 for one model)
   int count;
 };
 
@@ -64,7 +65,7 @@ __global__ void __launch_bounds__(256) sqnorm_multi_kernel(NormTable t, float* _
   if (threadIdx.x < 32) {
     float s = threadIdx.x < 8 ? red[threadIdx.x] : 0.f;
     s = warp_sum(s);
-    if (threadIdx.x == 0 && s != 0.f) atomicAdd(out, s);
+    if (threadIdx.x == 0 && s != 0.f) atomicAdd(out + t.slot[which], s);
   }
 }
 
@@ -99,15 +100,14 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
   p -= h.step_size * (m / denom);
 }
 
-__global__ void __launch_bounds__(256)
-adam_multi_kernel(AdamTable t, AdamHyper h, const float* __restrict__ sqnorm) {
-  const int which = blockIdx.y;
+// tensor `which` of the table: grid-stride over its elements
+__device__ __forceinline__ void adam_tensor(const AdamTable& t, int which, const AdamHyper& h,
+                                            float coef) {
   float* __restrict__ p = t.p[which];
   const float* __restrict__ g = t.g[which];
   float* __restrict__ m = t.m[which];
   float* __restrict__ v = t.v[which];
   const long long n = t.n[which];
-  const float coef = clip_coef(sqnorm, h.max_norm);
   const bool vec = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) |
                      reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) == 0;
   if (vec) {
@@ -137,6 +137,29 @@ adam_multi_kernel(AdamTable t, AdamHyper h, const float* __restrict__ sqnorm) {
   }
 }
 
+__global__ void __launch_bounds__(256)
+adam_multi_kernel(AdamTable t, AdamHyper h, const float* __restrict__ sqnorm) {
+  adam_tensor(t, blockIdx.y, h, clip_coef(sqnorm, h.max_norm));
+}
+
+// Several optimizers (the k folds of a cross-validation) in one launch: each tensor carries its own
+// lr, weight decay, bias corrections (its own step count) and the norm slot of its optimizer.
+struct MemberHyper {
+  float lr[OPT_MAXT], weight_decay[OPT_MAXT], step_size[OPT_MAXT], inv_bc2_sqrt[OPT_MAXT];
+  int slot[OPT_MAXT];
+};
+
+__global__ void __launch_bounds__(256)
+adam_member_kernel(const __grid_constant__ AdamTable t, const __grid_constant__ MemberHyper mh,
+                   AdamHyper h, const float* __restrict__ sqnorm) {
+  const int which = blockIdx.y;
+  h.lr = mh.lr[which];
+  h.weight_decay = mh.weight_decay[which];
+  h.step_size = mh.step_size[which];
+  h.inv_bc2_sqrt = mh.inv_bc2_sqrt[which];
+  adam_tensor(t, which, h, clip_coef(sqnorm ? sqnorm + mh.slot[which] : nullptr, h.max_norm));
+}
+
 unsigned grid_x(long long nmax) {
   long long bx = cdiv(cdiv(nmax, 4), 256);
   if (bx > 148 * 2) bx = 148 * 2;
@@ -160,6 +183,27 @@ int mmemo_grad_sqnorm_f32(int count, const float* const* grads, const int64_t* n
       MM_REQUIRE(grads[base + i] && numel[base + i] >= 0);
       t.g[i] = grads[base + i];
       t.n[i] = numel[base + i];
+      nmax = t.n[i] > nmax ? t.n[i] : nmax;
+    }
+    sqnorm_multi_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, sqnorm_out);
+    MM_LAUNCH_OK();
+  }
+  return MMEMO_OK;
+}
+
+int mmemo_grad_sqnorm_multi_f32(int count, const float* const* grads, const int64_t* numel,
+                                const int* slot, float* sqnorm_out, mmemo_stream_t s) {
+  MM_REQUIRE(count >= 0 && sqnorm_out && (count == 0 || (grads && numel && slot)));
+  cudaStream_t st = mm_stream(s);
+  for (int i = 0; i < count; ++i) MM_REQUIRE(grads[i] && numel[i] >= 0 && slot[i] >= 0);
+  for (int base = 0; base < count; base += OPT_MAXT) {
+    NormTable t = {};
+    long long nmax = 0;
+    t.count = count - base < OPT_MAXT ? count - base : OPT_MAXT;
+    for (int i = 0; i < t.count; ++i) {
+      t.g[i] = grads[base + i];
+      t.n[i] = numel[base + i];
+      t.slot[i] = slot[base + i];
       nmax = t.n[i] > nmax ? t.n[i] : nmax;
     }
     sqnorm_multi_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, sqnorm_out);
@@ -220,6 +264,51 @@ int mmemo_adam_step_f32(int count, float* const* params, const float* const* gra
       nmax = t.n[i] > nmax ? t.n[i] : nmax;
     }
     adam_multi_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, h, sqnorm);
+    MM_LAUNCH_OK();
+  }
+  return MMEMO_OK;
+}
+
+int mmemo_adam_step_multi_f32(int count, float* const* params, const float* const* grads,
+                              float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
+                              const float* lr, const int64_t* step, const float* weight_decay,
+                              const int* slot, float beta1, float beta2, float eps, int decoupled,
+                              const float* sqnorm, float max_norm, mmemo_stream_t s) {
+  MM_REQUIRE(count >= 0 && (count == 0 || (params && grads && exp_avg && exp_avg_sq && numel && lr &&
+                                           step && weight_decay && slot)));
+  MM_REQUIRE(!sqnorm || max_norm > 0.f);
+  for (int j = 0; j < count; ++j)
+    MM_REQUIRE(params[j] && grads[j] && exp_avg[j] && exp_avg_sq[j] && numel[j] >= 0 &&
+               step[j] >= 1 && slot[j] >= 0);
+  cudaStream_t st = mm_stream(s);
+  AdamHyper h = {};
+  h.beta1 = beta1; h.beta2 = beta2; h.eps = eps;
+  h.max_norm = max_norm;
+  h.decoupled = decoupled;
+  for (int base = 0; base < count; base += OPT_MAXT) {
+    static thread_local AdamTable t;
+    static thread_local MemberHyper mh;
+    t = AdamTable{};
+    long long nmax = 0;
+    t.count = count - base < OPT_MAXT ? count - base : OPT_MAXT;
+    for (int i = 0; i < t.count; ++i) {
+      const int j = base + i;
+      t.p[i] = params[j];
+      t.g[i] = const_cast<float*>(grads[j]);
+      t.m[i] = exp_avg[j];
+      t.v[i] = exp_avg_sq[j];
+      t.n[i] = numel[j];
+      nmax = t.n[i] > nmax ? t.n[i] : nmax;
+      // the same double-precision bias corrections as mmemo_adam_step_f32
+      const double bc1 = 1.0 - pow((double)beta1, (double)step[j]);
+      const double bc2 = 1.0 - pow((double)beta2, (double)step[j]);
+      mh.lr[i] = lr[j];
+      mh.weight_decay[i] = weight_decay[j];
+      mh.step_size[i] = (float)((double)lr[j] / bc1);
+      mh.inv_bc2_sqrt[i] = (float)(1.0 / sqrt(bc2));
+      mh.slot[i] = slot[j];
+    }
+    adam_member_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, mh, h, sqnorm);
     MM_LAUNCH_OK();
   }
   return MMEMO_OK;

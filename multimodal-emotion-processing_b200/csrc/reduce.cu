@@ -337,10 +337,10 @@ __global__ void __launch_bounds__(256) sum_grouped_kernel(const __grid_constant_
   }
 }
 
+// launch == false: check the arguments only (every chunk is checked before the first launch)
 template <typename T>
-int sum_grouped(int n_out, void* const* out, const int* n_in, const void* const* in,
-                const int64_t* numel, cudaStream_t st) {
-  if (n_out <= 0) return MMEMO_OK;
+int sum_grouped_chunk(int n_out, void* const* out, const int* n_in, const void* const* in,
+                      const int64_t* numel, bool launch, cudaStream_t st) {
   if (n_out > SG_MAXO) return MMEMO_ERR_ARG;
   static thread_local SumTable t;
   long long most = 0;
@@ -355,12 +355,28 @@ int sum_grouped(int n_out, void* const* out, const int* n_in, const void* const*
     }
     most = numel[i] > most ? numel[i] : most;
   }
-  if (most == 0) return MMEMO_OK;
+  if (!launch || most == 0) return MMEMO_OK;
   long long bx = cdiv(most, 256 * (16 / (long long)sizeof(T)));
   const long long cap = cdiv(148 * 8, n_out);
   if (bx > cap) bx = cap;
   MM_CUDA_OK(mm_launch(sum_grouped_kernel<T>, dim3((unsigned)bx, (unsigned)n_out), dim3(256), 0, st,
                        t));
+  return MMEMO_OK;
+}
+
+template <typename T>
+int sum_grouped(int n_out, void* const* out, const int* n_in, const void* const* in,
+                const int64_t* numel, cudaStream_t st) {
+  if (n_out <= 0) return MMEMO_OK;
+  for (int pass = 0; pass < 2; ++pass) {
+    int pos = 0;                 // first input of the chunk in the concatenated `in`
+    for (int c = 0; c < n_out; c += SG_MAXO) {
+      const int m = n_out - c < SG_MAXO ? n_out - c : SG_MAXO;
+      const int rc = sum_grouped_chunk<T>(m, out + c, n_in + c, in + pos, numel + c, pass == 1, st);
+      if (rc) return rc;
+      for (int i = c; i < c + m; ++i) pos += n_in[i];
+    }
+  }
   return MMEMO_OK;
 }
 
@@ -452,8 +468,9 @@ int rowsum(const void* x, int64_t ldx, float* out, int64_t M, int64_t N, int64_t
 }
 
 template <typename T>
-int dropout_multi(int n, const void* const* x, void* const* y, const int64_t* numel,
-                  const uint64_t* seeds, float p, const uint64_t* step, cudaStream_t st) {
+int dropout_multi_chunk(int n, const void* const* x, void* const* y, const int64_t* numel,
+                        const uint64_t* seeds, float p, const uint64_t* step, bool launch,
+                        cudaStream_t st) {
   if (n < 1 || n > DROP_MAXT) return MMEMO_ERR_ARG;
   MM_REQUIRE(x && y && numel && seeds && p >= 0.f && p < 1.f);
   DropTable t = {};
@@ -466,13 +483,79 @@ int dropout_multi(int n, const void* const* x, void* const* y, const int64_t* nu
     nmax = numel[i] > nmax ? numel[i] : nmax;
   }
   t.count = n;
-  if (nmax == 0) return MMEMO_OK;
+  if (!launch || nmax == 0) return MMEMO_OK;
   const long long per_block = 256 * (16 / sizeof(T)) * 4;      // four 16-byte accesses per thread
   long long gx = cdiv(nmax, per_block);
   gx = gx > 1184 ? 1184 : gx;                                  // 8 CTAs per SM at most
   MM_CUDA_OK(mm_launch(dropout_multi_kernel<T>, dim3((unsigned)gx, (unsigned)n), dim3(256), 0, st, t,
                        p, 1.0f / (1.0f - p),
                        reinterpret_cast<const unsigned long long*>(step)));
+  return MMEMO_OK;
+}
+
+template <typename T>
+int dropout_multi(int n, const void* const* x, void* const* y, const int64_t* numel,
+                  const uint64_t* seeds, float p, const uint64_t* step, cudaStream_t st) {
+  if (n < 1) return MMEMO_ERR_ARG;
+  MM_REQUIRE(x && y && numel && seeds);
+  for (int pass = 0; pass < 2; ++pass)
+    for (int c = 0; c < n; c += DROP_MAXT) {
+      const int rc = dropout_multi_chunk<T>(n - c < DROP_MAXT ? n - c : DROP_MAXT, x + c, y + c,
+                                            numel + c, seeds + c, p, step, pass == 1, st);
+      if (rc) return rc;
+    }
+  return MMEMO_OK;
+}
+
+int cast_multi_chunk(int count, const float* const* src, void* const* dst, const int64_t* n,
+                     bool launch, cudaStream_t st) {
+  if (count > CAST_MAXT) return MMEMO_ERR_ARG;
+  static thread_local CastTable t;
+  t = CastTable{};
+  t.count = count;
+  int64_t nmax = 0;
+  for (int i = 0; i < count; ++i) {
+    MM_REQUIRE(src[i] && dst[i] && n[i] >= 0);
+    // 16-byte aligned sources / 8-byte aligned destinations (vector accesses)
+    MM_REQUIRE((reinterpret_cast<uintptr_t>(src[i]) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(dst[i]) & 7) == 0);
+    t.src[i] = src[i];
+    t.dst[i] = static_cast<bf16*>(dst[i]);
+    t.n[i] = n[i];
+    nmax = n[i] > nmax ? n[i] : nmax;
+  }
+  if (!launch) return MMEMO_OK;
+  int64_t bx = cdiv(cdiv(nmax, 4), 256);
+  if (bx > 148) bx = 148;
+  if (bx < 1) bx = 1;
+  MM_CUDA_OK(mm_launch(cast_multi_kernel, dim3((unsigned)bx, (unsigned)count), dim3(256), 0, st, t));
+  return MMEMO_OK;
+}
+
+int colsum_grouped_chunk(int n, const void* const* x, float* const* out, const int64_t* M,
+                         int64_t N, bool launch, cudaStream_t st) {
+  if (n < 1 || n > CS_MAXP) return MMEMO_ERR_ARG;
+  if (N <= 0 || N % 8) return MMEMO_ERR_SHAPE;
+  static thread_local ColsumTable tb;
+  int64_t mmax = 0;
+  for (int i = 0; i < n; ++i) {
+    MM_REQUIRE(x[i] && out[i] && M[i] >= 0);
+    if (reinterpret_cast<uintptr_t>(x[i]) % 16) return MMEMO_ERR_SHAPE;
+    tb.x[i] = static_cast<const bf16*>(x[i]);
+    tb.out[i] = out[i];
+    tb.M[i] = M[i];
+    mmax = M[i] > mmax ? M[i] : mmax;
+  }
+  if (!launch || mmax == 0) return MMEMO_OK;
+  const int64_t groups = cdiv(N, 256);
+  // ~6 CTAs of 8 warps per SM over the whole group: with 2 the launch was latency-bound (the
+  // nine chains of a trunk layer, N = 192: 36 rows per warp in turn; cfg 1a step 1.335 -> 1.322 ms)
+  int64_t strips = cdiv(148 * 6, groups * n);
+  if (strips > cdiv(mmax, 32)) strips = cdiv(mmax, 32);
+  if (strips < 1) strips = 1;
+  MM_CUDA_OK(mm_launch(colsum_bf16_vec_grouped_kernel,
+                       dim3((unsigned)groups, (unsigned)strips, (unsigned)n), dim3(256), 0, st, tb,
+                       N));
   return MMEMO_OK;
 }
 
@@ -508,26 +591,12 @@ int mmemo_cast_f32_to_bf16(const float* src, void* dst, int64_t n, mmemo_stream_
 int mmemo_cast_f32_to_bf16_multi(int count, const float* const* src, void* const* dst,
                                  const int64_t* n, mmemo_stream_t s) {
   if (count <= 0) return MMEMO_OK;
-  if (count > CAST_MAXT) return MMEMO_ERR_ARG;
-  static thread_local CastTable t;
-  t = CastTable{};
-  t.count = count;
-  int64_t nmax = 0;
-  for (int i = 0; i < count; ++i) {
-    MM_REQUIRE(src[i] && dst[i] && n[i] >= 0);
-    // 16-byte aligned sources / 8-byte aligned destinations (vector accesses)
-    MM_REQUIRE((reinterpret_cast<uintptr_t>(src[i]) & 15) == 0 &&
-               (reinterpret_cast<uintptr_t>(dst[i]) & 7) == 0);
-    t.src[i] = src[i];
-    t.dst[i] = static_cast<bf16*>(dst[i]);
-    t.n[i] = n[i];
-    nmax = n[i] > nmax ? n[i] : nmax;
-  }
-  int64_t bx = cdiv(cdiv(nmax, 4), 256);
-  if (bx > 148) bx = 148;
-  if (bx < 1) bx = 1;
-  MM_CUDA_OK(mm_launch(cast_multi_kernel, dim3((unsigned)bx, (unsigned)count), dim3(256), 0,
-                       mm_stream(s), t));
+  for (int pass = 0; pass < 2; ++pass)          // check every chunk, then launch them
+    for (int c = 0; c < count; c += CAST_MAXT) {
+      const int rc = cast_multi_chunk(count - c < CAST_MAXT ? count - c : CAST_MAXT, src + c,
+                                      dst + c, n + c, pass == 1, mm_stream(s));
+      if (rc) return rc;
+    }
   return MMEMO_OK;
 }
 /* *out (float32, zero-initialised by the caller) += mean(x^2);  dx = dloss * 2 x / n */
@@ -602,31 +671,16 @@ int mmemo_cast_pad_f32_to_bf16_multi(int count, const float* const* src, const i
                        mm_stream(s), t));
   return MMEMO_OK;
 }
-/* out[i][c] += sum_m x[i][m, c] for n contiguous (M[i], N) bf16 matrices, one launch */
+/* out[i][c] += sum_m x[i][m, c] for n contiguous (M[i], N) bf16 matrices, one launch per CS_MAXP */
 int mmemo_colsum_grouped_bf16(int n, const void* const* x, float* const* out, const int64_t* M,
                               int64_t N, mmemo_stream_t s) {
-  if (n < 1 || n > CS_MAXP) return MMEMO_ERR_ARG;
-  if (N <= 0 || N % 8) return MMEMO_ERR_SHAPE;
-  static thread_local ColsumTable tb;
-  int64_t mmax = 0;
-  for (int i = 0; i < n; ++i) {
-    MM_REQUIRE(x[i] && out[i] && M[i] >= 0);
-    if (reinterpret_cast<uintptr_t>(x[i]) % 16) return MMEMO_ERR_SHAPE;
-    tb.x[i] = static_cast<const bf16*>(x[i]);
-    tb.out[i] = out[i];
-    tb.M[i] = M[i];
-    mmax = M[i] > mmax ? M[i] : mmax;
-  }
-  if (mmax == 0) return MMEMO_OK;
-  const int64_t groups = cdiv(N, 256);
-  // ~6 CTAs of 8 warps per SM over the whole group: with 2 the launch was latency-bound (the
-  // nine chains of a trunk layer, N = 192: 36 rows per warp in turn; cfg 1a step 1.335 -> 1.322 ms)
-  int64_t strips = cdiv(148 * 6, groups * n);
-  if (strips > cdiv(mmax, 32)) strips = cdiv(mmax, 32);
-  if (strips < 1) strips = 1;
-  MM_CUDA_OK(mm_launch(colsum_bf16_vec_grouped_kernel,
-                       dim3((unsigned)groups, (unsigned)strips, (unsigned)n), dim3(256), 0,
-                       mm_stream(s), tb, N));
+  if (n < 1) return MMEMO_ERR_ARG;
+  for (int pass = 0; pass < 2; ++pass)          // check every chunk, then launch them
+    for (int c = 0; c < n; c += CS_MAXP) {
+      const int rc = colsum_grouped_chunk(n - c < CS_MAXP ? n - c : CS_MAXP, x + c, out + c, M + c,
+                                          N, pass == 1, mm_stream(s));
+      if (rc) return rc;
+    }
   return MMEMO_OK;
 }
 int mmemo_cast_bf16_to_f32(const void* src, float* dst, int64_t n, mmemo_stream_t s) {

@@ -8,6 +8,7 @@
 // GROUPED: one launch serves up to MAXP independent problems (the nine chains of a fusion-trunk
 // layer, both towers of Concat_Trans / Base_model, the members of an ensemble) - the problem
 // table travels as a kernel parameter and blockIdx.x is mapped to (problem, batch, head, tile).
+// A call with more problems is split into consecutive chunks of MAXP, one set of launches each.
 //
 // Forward  (replaces others/realformer.py:189-203 and its twins): CTA = (b, h, 64 query rows),
 //   4 warps x 16 rows.  K_h, V_h (and the Q tile) are staged in shared memory by cp.async in an
@@ -34,7 +35,7 @@
 
 namespace {
 
-constexpr int MAXP = 40;          // problems per launch
+constexpr int MAXP = 40;          // problems per launch (a call takes any number: chunks of MAXP)
 // Kernel instantiations by the role of a layer in its chain.  The flags of a problem (previous
 // scores? scores written / stored? score gradients in / out?) are runtime data in M_GEN; the other
 // modes fix them at compile time, which removes the per-chunk pointer tests, the scalar fall-back
@@ -938,7 +939,7 @@ int bwd_mode(const mmemo_attn_problem& p) {
 // tail, instead of a last wave made of the slowest CTAs only.
 void heavy_first(const mmemo_attn_problem* ps, int n, int* idx) {
   for (int i = 0; i < n; ++i) idx[i] = i;
-  for (int i = 1; i < n; ++i) {          // stable insertion sort (n <= 40)
+  for (int i = 1; i < n; ++i) {          // stable insertion sort (n <= MAXP)
     const int v = idx[i];
     const int64_t w = ps[v].Lq * ps[v].Lk;
     int j = i - 1;
@@ -994,14 +995,18 @@ int fwd_launch(const mmemo_attn_problem* ps, int n, int mode, cudaStream_t st) {
 }  // namespace
 
 int resattn_mma_fwd(const mmemo_attn_problem* ps, int n, cudaStream_t st) {
-  if (n < 1 || n > MAXP) return MMEMO_ERR_ARG;
+  if (n < 1) return MMEMO_ERR_ARG;
   const int hd = (int)ps[0].hd;
-  for (int i = 0; i < n; ++i)
+  for (int i = 0; i < n; ++i)         // every problem is checked before the first launch
     if (ps[i].hd != hd || !resattn_mma_supported(ps[i], false)) return MMEMO_ERR_SHAPE;
-  // one launch per instantiation present (the problems of a trunk layer share their flags: one)
-  for (int mode = M_GEN; mode <= M_LAST; ++mode) {
-    const int rc = fwd_launch(ps, n, mode, st);
-    if (rc) return rc;
+  // chunks of MAXP problems; per chunk one launch per instantiation present (the problems of a
+  // trunk layer share their flags: one)
+  for (int c0 = 0; c0 < n; c0 += MAXP) {
+    const int m = n - c0 < MAXP ? n - c0 : MAXP;
+    for (int mode = M_GEN; mode <= M_LAST; ++mode) {
+      const int rc = fwd_launch(ps + c0, m, mode, st);
+      if (rc) return rc;
+    }
   }
   return MMEMO_OK;
 }
@@ -1102,11 +1107,8 @@ int bwd_launch(const mmemo_attn_problem* const* ps, int n, int warps, int mode, 
 }
 }  // namespace
 
-int resattn_mma_bwd(const mmemo_attn_problem* ps, int n, cudaStream_t st) {
-  if (n < 1 || n > MAXP) return MMEMO_ERR_ARG;
-  const int hd = (int)ps[0].hd;
-  for (int i = 0; i < n; ++i)
-    if (ps[i].hd != hd || !resattn_mma_supported(ps[i], true)) return MMEMO_ERR_SHAPE;
+namespace {
+int bwd_chunk(const mmemo_attn_problem* ps, int n, cudaStream_t st) {
   int fixed = 0;
   if (const char* e = getenv("MMEMO_ATTN_WARPS")) fixed = atoi(e);      // experiments
   // one launch per (CTA size, instantiation): all chains of realformer / robot_demo share one;
@@ -1127,6 +1129,19 @@ int resattn_mma_bwd(const mmemo_attn_problem* ps, int n, cudaStream_t st) {
       if (!done[j] && wj == w && bwd_mode(ps[j]) == mode) { sel[m++] = &ps[j]; done[j] = true; }
     }
     const int rc = bwd_launch(sel, m, w, mode, st);
+    if (rc) return rc;
+  }
+  return MMEMO_OK;
+}
+}  // namespace
+
+int resattn_mma_bwd(const mmemo_attn_problem* ps, int n, cudaStream_t st) {
+  if (n < 1) return MMEMO_ERR_ARG;
+  const int hd = (int)ps[0].hd;
+  for (int i = 0; i < n; ++i)         // every problem is checked before the first launch
+    if (ps[i].hd != hd || !resattn_mma_supported(ps[i], true)) return MMEMO_ERR_SHAPE;
+  for (int c0 = 0; c0 < n; c0 += MAXP) {          // chunks of MAXP problems
+    const int rc = bwd_chunk(ps + c0, n - c0 < MAXP ? n - c0 : MAXP, st);
     if (rc) return rc;
   }
   return MMEMO_OK;

@@ -51,8 +51,8 @@ def _opt(t: Tensor) -> Optional[Tensor]:
 
 
 # ------------------------------------------------------------------------------------------------
-# grouped LayerNorm / column sums (one launch per group; per-problem launches when the vector
-# kernels do not take a shape)
+# grouped LayerNorm / column sums (one library call per group, which launches per 40 problems;
+# per-problem launches when the vector kernels do not take a shape)
 # ------------------------------------------------------------------------------------------------
 def _vpa(ts):
     return _arr(C.c_void_p, [_p(t) for t in ts])
@@ -64,7 +64,7 @@ def ln_fwd_group(bf16: bool, res, xs, gates, gammas, betas, relu=False):
     stats = [torch.empty(2, x.numel() // x.shape[-1], dtype=F32, device=x.device) for x in xs]
     d = xs[0].shape[-1]
     ok = False
-    if 1 < len(xs) <= 40 and all(x.is_contiguous() for x in xs) and \
+    if len(xs) > 1 and all(x.is_contiguous() for x in xs) and \
             all(r is None or r.is_contiguous() for r in res):
         ok = ops._try_call(
             f"mmemo_add_ln_fwd_grouped_{'bf16' if bf16 else 'f32'}",
@@ -86,7 +86,7 @@ def ln_bwd_group(bf16: bool, dys, res, xs, gates, gammas, stats, want_dres: bool
     dxs = [torch.empty_like(x) for x in xs]
     dres = [torch.empty_like(x) if want_dres else None for x in xs]
     ok = False
-    if 1 < len(xs) <= 40 and all(t.is_contiguous() for t in list(xs) + list(dys)) and \
+    if len(xs) > 1 and all(t.is_contiguous() for t in list(xs) + list(dys)) and \
             all(r is None or r.is_contiguous() for r in res):
         ok = ops._try_call(
             f"mmemo_add_ln_bwd_grouped_{'bf16' if bf16 else 'f32'}",
@@ -107,7 +107,7 @@ def ln_bwd_group(bf16: bool, dys, res, xs, gates, gammas, stats, want_dres: bool
 def colsum_group(bf16: bool, xs, outs):
     """outs[g] (zero-initialised float32 [N]) += column sums of xs[g] (M_g, N)."""
     N = xs[0].shape[-1]
-    if bf16 and 1 < len(xs) <= 40 and N % 8 == 0 and all(x.is_contiguous() for x in xs):
+    if bf16 and len(xs) > 1 and N % 8 == 0 and all(x.is_contiguous() for x in xs):
         if ops._try_call("mmemo_colsum_grouped_bf16", len(xs), _vpa(xs), _vpa(outs),
                          _arr(C.c_int64, [x.numel() // N for x in xs]), N, _stream()):
             return
@@ -141,9 +141,10 @@ def merge_shared_grads(bf16: bool, inputs, grads):
             todo.append(gs)
         for i in ix[1:]:
             out[i] = None
-    for part in [todo[i:i + 16] for i in range(0, len(todo), 16)]:
-        name = f"mmemo_sum_grouped_{'bf16' if part[0][0].dtype == BF else 'f32'}"
-        _call(name, len(part), _vpa([gs[0] for gs in part]), _arr(C.c_int, [len(gs) for gs in part]),
+    for dt in dict.fromkeys(gs[0].dtype for gs in todo):
+        part = [gs for gs in todo if gs[0].dtype == dt]
+        _call(f"mmemo_sum_grouped_{'bf16' if dt == BF else 'f32'}", len(part),
+              _vpa([gs[0] for gs in part]), _arr(C.c_int, [len(gs) for gs in part]),
               _vpa([g_ for gs in part for g_ in gs]), _arr(C.c_int64, [gs[0].numel() for gs in part]),
               _stream())
     return out

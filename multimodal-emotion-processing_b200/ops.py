@@ -165,14 +165,11 @@ def shadow_bf16(*ws: Tensor) -> Tensor:
 
 def shadow_bf16_block(groups: Sequence[Sequence[Tensor]]) -> List[Tensor]:
     """bf16 shadows of several weight groups (each group = weights concatenated along dim 0) with
-    ONE cast launch; also fills the per-group cache used by ``shadow_bf16``."""
+    ONE cast call (one launch per 64 tensors); also fills the per-group cache used by
+    ``shadow_bf16``."""
     keys = [tuple((w.data_ptr(), w._version, tuple(w.shape)) for w in g) for g in groups]
     if all(k in _shadow for k in keys):
         return [_shadow[k] for k in keys]
-    flat = [w for g in groups for w in g]
-    if len(flat) > 64:
-        half = len(groups) // 2
-        return shadow_bf16_block(groups[:half]) + shadow_bf16_block(groups[half:])
     outs, srcs, dsts, ns = [], [], [], []
     for g, k in zip(groups, keys):
         ptrs = {e[0] for e in k}
@@ -1373,16 +1370,14 @@ def site_seeds(seed: int, G: int, site: int, n_sites: int = 2) -> List[int]:
 
 
 def _dropout_group(xs, ys, p: float, seeds) -> None:
-    """ys[i] = dropout(xs[i]) for up to 64 tensors per launch; xs[i] is ys[i] = in place.  Forward
-    and backward use the same seeds (same masks)."""
+    """ys[i] = dropout(xs[i]) in one call (one launch per 64 tensors); xs[i] is ys[i] = in place.
+    Forward and backward use the same seeds (same masks)."""
     if p <= 0.0 or not xs:
         return
     bf16 = xs[0].dtype == BF
     step = dropout_step(xs[0].device)
-    for i in range(0, len(xs), 64):
-        px, py, ps = xs[i:i + 64], ys[i:i + 64], seeds[i:i + 64]
-        assert all(t.is_contiguous() for t in px) and all(t.is_contiguous() for t in py)
-        _call(f"mmemo_dropout_multi_{_sfx(bf16)}", len(px),
-              _arr(C.c_void_p, [t.data_ptr() for t in px]), _arr(C.c_void_p, [t.data_ptr() for t in py]),
-              _arr(C.c_int64, [t.numel() for t in px]), _arr(C.c_uint64, list(ps)), float(p),
-              step.data_ptr(), _stream())
+    assert all(t.is_contiguous() for t in xs) and all(t.is_contiguous() for t in ys)
+    _call(f"mmemo_dropout_multi_{_sfx(bf16)}", len(xs),
+          _arr(C.c_void_p, [t.data_ptr() for t in xs]), _arr(C.c_void_p, [t.data_ptr() for t in ys]),
+          _arr(C.c_int64, [t.numel() for t in xs]), _arr(C.c_uint64, list(seeds)), float(p),
+          step.data_ptr(), _stream())

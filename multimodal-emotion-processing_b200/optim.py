@@ -28,6 +28,8 @@ from torch import Tensor
 
 from . import ops
 
+_CHUNK = 96      # tensors per launch of the multi-tensor kernels (csrc/optim.cu OPT_MAXT)
+
 
 def _ptrs(ts: List[Tensor]):
     return (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
@@ -84,12 +86,8 @@ class _FusedAdam(torch.optim.Optimizer):
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay,
                                       amsgrad=False))
 
-    @torch.no_grad()
-    def step(self, closure=None):
-        loss = None
-        if closure is not None:
-            with torch.enable_grad():
-                loss = closure()
+    def _collect(self):
+        """[(param_group, params with a gradient, their gradients)], state initialised."""
         groups = []
         for group in self.param_groups:
             ps = [p for p in group["params"] if p.grad is not None]
@@ -105,6 +103,15 @@ class _FusedAdam(torch.optim.Optimizer):
                     st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
                     st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
             groups.append((group, ps, gs))
+        return groups
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        groups = self._collect()
         if not groups:
             return loss
         sq = None
@@ -149,3 +156,62 @@ class AdamW(_FusedAdam):
                  weight_decay: float = 1e-2, amsgrad: bool = False,
                  max_grad_norm: Optional[float] = None):
         super().__init__(params, lr, betas, eps, weight_decay, amsgrad, max_grad_norm)
+
+
+def _arr(ctype, vals):
+    return (ctype * len(vals))(*vals)
+
+
+@torch.no_grad()
+def step_group(optimizers) -> None:
+    """``for opt in optimizers: opt.step()`` for several ``Adam`` / ``AdamW`` instances (the k folds
+    of a cross-validation, one model each) in one launch per 96 tensors, whatever their number.
+
+    Each optimizer keeps its own ``param_groups``, ``state`` and ``state_dict`` and ends up exactly
+    as if it had been stepped alone: its own lr (e.g. set by its own ``ReduceLROnPlateau``), weight
+    decay and step counts, and with ``max_grad_norm`` its gradients clipped by the norm over its own
+    parameters (one squared norm per optimizer, computed first, one launch per 96 tensors).
+    Optimizers that differ in class, ``betas``, ``eps`` or ``max_grad_norm`` are updated by one call
+    per such combination."""
+    opts = list(optimizers)
+    for o in opts:
+        if not isinstance(o, _FusedAdam):
+            raise TypeError(f"step_group takes mmemo_b200.optim.Adam / AdamW, not {type(o).__name__}")
+    collected = [o._collect() for o in opts]
+    sq = None
+    norm_g, norm_slot = [], []
+    for k, (o, groups) in enumerate(zip(opts, collected)):
+        if o.max_grad_norm is not None:
+            for _, _, gs in groups:
+                norm_g += gs
+                norm_slot += [k] * len(gs)
+    if norm_g:
+        sq = torch.zeros(len(opts), dtype=torch.float32, device=norm_g[0].device)
+        for i in range(0, len(norm_g), _CHUNK):
+            gs, sl = norm_g[i:i + _CHUNK], norm_slot[i:i + _CHUNK]
+            ops._call("mmemo_grad_sqnorm_multi_f32", len(gs), _ptrs(gs), _ns(gs), _arr(C.c_int, sl),
+                      sq.data_ptr(), ops._stream())
+    # [(param, grad, optimizer index, param_group)] per combination of the shared hyper-parameters
+    calls = {}
+    for k, (o, groups) in enumerate(zip(opts, collected)):
+        for group, ps, gs in groups:
+            key = (o._decoupled, tuple(group["betas"]), float(group["eps"]), o.max_grad_norm)
+            calls.setdefault(key, []).extend((p, g, k, group) for p, g in zip(ps, gs))
+    for (decoupled, (b1, b2), eps, max_norm), items in calls.items():
+        for i in range(0, len(items), _CHUNK):
+            part = items[i:i + _CHUNK]
+            pp = [it[0] for it in part]
+            st = [opts[it[2]].state[it[0]] for it in part]
+            ops._call("mmemo_adam_step_multi_f32", len(part), _ptrs(pp), _ptrs([it[1] for it in part]),
+                      _ptrs([s["exp_avg"] for s in st]), _ptrs([s["exp_avg_sq"] for s in st]),
+                      _ns(pp), _arr(C.c_float, [float(it[3]["lr"]) for it in part]),
+                      _arr(C.c_int64, [int(s["step"]) + 1 for s in st]),
+                      _arr(C.c_float, [float(it[3]["weight_decay"]) for it in part]),
+                      _arr(C.c_int, [it[2] for it in part]), float(b1), float(b2), eps,
+                      int(decoupled), None if sq is None or max_norm is None else sq.data_ptr(),
+                      float(max_norm or 0.0), ops._stream())
+        for p, _, k, _ in items:
+            opts[k].state[p]["step"] += 1
+        # (see _FusedAdam.step: the launch wrote the parameters through raw pointers)
+        torch._C._increment_version([it[0] for it in items])
+
