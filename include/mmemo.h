@@ -346,6 +346,19 @@ int mmemo_pool_bwd_f32(const float* dout, const int32_t* argmax, void* const* ds
 int mmemo_pool_bwd_bf16(const float* dout, const int32_t* argmax, void* const* dseg_ptrs,
                         const int64_t* group_len, int n_groups, int n_slots, int64_t B, int64_t d,
                         mmemo_stream_t stream);
+/* The same forward for n_towers >= 1 fusion trunks at once (the towers of every member of an
+ * ensemble: others/realformer.py:258-262 and cmu-mosei/run.py:314-318 / Ren-MME/run.py:266-270 once
+ * per tower and member), without argmax (inference).  seg_ptrs: HOST array [n_towers][n_groups *
+ * n_slots]; out: HOST array of n_towers (B, 2*n_slots*d) float32 outputs.  All towers share B, d,
+ * n_groups, n_slots and group_len.  Each out[t] is bitwise equal to mmemo_pool_fwd_* on tower t.
+ * Every tower is checked before the first launch; one launch per 16 towers (fewer when a tower has
+ * more than 16 segments: 256 segment pointers per launch). */
+int mmemo_pool_fwd_multi_f32(int n_towers, const void* const* seg_ptrs, const int64_t* group_len,
+                             int n_groups, int n_slots, int64_t B, int64_t d, float* const* out,
+                             mmemo_stream_t stream);
+int mmemo_pool_fwd_multi_bf16(int n_towers, const void* const* seg_ptrs, const int64_t* group_len,
+                              int n_groups, int n_slots, int64_t B, int64_t d, float* const* out,
+                              mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Heads and losses (float32 only; O(B*C) work).
@@ -377,6 +390,43 @@ int mmemo_rdrop_kl_fwd(const float* logits, float* out, int64_t B, int64_t C,
                        mmemo_stream_t stream);
 int mmemo_rdrop_kl_bwd(const float* dout, const float* logits, float* dlogits, int64_t B, int64_t C,
                        mmemo_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Ensemble head (inference, float32): y = (out_1 + ... + out_K) / K over K >= 1 members, summed as
+ * a left fold in member order without atomics (the same bits on every run).  Replaces, per member,
+ * the classifier linears and head of others/realformer.py:270-286, cmu-mosei/run.py:330-339,
+ * Ren-MME/run.py:283-292 or rencecps/run.py:141-148, and the averaging of
+ * others/realformer.py:418-420, Ren-MME/run.py:560, robot_demo.py:610-615.
+ *   MMEMO_HEAD_BILINEAR (y (B, C)):  last = w0 x0[b], this = w1 x1[b] (w0, w1: (C, F)),
+ *       z = sum_{j,m} this_j last_m trans[j,m,:] (trans (C,C,C)),
+ *       out = w_out [this || LN_C(z; ln_gamma, ln_beta)] + b_out   (w_out (C, 2C)).
+ *   MMEMO_HEAD_STATE_TRANSFER (y (B, P, C)): for row r = b*P + p of x0 (B*P rows),
+ *       h = ReLU(LN_d(w0 x0[r] + b0; ln_gamma, ln_beta))   (w0 (d, F)),
+ *       [o | g] = w_out h + b_out   (w_out (2C, d)), then the window recurrence of
+ *       mmemo_state_transfer_fwd with trans (C, C).
+ * x0 / x1 rows are ld0 / ld1 floats apart (>= F); weights are contiguous.  members: HOST array.
+ * C <= 16, d <= 1024, else MMEMO_ERR_SHAPE; a null required pointer is MMEMO_ERR_ARG.  Every member
+ * is checked before the first launch; one launch per 8 members (later launches add to y).
+ * ------------------------------------------------------------------------------------------- */
+#define MMEMO_HEAD_BILINEAR 0
+#define MMEMO_HEAD_STATE_TRANSFER 1
+typedef struct mmemo_ensemble_member {
+  const float* x0;        /* BILINEAR: x_last (B, F);  STATE_TRANSFER: x (B*P, F) */
+  int64_t ld0;
+  const float* x1;        /* BILINEAR: x_this (B, F);  STATE_TRANSFER: unused */
+  int64_t ld1;
+  const float* w0;        /* BILINEAR: W_last (C, F);  STATE_TRANSFER: W_fc (d, F) */
+  const float* w1;        /* BILINEAR: W_this (C, F);  STATE_TRANSFER: unused */
+  const float* b0;        /* BILINEAR: unused;         STATE_TRANSFER: b_fc (d) */
+  const float* ln_gamma;  /* LayerNorm over C (BILINEAR) or d (STATE_TRANSFER) */
+  const float* ln_beta;
+  const float* w_out;     /* BILINEAR: (C, 2C);        STATE_TRANSFER: W_cls (2C, d) */
+  const float* b_out;     /* BILINEAR: (C);            STATE_TRANSFER: b_cls (2C) */
+  const float* trans;     /* BILINEAR: (C, C, C);      STATE_TRANSFER: (C, C) */
+} mmemo_ensemble_member;
+int mmemo_ensemble_head_fwd(int kind, int n_members, const mmemo_ensemble_member* members,
+                            int64_t B, int64_t P, int64_t F, int64_t d, int64_t C, float eps,
+                            float* y, mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Data-parallel gradient exchange (new; the reference is single-GPU, others/realformer.py:16).

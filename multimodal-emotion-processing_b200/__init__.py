@@ -9,5 +9,5 @@ missing: there is no CPU fallback.
 __version__ = "0.1.0"
 
 from .blocks import get_precision, precision, set_precision  # noqa: E402,F401
-from . import batching, cmu_mosei, optim, realformer, ren_mme, rencecps, robot_demo, synth, trainer  # noqa: E402,F401
+from . import batching, cmu_mosei, ensemble, optim, realformer, ren_mme, rencecps, robot_demo, synth, trainer  # noqa: E402,F401
 from .encoder import ResidualEncoder  # noqa: E402,F401

@@ -28,6 +28,7 @@ _LN_BWD = [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp, 
 _ROWSUM = [_vp, _i64, _vp, _i64, _i64, _i64, _vp]
 _POOL_FWD = [_vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp, _vp]
 _POOL_BWD = [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _i64, _vp]
+_POOL_FWD_MULTI = [_i32, _vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp]
 _DROPOUT = [_vp, _vp, _i64, _f32, _u64, _vp]
 
 class AttnProblem(C.Structure):
@@ -40,6 +41,15 @@ class AttnProblem(C.Structure):
                 ("dq", _vp), ("dk", _vp), ("dv", _vp), ("lddq", _i64), ("lddk", _i64),
                 ("lddv", _i64), ("ds_prev", _vp), ("dc", _vp)]
 
+
+class EnsembleMember(C.Structure):
+    """mmemo_ensemble_member of include/mmemo.h (field order and types must match)."""
+    _fields_ = [("x0", _vp), ("ld0", _i64), ("x1", _vp), ("ld1", _i64), ("w0", _vp), ("w1", _vp),
+                ("b0", _vp), ("ln_gamma", _vp), ("ln_beta", _vp), ("w_out", _vp), ("b_out", _vp),
+                ("trans", _vp)]
+
+
+HEAD_BILINEAR, HEAD_STATE_TRANSFER = 0, 1      # MMEMO_HEAD_* of include/mmemo.h
 
 SIGNATURES = {
     "mmemo_version": [],
@@ -83,6 +93,8 @@ SIGNATURES = {
     "mmemo_dropout_multi_bf16": [_i32, _vp, _vp, _vp, _vp, _f32, _vp, _vp],
     "mmemo_pool_fwd_f32": _POOL_FWD, "mmemo_pool_fwd_bf16": _POOL_FWD,
     "mmemo_pool_bwd_f32": _POOL_BWD, "mmemo_pool_bwd_bf16": _POOL_BWD,
+    "mmemo_pool_fwd_multi_f32": _POOL_FWD_MULTI, "mmemo_pool_fwd_multi_bf16": _POOL_FWD_MULTI,
+    "mmemo_ensemble_head_fwd": [_i32, _i32, _vp, _i64, _i64, _i64, _i64, _i64, _f32, _vp, _vp],
     "mmemo_state_transfer_fwd": [_vp, _vp, _vp, _i64, _i64, _i64, _vp],
     "mmemo_state_transfer_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp],
     "mmemo_bilinear_head_fwd": [_vp] * 9 + [_i64, _i64, _f32, _vp],

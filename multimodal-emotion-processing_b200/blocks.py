@@ -204,16 +204,18 @@ def fusion_trunk(blocks: Sequence[nn.Module], n_layers: int, feats: Dict[str, to
     return fusion_trunk_multi([(blocks, feats, masks)], n_layers, keep_all)[0]
 
 
-def fusion_trunk_multi(towers, n_layers: int, keep_all: bool) -> List[torch.Tensor]:
+def fusion_trunk_multi(towers, n_layers: int, keep_all: bool, pool: bool = True) -> List:
     """Several independent trunks of the same architecture at once — the two towers of
     ``Concat_Trans`` / ``Base_model`` (cmu-mosei/run.py:330-331, Ren-MME/run.py:283-284), the
     members of an ensemble (robot_demo.py:610-614).  ``towers`` = [(blocks, feats, masks), ...];
-    returns one pooled tensor per tower.  Layer i of every chain of every tower is one grouped op
-    (``group_ops``); training dropout (Ren-MME and robot_demo train with p = 0.1) runs inside it as
-    one grouped launch per dropout site."""
+    returns one pooled tensor per tower, or with ``pool=False`` each tower's list of pooling
+    segments (the input of ``ops.pool`` / ``ops.pool_multi``).  Layer i of every chain of every
+    tower is one grouped op (``group_ops``); training dropout (Ren-MME and robot_demo train with
+    p = 0.1) runs inside it as one grouped launch per dropout site."""
     blk0 = towers[0][0][0]
     if not GROUPED_TRUNK:
-        return [_fusion_trunk_per_block(b, n_layers, f, m, keep_all) for b, f, m in towers]
+        segs = [_trunk_segments_per_block(b, n_layers, f, m, keep_all) for b, f, m in towers]
+        return [ops.pool(s, 3) for s in segs] if pool else segs
     drop_p = float(blk0.drop.p) if blk0.training else 0.0
     from . import group_ops
     bf = is_bf16()
@@ -241,19 +243,19 @@ def fusion_trunk_multi(towers, n_layers: int, keep_all: bool) -> List[torch.Tens
         for g in range(G):
             if keep_all or i + 1 == n_layers:
                 per_chain[g].append(qs[g])
-    pooled = []
+    segs = []
     for t in range(len(towers)):
         outs: Dict[str, List[torch.Tensor]] = {"l": [], "v": [], "a": []}
         for ci, (qm, _) in enumerate(CHAINS):
             outs[qm] += per_chain[t * len(CHAINS) + ci]
         # feature concat per modality, position concat in the order (l, a, v), mean||max pooling
-        pooled.append(ops.pool(outs["l"] + outs["a"] + outs["v"], 3))
-    return pooled
+        segs.append(outs["l"] + outs["a"] + outs["v"])
+    return [ops.pool(s, 3) for s in segs] if pool else segs
 
 
-def _fusion_trunk_per_block(blocks: Sequence[nn.Module], n_layers: int,
-                            feats: Dict[str, torch.Tensor], masks: Dict[str, torch.Tensor],
-                            keep_all: bool) -> torch.Tensor:
+def _trunk_segments_per_block(blocks: Sequence[nn.Module], n_layers: int,
+                              feats: Dict[str, torch.Tensor], masks: Dict[str, torch.Tensor],
+                              keep_all: bool) -> List[torch.Tensor]:
     outs: Dict[str, List[torch.Tensor]] = {"l": [], "v": [], "a": []}
     for ci, (qm, sm) in enumerate(CHAINS):
         q, s = feats[qm], None
@@ -266,5 +268,5 @@ def _fusion_trunk_per_block(blocks: Sequence[nn.Module], n_layers: int,
                 outs[qm].append(q)
         if not keep_all:
             outs[qm].append(q)
-    # feature concat per modality, position concat in the order (l, a, v), mean||max pooling
-    return ops.pool(outs["l"] + outs["a"] + outs["v"], 3)
+    # feature concat per modality, position concat in the order (l, a, v)
+    return outs["l"] + outs["a"] + outs["v"]

@@ -5,7 +5,7 @@
 // Ren-MME/run.py:266-270, robot_demo.py:435-439): four concat copies + two reductions.  Here every
 // chain output stays where its block wrote it; one kernel walks the segment table.
 // Pooling is mask-unaware (padded positions are pooled) exactly like the reference.
-#include "common.cuh"
+#include "pool.cuh"
 
 namespace {
 
@@ -26,32 +26,9 @@ pool_fwd_kernel(SegTable tb, int64_t B, int d, float* __restrict__ out, int32_t*
   const int64_t b = blockIdx.y;
   if (f >= F) return;
   const int slot = f / d, k = f - slot * d;
-  float sum = 0.f, mx = -INFINITY;
-  int arg = 0, pos = 0;
-  for (int g = 0; g < tb.n_groups; ++g) {
-    const T* __restrict__ p = static_cast<const T*>(tb.ptr[g * tb.n_slots + slot]) +
-                              b * (int64_t)tb.len[g] * d + k;
-    // eight independent loads in flight per thread (the positions of one feature are d elements
-    // apart: one load at a time left the kernel waiting on memory latency 320 times in a row)
-    const int n = tb.len[g];
-    int t = 0;
-    for (; t + 8 <= n; t += 8) {
-      float v[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] = to_f(p[(int64_t)(t + j) * d]);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        sum += v[j];
-        if (v[j] > mx) { mx = v[j]; arg = pos + j; }  // strict '>' keeps the FIRST maximum
-      }
-      pos += 8;
-    }
-    for (; t < n; ++t, ++pos) {
-      const float v = to_f(p[(int64_t)t * d]);
-      sum += v;
-      if (v > mx) { mx = v; arg = pos; }
-    }
-  }
+  float sum, mx;
+  int arg;
+  pool_column<T, true>(tb.ptr, tb.len, tb.n_groups, tb.n_slots, b, d, slot, k, sum, mx, &arg);
   out[b * 2 * F + f] = sum / (float)tb.total_len;
   out[b * 2 * F + F + f] = mx;
   amax[b * F + f] = arg;

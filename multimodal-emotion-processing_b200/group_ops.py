@@ -842,18 +842,22 @@ def project_into(xs, ws, biases, outs, poss=None) -> None:
     problem g writes ``x_g w_g^T + b_g (+ pos_g)`` into ``outs[g]``, a (rows, N_g) bf16 2-D view
     that may be a COLUMN SLICE of a wider buffer — the reference's ``cat`` of several projections
     (robot_demo.py:304-311) without the concat kernel — and ``pos_g`` may likewise be a column
-    slice of the (L, d) table added after that concat (robot_demo.py:415-417).  One cast launch
-    per 16 inputs and ONE tensor-core launch for all problems (up to 48)."""
+    slice of the (L, d) table added after that concat (robot_demo.py:415-417).  An input tensor
+    that several problems share (the members of an ensemble read the same features) is cast once.
+    One cast launch per 16 tensors and ONE tensor-core launch for all problems (up to 48)."""
     ops._need_cuda(*xs)
     G = len(xs)
     poss = poss if poss is not None else [None] * G
-    todo, xbs, wps = [], [], []
+    todo, xbs, wps, cast = [], [], [], {}
     for x in xs:
-        K = x.shape[-1]
-        x2 = x.reshape(-1, K)
-        x2 = x2 if x2.stride(1) == 1 else x2.contiguous()
-        xb = torch.empty(x2.shape[0], _pad8(K), dtype=BF, device=x.device)
-        todo.append((x2, xb))
+        xb = cast.get(id(x))
+        if xb is None:
+            K = x.shape[-1]
+            x2 = x.reshape(-1, K)
+            x2 = x2 if x2.stride(1) == 1 else x2.contiguous()
+            xb = torch.empty(x2.shape[0], _pad8(K), dtype=BF, device=x.device)
+            todo.append((x2, xb))
+            cast[id(x)] = xb
         xbs.append(xb)
     for w in ws:
         wps.append(_padded_shadow(w, todo))

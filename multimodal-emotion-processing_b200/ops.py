@@ -1109,6 +1109,31 @@ def pool(segs: Sequence[Tensor], n_groups: int = 3) -> Tensor:
     return pool_op(list(segs), n_groups)[0]
 
 
+def pool_multi(towers: Sequence[Sequence[Tensor]], n_groups: int = 3) -> List[Tensor]:
+    """Inference pooling of several trunks (same B, d, lengths) in one call: ``pool`` of every
+    tower's segment list, without argmax and without autograd."""
+    segs = [[t.contiguous() for t in tw] for tw in towers]
+    _need_cuda(*segs[0])
+    n_slots = len(segs[0]) // n_groups
+    B, _, d = segs[0][0].shape
+    _, lens, _ = _seg_table(segs[0], n_groups)
+    outs = [torch.empty(B, 2 * n_slots * d, dtype=F32, device=segs[0][0].device) for _ in segs]
+    _call(f"mmemo_pool_fwd_multi_{_sfx(segs[0][0].dtype == BF)}", len(segs),
+          _arr(C.c_void_p, [t.data_ptr() for tw in segs for t in tw]), lens, n_groups, n_slots,
+          B, d, _arr(C.c_void_p, [o.data_ptr() for o in outs]), _stream())
+    return outs
+
+
+def ensemble_head(kind: int, members: Sequence, B: int, P: int, F: int, d: int, n_cls: int,
+                  out: Tensor) -> None:
+    """``out`` (float32, (B, P, C) or (B, C)) = mean over ``members`` (``_lib.EnsembleMember``)
+    of their heads (include/mmemo.h mmemo_ensemble_head_fwd)."""
+    _need_cuda(out)
+    arr = (_lib.EnsembleMember * len(members))(*members)
+    _call("mmemo_ensemble_head_fwd", kind, len(members), C.cast(arr, C.c_void_p), B, P, F, d,
+          n_cls, LN_EPS, out.data_ptr(), _stream())
+
+
 # ------------------------------------------------------------------------------------------------
 # heads and losses (float32)
 # ------------------------------------------------------------------------------------------------

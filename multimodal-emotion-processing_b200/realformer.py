@@ -80,18 +80,26 @@ class Multi_class(nn.Module):
         self.normalization = nn.LayerNorm(dim)
         self.drop = nn.Dropout(DROP)
 
-    def forward(self, l, v, a, l_mask, v_mask, a_mask):
+    def positions(self, l, v, a):
+        """The three position tables, after checking the sequence lengths against them."""
         for x, pe in ((l, self.linguistic_position), (v, self.visual_position),
                       (a, self.acoustic_position)):
             if x.shape[1] != pe.len:  # the reference's `l + position(l)` broadcast would fail too
                 raise RuntimeError(f"sequence length {x.shape[1]} != position table {pe.len}")
-        pos = (self.linguistic_position.position_embeddings.weight,
-               self.visual_position.position_embeddings.weight,
-               self.acoustic_position.position_embeddings.weight)
-        l, v, a = self.unify_dimension(l, v, a, pos)       # projection + position add fused
-        x = fusion_trunk(self.multimodal_blocks, self.n_layers, {"l": l, "v": v, "a": a},
-                         {"l": as_mask(l_mask), "v": as_mask(v_mask), "a": as_mask(a_mask)},
-                         keep_all=False)
+        return (self.linguistic_position.position_embeddings.weight,
+                self.visual_position.position_embeddings.weight,
+                self.acoustic_position.position_embeddings.weight)
+
+    def _tower(self, l, v, a, l_mask, v_mask, a_mask):
+        """(blocks, projected + position-added features, masks) - the input of
+        ``fusion_trunk_multi`` (others/realformer.py:225-231)."""
+        l, v, a = self.unify_dimension(l, v, a, self.positions(l, v, a))   # position add fused
+        return (self.multimodal_blocks, {"l": l, "v": v, "a": a},
+                {"l": as_mask(l_mask), "v": as_mask(v_mask), "a": as_mask(a_mask)})
+
+    def forward(self, l, v, a, l_mask, v_mask, a_mask):
+        blocks, feats, masks = self._tower(l, v, a, l_mask, v_mask, a_mask)
+        x = fusion_trunk(blocks, self.n_layers, feats, masks, keep_all=False)
         x = ops.linear(x, self.fully_connected.weight, self.fully_connected.bias)   # float32 head
         x = ops.add_ln(None, x, None, self.normalization.weight, self.normalization.bias, relu=True)
         return ops.dropout(x, self.drop.p, self.training)

@@ -7,6 +7,7 @@ import torch.nn as nn
 
 from . import ops
 from .blocks import FullAttentionBlock, as_act, as_mask, fusion_trunk_multi, is_bf16
+from .ensemble import GraphedEnsemble
 
 DROP = 0.1  # robot_demo.py:41
 
@@ -100,7 +101,7 @@ def sigmoids(pred, offset):
     return torch.sigmoid(pred - offset)
 
 
-class Ensemble:
+class Ensemble(GraphedEnsemble):
     """Ensemble-of-models inference of ``demo_output`` / ``f1_calculation`` (robot_demo.py:526-581,
     597-622; SURVEY.md §8f-2): ``pred = (model_1(x) + ... + model_n(x)) / n`` under ``eval()`` and
     ``no_grad()``.
@@ -109,9 +110,8 @@ class Ensemble:
     batch 1 each member is ~350 launches of microsecond kernels, so the request is launch-bound.
     Here the members run on their own CUDA streams (forked from and joined into the caller's
     stream) and the whole request — input staging, all members, the average — is captured once per
-    input shape into a CUDA graph and replayed.  Weights are read at replay time from the members'
-    parameters (float32 mode); in bf16 mode the captured graph uses the bf16 weight shadows that
-    existed at capture time, so call ``refresh()`` after loading new weights.
+    input shape into a CUDA graph and replayed (``ensemble.GraphedEnsemble``: call ``refresh()``
+    after loading new weights in bf16 mode).
     """
 
     NAMES = ("l", "v_256", "v_512", "v_1024", "a", "l_mask", "v_mask", "a_mask")
@@ -119,18 +119,8 @@ class Ensemble:
     OFFSETS = {"happy": 0.1, "sad": 0.1, "angry": -0.1, "disgust": 0.0, "surprise": 0.1, "fear": 0.0}
 
     def __init__(self, models, use_graph: bool = True):
-        self.models = list(models)
-        if not self.models:
-            raise ValueError("Ensemble needs at least one model")
-        for m in self.models:
-            m.eval()
-        self.use_graph = use_graph
-        self._graphs = {}      # input-shape key -> (graph, static inputs, static output)
+        super().__init__(models, use_graph)
         self._streams = None
-
-    def refresh(self) -> None:
-        """Drop the captured graphs (after load_state_dict / precision changes)."""
-        self._graphs.clear()
 
     def _forward(self, args):
         """All members at once.  Members that are this module's ``Multi_class`` with one
@@ -196,33 +186,7 @@ class Ensemble:
 
     @torch.no_grad()
     def __call__(self, l, v_256, v_512, v_1024, a, l_mask, v_mask, a_mask):
-        args = (l, v_256, v_512, v_1024, a, l_mask, v_mask, a_mask)
-        if not all(t.is_cuda for t in args):
-            raise RuntimeError("mmemo_b200 runs on CUDA tensors only (no CPU fallback)")
-        if not self.use_graph:
-            return self._forward(args)
-        from .blocks import get_precision
-        key = (get_precision(),) + tuple((tuple(t.shape), t.dtype) for t in args)
-        entry = self._graphs.get(key)
-        if entry is None:
-            static_in = [torch.empty_like(t) for t in args]
-            for s, t in zip(static_in, args):
-                s.copy_(t)
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):          # warm-up off the capture: allocator, shadows
-                for _ in range(2):
-                    self._forward(static_in)
-            torch.cuda.current_stream().wait_stream(side)
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                static_out = self._forward(static_in)
-            entry = (graph, static_in, static_out)
-            self._graphs[key] = entry
-        graph, static_in, static_out = entry
-        torch._foreach_copy_(static_in, list(args))
-        graph.replay()
-        return static_out.clone()
+        return self._run((l, v_256, v_512, v_1024, a, l_mask, v_mask, a_mask))
 
     def emotions(self, pred: torch.Tensor) -> dict:
         """The scores ``demo_output`` prints for sample 0: sigmoid(logit - offset), rounded to 2
