@@ -427,6 +427,32 @@ typedef struct mmemo_ensemble_member {
 int mmemo_ensemble_head_fwd(int kind, int n_members, const mmemo_ensemble_member* members,
                             int64_t B, int64_t P, int64_t F, int64_t d, int64_t C, float eps,
                             float* y, mmemo_stream_t stream);
+/* The same, and every member's own output out_k in y_members (K, B, P, C) float32 (P = 1 for
+ * BILINEAR); y is bitwise what mmemo_ensemble_head_fwd writes. */
+int mmemo_ensemble_head_fwd_members(int kind, int n_members, const mmemo_ensemble_member* members,
+                                    int64_t B, int64_t P, int64_t F, int64_t d, int64_t C,
+                                    float eps, float* y, float* y_members, mmemo_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Fold-ensemble uncertainty (inference, new: the reference scripts only sum the logits).  logits
+ * (K, N, C) contiguous, T = float32 / bf16, K >= 1 folds of N rows; natural log, nats.  Per row n,
+ * with p_k = softmax(logits[k, n]) (max subtracted):
+ *   mean_prob[n, c]      = (1/K) sum_k p_k[c]                                       (N, C)
+ *   var_prob[n, c]       = (1/(K-1)) sum_k (p_k[c] - mean_prob[n, c])^2, 0 if K = 1  (N, C)
+ *   entropy[n]           = -sum_c mean_prob log mean_prob                          (N)
+ *   expected_entropy[n]  = (1/K) sum_k -sum_c p_k[c] log p_k[c]                     (N)
+ *   mutual_info[n]       = max(entropy - expected_entropy, 0), 0 if K = 1          (N)
+ *   label[n]             = first argmax_c mean_prob[n, c]                          (N) int64
+ * One warp per row, the folds in registers.  C <= 1024, else MMEMO_ERR_SHAPE.
+ * ------------------------------------------------------------------------------------------- */
+int mmemo_fold_uncertainty_f32(const void* logits, int64_t K, int64_t N, int64_t C,
+                               float* mean_prob, float* var_prob, float* entropy,
+                               float* expected_entropy, float* mutual_info, int64_t* label,
+                               mmemo_stream_t stream);
+int mmemo_fold_uncertainty_bf16(const void* logits, int64_t K, int64_t N, int64_t C,
+                                float* mean_prob, float* var_prob, float* entropy,
+                                float* expected_entropy, float* mutual_info, int64_t* label,
+                                mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Data-parallel gradient exchange (new; the reference is single-GPU, others/realformer.py:16).

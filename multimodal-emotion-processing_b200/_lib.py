@@ -30,6 +30,7 @@ _POOL_FWD = [_vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp, _vp]
 _POOL_BWD = [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _i64, _vp]
 _POOL_FWD_MULTI = [_i32, _vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp]
 _DROPOUT = [_vp, _vp, _i64, _f32, _u64, _vp]
+_FOLD_UQ = [_vp, _i64, _i64, _i64] + [_vp] * 6 + [_vp]
 
 class AttnProblem(C.Structure):
     """mmemo_attn_problem of include/mmemo.h (field order and types must match)."""
@@ -95,6 +96,9 @@ SIGNATURES = {
     "mmemo_pool_bwd_f32": _POOL_BWD, "mmemo_pool_bwd_bf16": _POOL_BWD,
     "mmemo_pool_fwd_multi_f32": _POOL_FWD_MULTI, "mmemo_pool_fwd_multi_bf16": _POOL_FWD_MULTI,
     "mmemo_ensemble_head_fwd": [_i32, _i32, _vp, _i64, _i64, _i64, _i64, _i64, _f32, _vp, _vp],
+    "mmemo_ensemble_head_fwd_members": [_i32, _i32, _vp, _i64, _i64, _i64, _i64, _i64, _f32, _vp,
+                                        _vp, _vp],
+    "mmemo_fold_uncertainty_f32": _FOLD_UQ, "mmemo_fold_uncertainty_bf16": _FOLD_UQ,
     "mmemo_state_transfer_fwd": [_vp, _vp, _vp, _i64, _i64, _i64, _vp],
     "mmemo_state_transfer_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp],
     "mmemo_bilinear_head_fwd": [_vp] * 9 + [_i64, _i64, _f32, _vp],

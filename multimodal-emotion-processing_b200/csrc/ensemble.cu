@@ -2,6 +2,7 @@
 // robot_demo.py:610-615: pred = mean of the members' logits).
 //   pool_fwd_multi    : the mean || max pooling of many fusion trunks (towers) in one launch
 //   ensemble_head_fwd : every member's classifier linears + head, and the member mean, in one launch
+//                       (_members: each member's output as well, for fold_uncertainty)
 #include <cooperative_groups.h>
 #include <math.h>
 
@@ -121,7 +122,8 @@ __device__ __forceinline__ float head_sigmoid(float x) { return 1.0f / (1.0f + e
 
 template <bool ST>
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(NT, 1)
-ensemble_head_kernel(HeadTable tb, HeadShape sh, float* __restrict__ y, int member0, int n_total) {
+ensemble_head_kernel(HeadTable tb, HeadShape sh, float* __restrict__ y, float* __restrict__ ym,
+                     int member0, int n_total) {
   extern __shared__ float sm[];
   cg::cluster_group cluster = cg::this_cluster();
   const int rank = (int)cluster.block_rank();
@@ -236,10 +238,12 @@ ensemble_head_kernel(HeadTable tb, HeadShape sh, float* __restrict__ y, int memb
             o = (1.0f - alpha) * o + alpha * tanhf(uu);
           }
           if (on) {
-            float* yp = y + ((int64_t)s * P + p) * C + lane;
+            const int64_t e = ((int64_t)s * P + p) * C + lane;
+            float* yp = y + e;
             float acc = gm == 0 ? o : *yp + o;
             if (gm + 1 == n_total) acc = acc / (float)n_total;
             *yp = acc;
+            if (ym) ym[(int64_t)gm * sh.B * P * C + e] = o;
           }
           op = o;
           gp = g;
@@ -283,6 +287,7 @@ ensemble_head_kernel(HeadTable tb, HeadShape sh, float* __restrict__ y, int memb
           float acc = gm == 0 ? o : *yp + o;
           if (gm + 1 == n_total) acc = acc / (float)n_total;
           *yp = acc;
+          if (ym) ym[((int64_t)gm * sh.B + s) * C + lane] = o;
         }
       }
     }
@@ -311,9 +316,12 @@ int mmemo_pool_fwd_multi_bf16(int n_towers, const void* const* seg_ptrs, const i
                               mm_stream(s));
 }
 
-int mmemo_ensemble_head_fwd(int kind, int n_members, const mmemo_ensemble_member* members,
-                            int64_t B, int64_t P, int64_t F, int64_t d, int64_t C, float eps,
-                            float* y, mmemo_stream_t s) {
+}  // extern "C"
+
+namespace {
+int ensemble_head(int kind, int n_members, const mmemo_ensemble_member* members, int64_t B,
+                  int64_t P, int64_t F, int64_t d, int64_t C, float eps, float* y, float* ym,
+                  mmemo_stream_t s) {
   MM_REQUIRE(kind == MMEMO_HEAD_BILINEAR || kind == MMEMO_HEAD_STATE_TRANSFER);
   MM_REQUIRE(n_members >= 1 && members && y && B >= 0 && F >= 1);
   const bool st = kind == MMEMO_HEAD_STATE_TRANSFER;
@@ -349,9 +357,23 @@ int mmemo_ensemble_head_fwd(int kind, int n_members, const mmemo_ensemble_member
   for (int k0 = 0; k0 < n_members; k0 += HEAD_MAX_MEMBERS) {
     tb.n = n_members - k0 < HEAD_MAX_MEMBERS ? n_members - k0 : HEAD_MAX_MEMBERS;
     for (int k = 0; k < tb.n; ++k) tb.m[k] = members[k0 + k];
-    kern<<<grid, NT, smem, mm_stream(s)>>>(tb, sh, y, k0, n_members);
+    kern<<<grid, NT, smem, mm_stream(s)>>>(tb, sh, y, ym, k0, n_members);
     MM_LAUNCH_OK();
   }
   return MMEMO_OK;
+}
+}  // namespace
+
+extern "C" {
+int mmemo_ensemble_head_fwd(int kind, int n_members, const mmemo_ensemble_member* members,
+                            int64_t B, int64_t P, int64_t F, int64_t d, int64_t C, float eps,
+                            float* y, mmemo_stream_t s) {
+  return ensemble_head(kind, n_members, members, B, P, F, d, C, eps, y, nullptr, s);
+}
+int mmemo_ensemble_head_fwd_members(int kind, int n_members, const mmemo_ensemble_member* members,
+                                    int64_t B, int64_t P, int64_t F, int64_t d, int64_t C,
+                                    float eps, float* y, float* y_members, mmemo_stream_t s) {
+  MM_REQUIRE(y_members);
+  return ensemble_head(kind, n_members, members, B, P, F, d, C, eps, y, y_members, s);
 }
 }

@@ -10,8 +10,35 @@ grouped LayerNorm (``Base_model``), one ``fusion_trunk_multi`` over every tower 
 grouped pooling launch and one ensemble-head launch that computes each member's classifier linears
 and head and writes only the member mean.  ``GraphedEnsemble`` captures a request per input shape
 into a CUDA graph and replays it; ``robot_demo.Ensemble`` uses it as well.
+
+Uncertainty.  ``Ensemble(...)(*batch, return_uncertainty=True)`` returns ``(logits, unc)``:
+``logits`` is bitwise the output of the same call without the flag, and ``unc`` an ``Uncertainty``
+computed from the k members' own logits (the head launch also writes them, then one
+``fold_uncertainty`` launch reduces them).  With ``p_i = softmax(logits of member i)`` over the C
+classes, natural logarithms (entropies in nats) and one value per utterance (per window for
+``State_Transfer``):
+
+- ``mean_prob``        ``(..., C)``  ``(1/k) sum_i p_i``; each row sums to 1.
+- ``variance``         ``(..., C)``  ``(1/(k-1)) sum_i (p_i - mean_prob)^2`` per class: how much the
+                                      folds disagree (unbiased; 0 when k = 1).
+- ``entropy``          ``(...)``     ``-sum_c mean_prob log mean_prob``, the predictive entropy,
+                                      in [0, log C].
+- ``expected_entropy`` ``(...)``     ``(1/k) sum_i -sum_c p_i log p_i``: the uncertainty each fold
+                                      reports on its own (noise in the input itself).
+- ``mutual_info``      ``(...)``     ``entropy - expected_entropy``, the part due to the folds
+                                      disagreeing; >= 0 (clamped at 0 against rounding; 0 when
+                                      k = 1).
+- ``label``            ``(...)``     int64, ``argmax mean_prob`` (the first on ties).  This is the
+                                      argmax of the mean probability, which can differ from the
+                                      argmax of the mean logits.
+
+``fold_uncertainty(fold_logits)`` is the same reduction for any ``(k, ..., C)`` float32 / bfloat16
+CUDA tensor (one sm_100a kernel, ``csrc/uncertainty.cu``); ``fold_uncertainty_reference`` computes
+it with PyTorch operations on any device, in float64, and is what the tests compare against.
 """
 from __future__ import annotations
+
+from typing import NamedTuple
 
 import torch
 
@@ -48,11 +75,13 @@ class GraphedEnsemble:
         raise NotImplementedError
 
     @torch.no_grad()
-    def _run(self, args):
+    def _run(self, args, *flags):
+        """``_forward(args, *flags)``, a Tensor or a tuple of Tensors; ``flags`` are part of the
+        graph key."""
         ops._need_cuda(*args)
         if not self.use_graph:
-            return self._forward(args)
-        key = (get_precision(),) + tuple((tuple(t.shape), t.dtype) for t in args)
+            return self._forward(args, *flags)
+        key = flags + (get_precision(),) + tuple((tuple(t.shape), t.dtype) for t in args)
         entry = self._graphs.get(key)
         if entry is None:
             static_in = [torch.empty_like(t) for t in args]
@@ -62,17 +91,59 @@ class GraphedEnsemble:
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):          # warm-up off the capture: allocator, shadows
                 for _ in range(2):
-                    self._forward(static_in)
+                    self._forward(static_in, *flags)
             torch.cuda.current_stream().wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                static_out = self._forward(static_in)
+                static_out = self._forward(static_in, *flags)
             entry = (graph, static_in, static_out)
             self._graphs[key] = entry
         graph, static_in, static_out = entry
         torch._foreach_copy_(static_in, list(args))
         graph.replay()
+        if isinstance(static_out, tuple):
+            return tuple(t.clone() for t in static_out)
         return static_out.clone()
+
+
+class Uncertainty(NamedTuple):
+    """How sure a k-fold ensemble is, per row of its output (definitions: module docstring)."""
+    mean_prob: torch.Tensor         # (..., C) float32
+    variance: torch.Tensor          # (..., C) float32
+    entropy: torch.Tensor           # (...) float32, nats
+    expected_entropy: torch.Tensor  # (...) float32, nats
+    mutual_info: torch.Tensor       # (...) float32, nats
+    label: torch.Tensor             # (...) int64
+
+
+def fold_uncertainty(fold_logits: torch.Tensor) -> Uncertainty:
+    """``Uncertainty`` of fold logits ``(k, ..., C)`` (float32 or bfloat16, contiguous, CUDA) in one
+    kernel launch on the current stream.  CPU tensors raise; use ``fold_uncertainty_reference``."""
+    return Uncertainty(*ops.fold_uncertainty(fold_logits))
+
+
+def fold_uncertainty_reference(fold_logits: torch.Tensor,
+                               dtype: torch.dtype = torch.float64) -> Uncertainty:
+    """The reduction of ``fold_uncertainty`` with PyTorch operations, on any device: computed in
+    ``dtype`` (float64 by default; float32 gives an eager baseline at the kernel's precision) from
+    the max-subtracted logits, returned as float32 (label int64)."""
+    if fold_logits.dim() < 2 or fold_logits.shape[0] < 1 or fold_logits.shape[-1] < 1:
+        raise ValueError("fold logits must have shape (K, ..., C) with K >= 1 and C >= 1, got "
+                         f"{tuple(fold_logits.shape)}")
+    x = fold_logits.to(dtype)
+    k = x.shape[0]
+    z = x - x.amax(-1, keepdim=True)
+    e = z.exp()
+    s = e.sum(-1, keepdim=True)
+    p = e / s
+    fold_h = s.squeeze(-1).log() - torch.where(p > 0, p * z, torch.zeros_like(p)).sum(-1)
+    mean = p.mean(0)
+    var = (p - mean).square().sum(0) / (k - 1) if k > 1 else torch.zeros_like(mean)
+    h = -torch.special.xlogy(mean, mean).sum(-1)
+    eh = fold_h.mean(0)
+    mi = (h - eh).clamp_min(0) if k > 1 else torch.zeros_like(h)
+    return Uncertainty(mean.float(), var.float(), h.float(), eh.float(), mi.float(),
+                       mean.argmax(-1))
 
 
 _FAMILIES = (State_Transfer, Concat_Trans, Base_model, Concat_Linear)
@@ -122,7 +193,8 @@ class Ensemble(GraphedEnsemble):
     shaped like one member's output.  Members: k fold models of ONE of ``State_Transfer``,
     ``Concat_Trans``, ``Base_model`` or ``Concat_Linear`` with equal state_dict shapes and equal
     ``n_heads`` / ``n_layers`` (``ValueError`` otherwise); the call takes the members' own forward
-    arguments, on CUDA."""
+    arguments, on CUDA.  ``return_uncertainty=True`` returns ``(logits, Uncertainty)`` instead
+    (module docstring); ``logits`` is unchanged."""
 
     def __init__(self, models, use_graph: bool = True):
         models = list(models)
@@ -130,16 +202,31 @@ class Ensemble(GraphedEnsemble):
         super().__init__(models, use_graph)
 
     @torch.no_grad()
-    def __call__(self, *args):
-        return self._run(args)
+    def __call__(self, *args, return_uncertainty: bool = False):
+        if not return_uncertainty:
+            return self._run(args)
+        logits, *unc = self._run(args, True)
+        return logits, Uncertainty(*unc)
 
-    def _forward(self, args):
+    def _forward(self, args, uncertainty: bool = False):
+        """The mean logits, or with ``uncertainty`` the tuple (mean logits, *Uncertainty)."""
         m0 = self.models[0]
         if isinstance(m0, State_Transfer):
-            return self._state_transfer(args)
+            return self._state_transfer(args, uncertainty)
         if isinstance(m0, Concat_Linear):
-            return self._concat_linear(args[0])
-        return self._bilinear(args)
+            return self._concat_linear(args[0], uncertainty)
+        return self._bilinear(args, uncertainty)
+
+    def _head(self, kind, mem, B, P, F, d, n_cls, shape, device, uncertainty):
+        """One ensemble-head launch into a new (shape) float32 output; with ``uncertainty`` it also
+        writes every member's output and one fold_uncertainty launch reduces them."""
+        out = torch.empty(shape, dtype=torch.float32, device=device)
+        if not uncertainty:
+            ops.ensemble_head(kind, mem, B, P, F, d, n_cls, out)
+            return out
+        folds = torch.empty((len(mem),) + tuple(shape), dtype=torch.float32, device=device)
+        ops.ensemble_head(kind, mem, B, P, F, d, n_cls, out, folds)
+        return (out,) + ops.fold_uncertainty(folds)
 
     # -- shared pieces ------------------------------------------------------------------------
     @staticmethod
@@ -164,7 +251,7 @@ class Ensemble(GraphedEnsemble):
                 zip(x3, (u.linguistic, u.visual, u.acoustic), poss)]
 
     # -- families -----------------------------------------------------------------------------
-    def _state_transfer(self, args):
+    def _state_transfer(self, args, uncertainty):
         """others/realformer.py:266-286 for every member: the B*P windows folded into the batch."""
         l, v, a, l_mask, v_mask, a_mask = args
         B, P = l.shape[0], l.shape[1]
@@ -186,11 +273,10 @@ class Ensemble(GraphedEnsemble):
                 ln_beta=_p(f.normalization.bias), w_out=_p(m.classifier.weight),
                 b_out=_p(m.classifier.bias), trans=_p(m.trans)))
         d, n_cls = f.fully_connected.weight.shape[0], m.trans.shape[0]
-        out = torch.empty(B, P, n_cls, dtype=torch.float32, device=l.device)
-        ops.ensemble_head(_lib.HEAD_STATE_TRANSFER, mem, B, P, pooled[0].shape[1], d, n_cls, out)
-        return out
+        return self._head(_lib.HEAD_STATE_TRANSFER, mem, B, P, pooled[0].shape[1], d, n_cls,
+                          (B, P, n_cls), l.device, uncertainty)
 
-    def _bilinear(self, args):
+    def _bilinear(self, args, uncertainty):
         """cmu-mosei/run.py:321-339 / Ren-MME/run.py:273-292 for every member: two towers each."""
         if isinstance(self.models[0], Concat_Trans):
             l, v, a, l_mask, v_mask, a_mask = args
@@ -225,9 +311,10 @@ class Ensemble(GraphedEnsemble):
             norm = m.norm1 if isinstance(m, Concat_Trans) else m.norm3
             mem.append(self._bilinear_member(last, this, m.intensity.classifier.weight,
                                              m.stimulation.classifier.weight, norm, m.out, m.trans))
-        return self._bilinear_head(mem, pooled[0].shape[0], pooled[0].shape[1], pooled[0].device)
+        return self._bilinear_head(mem, pooled[0].shape[0], pooled[0].shape[1], pooled[0].device,
+                                   uncertainty)
 
-    def _concat_linear(self, feat):
+    def _concat_linear(self, feat, uncertainty):
         """rencecps/run.py:130-148 for every member: feat (B, 2, F); the two halves are read through
         row strides."""
         feat = feat if feat.dtype == torch.float32 else feat.float()
@@ -236,7 +323,7 @@ class Ensemble(GraphedEnsemble):
         mem = [self._bilinear_member(feat[:, 0], feat[:, 1], m.intensity.weight,
                                      m.stimulation.weight, m.norm, m.out, m.trans)
                for m in self.models]
-        return self._bilinear_head(mem, B, F, feat.device)
+        return self._bilinear_head(mem, B, F, feat.device, uncertainty)
 
     @staticmethod
     def _bilinear_member(last, this, w_last, w_this, norm, out, trans):
@@ -245,8 +332,7 @@ class Ensemble(GraphedEnsemble):
             w0=_p(w_last), w1=_p(w_this), b0=None, ln_gamma=_p(norm.weight), ln_beta=_p(norm.bias),
             w_out=_p(out.weight), b_out=_p(out.bias), trans=_p(trans))
 
-    def _bilinear_head(self, mem, B, F, device):
+    def _bilinear_head(self, mem, B, F, device, uncertainty):
         n_cls = self.models[0].trans.shape[0]
-        out = torch.empty(B, n_cls, dtype=torch.float32, device=device)
-        ops.ensemble_head(_lib.HEAD_BILINEAR, mem, B, 1, F, 0, n_cls, out)
-        return out
+        return self._head(_lib.HEAD_BILINEAR, mem, B, 1, F, 0, n_cls, (B, n_cls), device,
+                          uncertainty)

@@ -1125,13 +1125,53 @@ def pool_multi(towers: Sequence[Sequence[Tensor]], n_groups: int = 3) -> List[Te
 
 
 def ensemble_head(kind: int, members: Sequence, B: int, P: int, F: int, d: int, n_cls: int,
-                  out: Tensor) -> None:
+                  out: Tensor, member_out: Optional[Tensor] = None) -> None:
     """``out`` (float32, (B, P, C) or (B, C)) = mean over ``members`` (``_lib.EnsembleMember``)
-    of their heads (include/mmemo.h mmemo_ensemble_head_fwd)."""
+    of their heads (include/mmemo.h mmemo_ensemble_head_fwd).  ``member_out`` (float32, (K,) +
+    out.shape): also each member's own output (mmemo_ensemble_head_fwd_members)."""
     _need_cuda(out)
     arr = (_lib.EnsembleMember * len(members))(*members)
-    _call("mmemo_ensemble_head_fwd", kind, len(members), C.cast(arr, C.c_void_p), B, P, F, d,
-          n_cls, LN_EPS, out.data_ptr(), _stream())
+    if member_out is None:
+        _call("mmemo_ensemble_head_fwd", kind, len(members), C.cast(arr, C.c_void_p), B, P, F, d,
+              n_cls, LN_EPS, out.data_ptr(), _stream())
+        return
+    assert member_out.dtype == F32 and member_out.is_contiguous()
+    assert member_out.shape == (len(members),) + tuple(out.shape)
+    _call("mmemo_ensemble_head_fwd_members", kind, len(members), C.cast(arr, C.c_void_p), B, P, F,
+          d, n_cls, LN_EPS, out.data_ptr(), member_out.data_ptr(), _stream())
+
+
+FOLD_UQ_MAX_CLASSES = 1024
+
+
+def fold_uncertainty(logits: Tensor) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """Fold logits ``(K, *rows, C)`` (float32 or bfloat16, contiguous, CUDA) -> (mean_prob,
+    var_prob, entropy, expected_entropy, mutual_info, label): float32 ``(*rows, C)`` twice,
+    float32 ``(*rows)`` three times and int64 ``(*rows)`` (include/mmemo.h
+    mmemo_fold_uncertainty_*).  One launch; no autograd."""
+    if not isinstance(logits, Tensor) or logits.dim() < 2:
+        raise ValueError("fold_uncertainty: logits must be a tensor of shape (K, ..., C)")
+    if logits.dtype not in (F32, BF):
+        raise TypeError(f"fold_uncertainty: logits must be float32 or bfloat16, got {logits.dtype}")
+    _need_cuda(logits)
+    if not logits.is_contiguous():
+        raise ValueError("fold_uncertainty: logits must be contiguous")
+    K, rows, n_cls = logits.shape[0], tuple(logits.shape[1:-1]), logits.shape[-1]
+    if K < 1 or n_cls < 1:
+        raise ValueError(f"fold_uncertainty: need K >= 1 folds and C >= 1 classes, got shape "
+                         f"{tuple(logits.shape)}")
+    if n_cls > FOLD_UQ_MAX_CLASSES:
+        raise ValueError(f"fold_uncertainty: C = {n_cls} classes, at most {FOLD_UQ_MAX_CLASSES}")
+    N = math.prod(rows)
+    dev = logits.device
+    mean_p = torch.empty(*rows, n_cls, dtype=F32, device=dev)
+    var_p = torch.empty(*rows, n_cls, dtype=F32, device=dev)
+    ent, exp_ent, mi = (torch.empty(rows, dtype=F32, device=dev) for _ in range(3))
+    label = torch.empty(rows, dtype=torch.int64, device=dev)
+    _call(f"mmemo_fold_uncertainty_{_sfx(logits.dtype == BF)}", logits.data_ptr(), K, N, n_cls,
+          mean_p.data_ptr(), var_p.data_ptr(), ent.data_ptr(), exp_ent.data_ptr(), mi.data_ptr(),
+          label.data_ptr(), _stream())
+    return mean_p, var_p, ent, exp_ent, mi, label
 
 
 # ------------------------------------------------------------------------------------------------
