@@ -4,13 +4,12 @@
 from __future__ import annotations
 
 import contextlib
-import os
 from typing import Dict, List, Optional, Sequence
 
 import torch
 import torch.nn as nn
 
-from . import ops
+from . import group_ops, ops
 
 _STATE = {"bf16": False}
 
@@ -64,6 +63,20 @@ def _split_check(dim: int, n_heads: int) -> None:
         raise RuntimeError(f"dim {dim} is not divisible by n_heads {n_heads}")
 
 
+def _group_of_one(blk: nn.Module, op, q, kv, mask, scores, emit_scores: bool):
+    """``blk`` on K = V as a trunk group of one problem (``group_ops``): one autograd node for the
+    whole block, training dropout included; returns ``(out, scores or None)``."""
+    same = q is kv
+    q = as_act(q)
+    kv = q if same else as_act(kv)
+    m = as_mask(mask)
+    drop_p = float(blk.drop.p) if blk.training else 0.0
+    out = op([q], [kv], [m if m is not None else torch.empty(0, device=q.device)],
+             [scores] if scores is not None else [], blk._params(), blk.n_heads, is_bf16(),
+             emit_scores, drop_p, ops.next_dropout_seed() if drop_p > 0 else 0)
+    return out[0], (out[1] if out[1].numel() else None)
+
+
 class FullAttentionBlock(nn.Module):
     """RealFormer block with QKV projections, ReZero-gated post-LN and FFN.
     Reference: others/realformer.py:154-209 (ffn multiplier from the global ``FFN``) and
@@ -94,7 +107,7 @@ class FullAttentionBlock(nn.Module):
         """dp.GradReducer protocol: the parameters whose gradients the fused backward accumulates
         into ONE zero-filled buffer, with their offsets (the reducer carves that buffer out of an
         all-reduce bucket, so nothing is copied)."""
-        return ops.full_block_grad_layout(self._params())
+        return group_ops.full_grad_unit(self._params())
 
     def multi_head_attention(self, q, k, v, mask, scores=None):
         """Projected attention + output projection; returns (drop(proj(att v)), scores)."""
@@ -111,16 +124,9 @@ class FullAttentionBlock(nn.Module):
         """``emit_scores=False`` (not a reference argument; used by the fusion trunk for the last
         layer of a chain, whose scores feed nothing) skips writing the score tensor and returns
         ``(q, None)``; the default returns the scores like the reference."""
+        if k is v:
+            return _group_of_one(self, group_ops.trunk_full_op, q, k, mask, scores, emit_scores)
         bf = is_bf16()
-        fused = (k is v) and not (self.training and self.drop.p > 0)
-        if fused:  # one autograd node for the whole block
-            same = q is k
-            q = as_act(q)
-            k = q if same else as_act(k)
-            out = ops.block_full_op(q, k, as_mask(mask), scores, self._params(), self.n_heads, bf,
-                                    emit_scores, q is k)
-            s = out[1]
-            return out[0], (s if s.numel() else None)
         x, s = self.multi_head_attention(q, k, v, mask, scores)
         q = as_act(q)
         h1 = ops.add_ln(q, x, self.a, self.norm1.weight, self.norm1.bias)
@@ -157,7 +163,7 @@ class LiteAttentionBlock(nn.Module):
 
     def mmemo_grad_unit(self):
         """dp.GradReducer protocol (see FullAttentionBlock.mmemo_grad_unit)."""
-        return ops.lite_block_grad_layout(self._params())
+        return group_ops.lite_grad_unit(self._params())
 
     def multi_head_attention(self, q, k, v, mask, scores=None):
         bf = is_bf16()
@@ -167,18 +173,10 @@ class LiteAttentionBlock(nn.Module):
         return ops.dropout(x, self.drop.p, self.training), s
 
     def forward(self, q, k, v, mask, scores=None, emit_scores: bool = True):
+        if k is v:
+            return _group_of_one(self, group_ops.trunk_lite_op, q, k, mask, scores, emit_scores)
         bf = is_bf16()
         n = self._norm
-        fused = (k is v) and not (self.training and self.drop.p > 0)
-        if fused:
-            same = q is k
-            q = as_act(q)
-            k = q if same else as_act(k)
-            out = ops.block_lite_op(q, k, as_mask(mask), scores,
-                                    [self.proj.weight, self.minus.weight, n.weight, n.bias, self.c],
-                                    self.n_heads, bf, emit_scores)
-            s = out[1]
-            return out[0], (s if s.numel() else None)
         x, s = self.multi_head_attention(q, k, v, mask, scores)
         y = ops.linear(torch.cat([as_act(q), x], dim=-1), self.minus.weight, bf16=bf)
         y = ops.add_ln(None, y, None, n.weight, n.bias)
@@ -189,11 +187,6 @@ class LiteAttentionBlock(nn.Module):
 # others/realformer.py:232-257, cmu-mosei/run.py:278-313 — ll lv la vv vl va aa al av
 CHAINS = [("l", "l"), ("l", "v"), ("l", "a"), ("v", "v"), ("v", "l"), ("v", "a"),
           ("a", "a"), ("a", "l"), ("a", "v")]
-
-
-# One grouped launch per kernel and layer over all chains (group_ops.py); False = the per-block
-# path (one autograd node per block), kept for A/B measurements and as the dropout-training path.
-GROUPED_TRUNK = os.environ.get("MMEMO_GROUPED_TRUNK", "1") != "0"
 
 
 def fusion_trunk(blocks: Sequence[nn.Module], n_layers: int, feats: Dict[str, torch.Tensor],
@@ -213,11 +206,7 @@ def fusion_trunk_multi(towers, n_layers: int, keep_all: bool, pool: bool = True)
     tower is one grouped op (``group_ops``); training dropout (Ren-MME and robot_demo train with
     p = 0.1) runs inside it as one grouped launch per dropout site."""
     blk0 = towers[0][0][0]
-    if not GROUPED_TRUNK:
-        segs = [_trunk_segments_per_block(b, n_layers, f, m, keep_all) for b, f, m in towers]
-        return [ops.pool(s, 3) for s in segs] if pool else segs
     drop_p = float(blk0.drop.p) if blk0.training else 0.0
-    from . import group_ops
     bf = is_bf16()
     full = isinstance(blk0, FullAttentionBlock)
     op = group_ops.trunk_full_op if full else group_ops.trunk_lite_op
@@ -251,22 +240,3 @@ def fusion_trunk_multi(towers, n_layers: int, keep_all: bool, pool: bool = True)
         # feature concat per modality, position concat in the order (l, a, v), mean||max pooling
         segs.append(outs["l"] + outs["a"] + outs["v"])
     return [ops.pool(s, 3) for s in segs] if pool else segs
-
-
-def _trunk_segments_per_block(blocks: Sequence[nn.Module], n_layers: int,
-                              feats: Dict[str, torch.Tensor], masks: Dict[str, torch.Tensor],
-                              keep_all: bool) -> List[torch.Tensor]:
-    outs: Dict[str, List[torch.Tensor]] = {"l": [], "v": [], "a": []}
-    for ci, (qm, sm) in enumerate(CHAINS):
-        q, s = feats[qm], None
-        src, m = feats[sm], masks[sm]
-        for i in range(n_layers):
-            blk = blocks[n_layers * ci + i]
-            # the last layer's scores feed nothing: do not write them
-            q, s = blk(q, src, src, m, s, emit_scores=i + 1 < n_layers)
-            if keep_all:
-                outs[qm].append(q)
-        if not keep_all:
-            outs[qm].append(q)
-    # feature concat per modality, position concat in the order (l, a, v)
-    return outs["l"] + outs["a"] + outs["v"]

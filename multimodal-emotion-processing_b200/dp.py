@@ -203,9 +203,6 @@ class GradReducer:
                 ops.register_zbuf_dest(u.key, b.flat, off, u.total)
             for p, off in zip(b.params, b.offsets):
                 self._slot[p] = (bi, off)
-                if p.is_cuda and p.dim() >= 2 and self.zero_copy and p not in unit_of:
-                    # large weights: the fused backward writes dW straight into this slot
-                    ops.register_grad_dest(p, b.flat, off)
         self._built = True
 
     def _try_symmetric(self, sizes: List[int], device):
@@ -404,4 +401,4 @@ class GradReducer:
         self._hooks = []
         if self.buckets:      # the fused backward must stop writing into this reducer's buckets
             from . import ops
-            ops.unregister_grad_dests([b.flat for b in self.buckets])
+            ops.unregister_zbuf_dests([b.flat for b in self.buckets])

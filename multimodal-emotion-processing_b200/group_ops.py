@@ -3,12 +3,12 @@
 The nine chains of a fusion trunk (others/realformer.py:232-257, cmu-mosei/run.py:278-313,
 Ren-MME/run.py:230-265, robot_demo.py:399-434) are mutually independent (they share only their
 read-only inputs l, v, a), and so are the two towers of ``Concat_Trans`` / ``Base_model`` and the
-members of an inference ensemble.  The reference (and the per-block ops of ``ops.py``) walk them one
-after the other: 9 x n_layers blocks x ~18 launches of microsecond kernels per trunk.  Here layer i
-of every chain is ONE custom op whose forward / backward issue one GROUPED launch per kernel kind
-(weight casts, Q|KV projections, attention, output projection, LayerNorm, FFN, weight gradients ...)
-with the per-problem pointers in a table - ~8 launches per layer forward and ~10 backward,
-independent of the number of chains.
+members of an inference ensemble.  The reference walks them one after the other: 9 x n_layers
+blocks x ~18 launches of microsecond kernels per trunk.  Here layer i of every chain is ONE custom
+op whose forward / backward issue one GROUPED launch per kernel kind (weight casts, Q|KV
+projections, attention, output projection, LayerNorm, FFN, weight gradients ...) with the
+per-problem pointers in a table - ~8 launches per layer forward and ~10 backward, independent of
+the number of chains.  A block called on its own (``blocks.py``, K = V) is a group of one problem.
 
 Problem g of a group: q-stream ``qs[g]`` (B, Lq_g, d), source ``kvs[g]`` (B, Lk_g, d) (K = V, like
 every caller in the reference), mask ``masks[g]`` (B, Lk_g), previous scores ``s_prevs[g]`` or none,
@@ -154,9 +154,13 @@ def merge_shared_grads(bf16: bool, inputs, grads):
 # grouped attention core
 # ------------------------------------------------------------------------------------------------
 def _mma_group_ok(bf16: bool, qs, kvs, H: int, same_kv: bool) -> bool:
-    """True when every problem of the group runs on the mma.sync attention kernels (forward and
-    backward); the scores of such a group use the padded row stride."""
-    if not bf16:
+    """True when the group's attention runs as grouped mma.sync launches (forward and backward);
+    the scores of such a group use the padded row stride."""
+    # A group of one problem (a block called on its own) takes the per-problem entry points
+    # instead: they pick the tcgen05 kernels where those are faster (resattn_tc.cu, and
+    # resattn_tc2.cu for Lk = 256, which the check below does not exclude), and its scores keep
+    # the reference's unpadded (B, H, Lq, Lk) layout.  Fusion trunks have at least 9 problems.
+    if not bf16 or len(qs) < 2:
         return False
     lib = _lib.load()
     d = qs[0].shape[-1]
@@ -293,23 +297,41 @@ def trunk_full_op(qs: Sequence[Tensor], kvs: Sequence[Tensor], masks: Sequence[T
     return out
 
 
-def _full_zlayout(d: int, dff: int):
-    """Per-problem zero buffer: [dp2 (1+2d) | dp1 (1+2d) | db_f2 (d) | db_f1 (dff) | dc (1) | pad]
-    then dWq (d,d) dWkv (2d,d) dWo (d,d) dWf1 (dff,d) dWf2 (d,dff)."""
-    n_small, sizes = ops._zbuf_layout(d, dff)       # (the per-block op and the reducer share it)
-    return n_small, sizes, n_small + sum(sizes)
+def _pad64(n: int) -> int:
+    return (n + 63) // 64 * 64          # floats: 256-byte aligned
+
+
+def _full_zlen(d: int, dff: int) -> int:
+    return _pad64(2 * (1 + 2 * d) + d + dff + 1) + 4 * d * d + 2 * dff * d
 
 
 def _full_zviews(z: Tensor, d: int, dff: int):
-    n_small, sizes, _ = _full_zlayout(d, dff)
+    """Per-problem zero buffer: [dp2 (1+2d) | dp1 (1+2d) | db_f2 (d) | db_f1 (dff) | dc (1) | pad
+    to 256 B] then dWq (d,d) dWkv (2d,d) dWo (d,d) dWf1 (dff,d) dWf2 (d,dff)."""
     dp2, dp1 = z[:1 + 2 * d], z[1 + 2 * d:2 * (1 + 2 * d)]
     o = 2 * (1 + 2 * d)
     db_f2, db_f1, dc = z[o:o + d], z[o + d:o + d + dff], z[o + d + dff:o + d + dff + 1]
-    ws, o = [], n_small
-    for n, sh in zip(sizes, [(d, d), (2 * d, d), (d, d), (dff, d), (d, dff)]):
-        ws.append(z[o:o + n].view(sh))
-        o += n
+    ws, o = [], _pad64(o + d + dff + 1)
+    for sh in [(d, d), (2 * d, d), (d, d), (dff, d), (d, dff)]:
+        ws.append(z[o:o + sh[0] * sh[1]].view(sh))
+        o += sh[0] * sh[1]
     return dp2, dp1, db_f2, db_f1, dc, ws
+
+
+def _full_pgrads(z: Tensor, d: int, dff: int) -> List[Tensor]:
+    """The gradient of every parameter of a full block (order: N_FULL) as a view of its buffer."""
+    dp2, dp1, db_f2, db_f1, dc, ws = _full_zviews(z, d, dff)
+    return [ws[0], ws[1][:d], ws[1][d:], ws[2], dp1[1:1 + d], dp1[1 + d:], dp2[1:1 + d], dp2[1 + d:],
+            ws[3], db_f1, ws[4], db_f2, dp1[0:1], dp2[0:1], dc]
+
+
+def full_grad_unit(params: Sequence[Tensor]):
+    """(key parameter, [(parameter, offset in floats)], total floats) of a full block's gradient
+    buffer, for dp.GradReducer; the offsets are those of the views the backward hands to autograd."""
+    d, dff = params[0].shape[0], params[8].shape[0]
+    z = torch.empty(_full_zlen(d, dff), device="meta")
+    offsets = [g.storage_offset() for g in _full_pgrads(z, d, dff)]
+    return params[0], list(zip(params, offsets)), z.numel()
 
 
 @torch.library.custom_op("mmemo::trunk_full_bwd", mutates_args=())
@@ -318,7 +340,7 @@ def trunk_full_bwd_op(dh2s: Sequence[Tensor], ds_nexts: Sequence[Tensor], qs: Se
                       saved: Sequence[Tensor], params: Sequence[Tensor], n_heads: int, bf16: bool,
                       need_dsprev: bool, drop_p: float, drop_seed: int) -> List[Tensor]:
     """Returns per problem [dq, dkv, ds_prev] (empty placeholders where undefined) followed by ONE
-    float32 buffer holding every parameter gradient of the group (layout: _full_zlayout)."""
+    float32 buffer holding every parameter gradient of the group (layout: _full_zviews)."""
     G = len(qs)
     dt, dev = _act_dtype(bf16), qs[0].device
     d = qs[0].shape[-1]
@@ -337,7 +359,7 @@ def trunk_full_bwd_op(dh2s: Sequence[Tensor], ds_nexts: Sequence[Tensor], qs: Se
     sp = [s_prevs[g] if len(s_prevs) else None for g in range(G)]
     dsn = [_opt(t) for t in ds_nexts]
     dh2s = [t.contiguous() for t in dh2s]
-    _, _, zlen = _full_zlayout(d, dff)
+    zlen = _full_zlen(d, dff)
     # data parallel: every block's buffer is a region of an all-reduce bucket, zero-filled by the
     # reducer (dp.GradReducer, ops.register_zbuf_dest) - no fill here, no gradient copies later
     zbs = ops.claim_zbufs([p[0] for p in P], zlen)
@@ -445,7 +467,7 @@ def _trunk_full_backward(ctx, grads):
     zall = res[-1]
     d = qs[0].shape[-1]
     dff = params[8].shape[0]
-    _, _, zlen = _full_zlayout(d, dff)
+    zlen = _full_zlen(d, dff)
     dqs, dkvs, dsps, pgrads = [], [], [], []
     for g in range(G):
         dq, dkv, dsp = res[3 * g:3 * g + 3]
@@ -453,10 +475,8 @@ def _trunk_full_backward(ctx, grads):
         dkvs.append(dkv if dkv.numel() else None)
         dsps.append(dsp if dsp.numel() else None)
         zb = zall[g * zlen:(g + 1) * zlen] if zall.numel() else ops.zbuf_region(params[N_FULL * g])
-        dp2, dp1, db_f2, db_f1, dc, ws = _full_zviews(zb, d, dff)
-        pgrads += [ws[0], ws[1][:d], ws[1][d:], ws[2], dp1[1:1 + d], dp1[1 + d:], dp2[1:1 + d],
-                   dp2[1 + d:], ws[3], db_f1, ws[4], db_f2, dp1[0:1], dp2[0:1],
-                   dc if ctx.has_prev else None]
+        pg = _full_pgrads(zb, d, dff)
+        pgrads += pg[:-1] + [pg[-1] if ctx.has_prev else None]
     n_prev = G if ctx.has_prev else 0
     return (dqs, dkvs, [None] * G, dsps if need_dsprev else [None] * n_prev, pgrads, None, None,
             None, None, None)
@@ -515,17 +535,31 @@ def trunk_lite_op(qs: Sequence[Tensor], kvs: Sequence[Tensor], masks: Sequence[T
     return out
 
 
-def _lite_zlayout(d: int):
-    """[dpn (1+2d) | dc (1) | pad] then dWo (d,d), dWm (d,2d)."""
-    return ops.lite_zlayout(d)
+def _lite_zlen(d: int) -> int:
+    return _pad64(2 + 2 * d) + 3 * d * d
 
 
 def _lite_zviews(z: Tensor, d: int):
-    n_small, _ = _lite_zlayout(d)
+    """[dpn (1+2d) | dc (1) | pad to 256 B] then dWo (d,d), dWm (d,2d)."""
+    o = _pad64(2 + 2 * d)
     dpn, dc = z[:1 + 2 * d], z[1 + 2 * d:2 + 2 * d]
-    dwo = z[n_small:n_small + d * d].view(d, d)
-    dwm = z[n_small + d * d:n_small + 3 * d * d].view(d, 2 * d)
+    dwo = z[o:o + d * d].view(d, d)
+    dwm = z[o + d * d:o + 3 * d * d].view(d, 2 * d)
     return dpn, dc, dwo, dwm
+
+
+def _lite_pgrads(z: Tensor, d: int) -> List[Tensor]:
+    """The gradient of every parameter of a lite block (order: N_LITE) as a view of its buffer."""
+    dpn, dc, dwo, dwm = _lite_zviews(z, d)
+    return [dwo, dwm, dpn[1:1 + d], dpn[1 + d:], dc]
+
+
+def lite_grad_unit(params: Sequence[Tensor]):
+    """Like full_grad_unit for a lite block."""
+    d = params[0].shape[0]
+    z = torch.empty(_lite_zlen(d), device="meta")
+    offsets = [g.storage_offset() for g in _lite_pgrads(z, d)]
+    return params[0], list(zip(params, offsets)), z.numel()
 
 
 @torch.library.custom_op("mmemo::trunk_lite_bwd", mutates_args=())
@@ -552,7 +586,7 @@ def trunk_lite_bwd_op(douts: Sequence[Tensor], ds_nexts: Sequence[Tensor], qs: S
         masked = [torch.empty_like(t) for t in douts]
         ops._dropout_group(douts, masked, drop_p, ops.site_seeds(drop_seed, G, 1))
         douts = masked
-    _, zlen = _lite_zlayout(d)
+    zlen = _lite_zlen(d)
     zbs = ops.claim_zbufs([p[0] for p in P], zlen)       # (see trunk_full_bwd_op)
     if zbs is None:
         zall = torch.zeros(G * zlen, dtype=F32, device=dev)
@@ -642,7 +676,7 @@ def _trunk_lite_backward(ctx, grads):
                             *ctx.drop)
     zall = res[-1]
     d = qs[0].shape[-1]
-    _, zlen = _lite_zlayout(d)
+    zlen = _lite_zlen(d)
     dqs, dkvs, dsps, pgrads = [], [], [], []
     for g in range(G):
         dq, dkv, dsp = res[3 * g:3 * g + 3]
@@ -650,8 +684,8 @@ def _trunk_lite_backward(ctx, grads):
         dkvs.append(dkv if dkv.numel() else None)
         dsps.append(dsp if dsp.numel() else None)
         zb = zall[g * zlen:(g + 1) * zlen] if zall.numel() else ops.zbuf_region(params[N_LITE * g])
-        dpn, dc, dwo, dwm = _lite_zviews(zb, d)
-        pgrads += [dwo, dwm, dpn[1:1 + d], dpn[1 + d:], dc if ctx.has_prev else None]
+        pg = _lite_pgrads(zb, d)
+        pgrads += pg[:-1] + [pg[-1] if ctx.has_prev else None]
     n_prev = G if ctx.has_prev else 0
     return (dqs, dkvs, [None] * G, dsps if need_dsprev else [None] * n_prev, pgrads, None, None,
             None, None, None)

@@ -213,95 +213,45 @@ def _rows(x: Tensor) -> Tuple[Tensor, int, int]:
 
 
 # ------------------------------------------------------------------------------------------------
-# gradient destinations: data-parallel training (dp.GradReducer) registers, per parameter, its slot
-# in a flat all-reduce bucket; the fused block backward then lets the weight-gradient GEMMs write
-# straight into the bucket (no per-parameter copy).  Only valid while p.grad is None at backward
-# time (zero_grad(set_to_none=True)); the reducer disables it otherwise.
+# gradient regions: the backward of a fused block layer (group_ops) accumulates ALL parameter
+# gradients of a block (weight gradients + the small "+=" outputs) into one zero-filled buffer
+# ("zbuf", layout: group_ops.full_grad_unit / lite_grad_unit).  Under data parallelism the reducer
+# (dp.GradReducer) gives every block a contiguous bucket region with that layout and registers it
+# here, keyed by the block's first weight: the block's zbuf IS then a bucket slice, p.grad of all
+# its parameters are views of the bucket, and nothing is copied or filled per block.  Only valid
+# while p.grad is None at backward time (zero_grad(set_to_none=True)); the reducer disables it
+# otherwise.
 # ------------------------------------------------------------------------------------------------
-_grad_dest: dict = {}
+_zbuf_dest: dict = {}
 grad_dest_enabled = True
-# set by dp.GradReducer.backward(): the bucket slots were zero-filled before this backward, so
-# kernels that accumulate into them (split-K reduce-add) need no fill of their own
+# set by dp.GradReducer.backward(): the bucket regions were zero-filled before this backward
 grad_dest_zeroed = False
 
 
-# A slot can be WRITTEN by one op per backward: a parameter that is used twice (shared weights)
-# gets a fresh buffer for its second gradient and autograd sums the two as usual.
+# A region can be WRITTEN by one op per backward: a block that is used twice (shared weights) gets
+# a fresh buffer for its second gradient and autograd sums the two as usual.
 _dest_claimed: set = set()
-
-
-def register_grad_dest(param: Tensor, flat: Tensor, offset: int) -> None:
-    _grad_dest[param.data_ptr()] = (flat, offset, param.numel())
-
-
-def begin_backward() -> None:
-    """Called by dp.GradReducer.backward(): every slot is writable again."""
-    _dest_claimed.clear()
-
-
-def _claim(*ws: Tensor) -> bool:
-    keys = [w.data_ptr() for w in ws]
-    if any(k in _dest_claimed for k in keys):
-        return False
-    _dest_claimed.update(keys)
-    return True
-
-
-def clear_grad_dest() -> None:
-    _grad_dest.clear()
-    _zbuf_dest.clear()
-
-
-def unregister_grad_dests(flats: Sequence[Tensor]) -> None:
-    """Forget every destination that lives in one of ``flats`` (a reducer that goes away must not
-    leave entries keyed by parameter addresses a later model could reuse)."""
-    ids = {id(f) for f in flats}
-    for reg in (_grad_dest, _zbuf_dest):
-        for k in [k for k, v in reg.items() if id(v[0]) in ids]:
-            del reg[k]
-
-
-# The fused full block accumulates ALL its parameter gradients (five weight gradients + the small
-# "+=" outputs) into one zero-filled buffer ("zbuf", layout: full_block_grad_layout).  Under data
-# parallelism the reducer gives every block a contiguous bucket region with that layout and
-# registers it here (keyed by the block's Wq): the block's zbuf IS then a bucket slice, p.grad of
-# all 15 parameters are views of the bucket, and nothing is copied or filled per block.
-_zbuf_dest: dict = {}
 
 
 def register_zbuf_dest(key: Tensor, flat: Tensor, offset: int, total: int) -> None:
     _zbuf_dest[key.data_ptr()] = (flat, offset, total)
 
 
-def full_block_grad_layout(params: Sequence[Tensor]):
-    """(key parameter, [(parameter, offset in floats)], total floats) of a full block's zbuf; the
-    offsets are the views _block_full_backward hands to autograd."""
-    wq, wk, wv, wo, n1w, n1b, n2w, n2b, f1w, f1b, f2w, f2b, ga, gb, gc = params
-    d, dff = wq.shape[0], f1w.shape[0]
-    n_small, sizes = _zbuf_layout(d, dff)
-    p1, zo = 1 + 2 * d, 2 * (1 + 2 * d)
-    lay = [(gb, 0), (n2w, 1), (n2b, 1 + d), (ga, p1), (n1w, p1 + 1), (n1b, p1 + 1 + d),
-           (f2b, zo), (f1b, zo + d), (gc, zo + d + dff)]
-    o = n_small
-    for w, n in zip((wq, wk, wv, wo, f1w, f2w), (d * d, d * d, d * d, d * d, dff * d, d * dff)):
-        lay.append((w, o))
-        o += n
-    assert o == n_small + sum(sizes)
-    return wq, lay, o
+def begin_backward() -> None:
+    """Called by dp.GradReducer.backward(): every region is writable again."""
+    _dest_claimed.clear()
 
 
-def lite_zlayout(d: int):
-    """Zero buffer of a lite block: [dpn (1+2d) | dc (1) | pad] then dWo (d,d), dWm (d,2d)."""
-    n_small = (1 + 2 * d + 1 + 63) // 64 * 64
-    return n_small, n_small + d * d + 2 * d * d
+def clear_grad_dest() -> None:
+    _zbuf_dest.clear()
 
 
-def lite_block_grad_layout(params: Sequence[Tensor]):
-    """Like full_block_grad_layout for the lite block (params: Wo, Wm, norm weight, norm bias, c)."""
-    wo, wm, nw, nb, c = params
-    d = wo.shape[0]
-    n_small, total = lite_zlayout(d)
-    return wo, [(nw, 1), (nb, 1 + d), (c, 1 + 2 * d), (wo, n_small), (wm, n_small + d * d)], total
+def unregister_zbuf_dests(flats: Sequence[Tensor]) -> None:
+    """Forget every region that lives in one of ``flats`` (a reducer that goes away must not
+    leave entries keyed by parameter addresses a later model could reuse)."""
+    ids = {id(f) for f in flats}
+    for k in [k for k, v in _zbuf_dest.items() if id(v[0]) in ids]:
+        del _zbuf_dest[k]
 
 
 def claim_zbufs(keys: Sequence[Tensor], total: int) -> Optional[List[Tensor]]:
@@ -323,34 +273,8 @@ def zbuf_region(key: Tensor) -> Tensor:
     return z[0][z[1]:z[1] + z[2]]
 
 
-def _dest(w: Tensor) -> Optional[Tensor]:
-    e = _grad_dest.get(w.data_ptr()) if grad_dest_enabled else None
-    if e is None or e[2] != w.numel():
-        return None
-    return e[0][e[1]:e[1] + e[2]].view(w.shape)
-
-
-def _dest_pair(wa: Tensor, wb: Tensor) -> Optional[Tensor]:
-    """One (rows_a + rows_b, cols) buffer when the two parameters own adjacent bucket slots."""
-    if not grad_dest_enabled:
-        return None
-    ea, eb = _grad_dest.get(wa.data_ptr()), _grad_dest.get(wb.data_ptr())
-    if ea is None or eb is None or ea[0] is not eb[0] or ea[1] + ea[2] != eb[1]:
-        return None
-    return ea[0][ea[1]:ea[1] + ea[2] + eb[2]].view(wa.shape[0] + wb.shape[0], -1)
-
-
-def _wgrad(w: Tensor, rows: int, cols: int):
-    """(buffer to write dW into, tensor to return from the custom op)."""
-    d = _dest(w)
-    if d is not None and _claim(w):
-        return d.view(rows, cols), torch.empty(0, device=w.device)
-    buf = torch.empty(rows, cols, dtype=F32, device=w.device)
-    return buf, buf
-
-
 # ------------------------------------------------------------------------------------------------
-# raw launch helpers (no autograd) -- shared by the fine-grained ops and the fused block ops
+# raw launch helpers (no autograd) -- shared by the fine-grained ops and the grouped ops
 # ------------------------------------------------------------------------------------------------
 def _linear_fwd(bf16, x, w, bias, pos, out, relu=False, accumulate=False, ldw=None, N=None, K=None):
     x, M, ldx = _rows(x)
@@ -759,300 +683,6 @@ def _resattn_backward(ctx, do, ds, _dstat):
 
 
 resattn_op.register_autograd(_resattn_backward, setup_context=_resattn_setup)
-
-
-# ------------------------------------------------------------------------------------------------
-# mmemo::block_full — the whole RealFormer block as ONE autograd node
-#   (others/realformer.py:182-209 == robot_demo.py:347-374)
-# params order: wq wk wv wo  n1w n1b n2w n2b  f1w f1b f2w f2b  a b c
-# ------------------------------------------------------------------------------------------------
-@torch.library.custom_op("mmemo::block_full", mutates_args=())
-def block_full_op(q: Tensor, kv: Tensor, mask: Optional[Tensor], s_prev: Optional[Tensor],
-                  params: Sequence[Tensor], n_heads: int, bf16: bool, emit_s: bool,
-                  same_qkv: bool) -> List[Tensor]:
-    _need_cuda(q, kv)
-    wq, wk, wv, wo, n1w, n1b, n2w, n2b, f1w, f1b, f2w, f2b, ga, gb, gc = params
-    B, Lq, d = q.shape
-    Lk = kv.shape[1]
-    dt, dev = _act_dtype(bf16), q.device
-    q = q.contiguous()
-    kv = q if same_qkv else kv.contiguous()
-    if bf16:   # all bf16 weight shadows of the block in one cast launch
-        shadow_bf16_block([[wq], [wk, wv], [wo], [f1w], [f2w]])
-    # Q projection and fused [K|V] projection (one GEMM, N = 2d)
-    qp = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    kvp = torch.empty(B, Lk, 2 * d, dtype=dt, device=dev)
-    _linear_fwd_group(bf16, [(q, _weight(bf16, wq), None, qp.view(-1, d), False),
-                             (kv, _weight(bf16, wk, wv), None, kvp.view(-1, 2 * d), False)])
-    kp, vp = kvp[..., :d], kvp[..., d:]
-    o, s, stat = _attn_fwd(bf16, qp, kp, vp, mask, s_prev, gc, n_heads, emit_s)
-    # output projection, gated residual + LN1
-    x = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_fwd(bf16, o, _weight(bf16, wo), None, None, x.view(-1, d))
-    h1, st1 = _add_ln_fwd(bf16, q, x, ga, n1w, n1b)
-    # FFN (ReLU fused in the first GEMM's epilogue), gated residual + LN2
-    dff = f1w.shape[0]
-    f1 = torch.empty(B, Lq, dff, dtype=dt, device=dev)
-    f2 = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_fwd(bf16, h1, _weight(bf16, f1w), f1b, None, f1.view(-1, dff), relu=True)
-    _linear_fwd(bf16, f1, _weight(bf16, f2w), f2b, None, f2.view(-1, d))
-    h2, st2 = _add_ln_fwd(bf16, h1, f2, gb, n2w, n2b)
-    e = torch.empty(0, device=dev)
-    return [h2, s if s is not None else e, qp, kvp, o, stat, x, h1, st1, f1, f2, st2]
-
-
-def _zbuf_layout(d: int, dff: int):
-    """(floats of the small "+=" outputs rounded to 256 B, [sizes of dWq, dWkv, dWo, dWf1, dWf2])."""
-    n_small = (2 * (1 + 2 * d) + d + dff + 1 + 63) // 64 * 64
-    return n_small, [d * d, 2 * d * d, d * d, dff * d, d * dff]
-
-
-def _zbuf_weights(zbuf: Tensor, d: int, dff: int):
-    n_small, sizes = _zbuf_layout(d, dff)
-    shapes = [(d, d), (2 * d, d), (d, d), (dff, d), (d, dff)]
-    out, o = [], n_small
-    for n, sh in zip(sizes, shapes):
-        out.append(zbuf[o:o + n].view(sh))
-        o += n
-    return out
-
-
-@torch.library.custom_op("mmemo::block_full_bwd", mutates_args=())
-def block_full_bwd_op(dh2: Tensor, ds_next: Optional[Tensor], q: Tensor, kv: Tensor,
-                      mask: Optional[Tensor], s_prev: Optional[Tensor], s: Optional[Tensor],
-                      saved: Sequence[Tensor], params: Sequence[Tensor], n_heads: int, bf16: bool,
-                      same_qkv: bool, need_dsprev: bool) -> List[Tensor]:
-    wq, wk, wv, wo, n1w, n1b, n2w, n2b, f1w, f1b, f2w, f2b, ga, gb, gc = params
-    qp, kvp, o, stat, x, h1, st1, f1, f2, st2 = saved
-    B, Lq, d = q.shape
-    Lk = kv.shape[1]
-    dff = f1w.shape[0]
-    dt, dev = _act_dtype(bf16), q.device
-    q = q.contiguous()
-    kv = q if same_qkv else kv.contiguous()
-    dh2 = dh2.contiguous()
-    # one zero-filled buffer for every "+=" output of the block (LN params, biases, dc)
-    # ... and, unless they have a data-parallel bucket slot, for the five weight gradients
-    in_z = _dest(wq) is None
-    n_small, w_sizes = _zbuf_layout(d, dff)
-    zd = _zbuf_dest.get(wq.data_ptr()) if (grad_dest_enabled and grad_dest_zeroed) else None
-    in_bucket = zd is not None and zd[2] == n_small + sum(w_sizes) and _claim(wq)
-    if in_bucket:
-        zbuf = zd[0][zd[1]:zd[1] + zd[2]]     # a bucket region, zero-filled by the reducer
-        in_z = True
-    else:
-        zbuf = torch.zeros(n_small + (sum(w_sizes) if in_z else 0), dtype=F32, device=dev)
-    z_dp2, z_dp1 = zbuf[:1 + 2 * d], zbuf[1 + 2 * d:2 * (1 + 2 * d)]
-    zo = 2 * (1 + 2 * d)
-    # LN2: h2 = LN(h1 + b*f2)
-    # (the column sums of df2 = the bias gradient of the second FFN layer come out of the same pass)
-    db_f2 = zbuf[zo:zo + d]
-    dh1, df2, dp2 = _add_ln_bwd(bf16, dh2, h1, f2, gb, n2w, None, st2, False, True, dpar=z_dp2,
-                                dxsum=db_f2)
-    # FFN backward; df1 = (df2 W2) * (f1 > 0) fused in the GEMM epilogue
-    df1 = torch.empty(B, Lq, dff, dtype=dt, device=dev)
-    _linear_bwd_x(bf16, df2, _weight(bf16, f2w), df1.view(-1, dff), relu_src=f1.view(-1, dff))
-    if in_z:
-        dw_q, dw_kv, dw_o, dw_f1, dw_f2 = _zbuf_weights(zbuf, d, dff)
-        r_q = r_kv = r_o = r_f1 = r_f2 = None       # returned through zbuf
-    else:
-        dw_f2, r_f2 = _wgrad(f2w, d, dff)
-    _linear_bwd_x(bf16, df1, _weight(bf16, f1w), dh1.view(-1, d), accumulate=True)
-    if not in_z:
-        dw_f1, r_f1 = _wgrad(f1w, dff, d)
-    db_f1 = zbuf[zo + d:zo + d + dff]
-    _rowsum(bf16, df1.view(-1, dff), db_f1)
-    # LN1: h1 = LN(q + a*x)
-    dq, dx, dp1 = _add_ln_bwd(bf16, dh1, q, x, ga, n1w, None, st1, False, True, dpar=z_dp1)
-    # output projection
-    do = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_bwd_x(bf16, dx, _weight(bf16, wo), do.view(-1, d))
-    if not in_z:
-        dw_o, r_o = _wgrad(wo, d, d)
-    # attention core
-    dqp = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    dkvp = torch.empty(B, Lk, 2 * d, dtype=dt, device=dev)
-    ds_prev, _ = _attn_bwd(bf16, do, qp, kvp[..., :d], kvp[..., d:], mask, s, s_prev, gc, ds_next,
-                           o, stat, n_heads, dqp, dkvp[..., :d], dkvp[..., d:], need_dsprev,
-                           dc_out=zbuf[zo + d + dff:zo + d + dff + 1])
-    # projections: dq += dqp Wq ; dkv = dkvp [Wk;Wv]
-    all_dest = False
-    if not in_z:
-        dw_q, r_q = _wgrad(wq, d, d)
-        dw_kv = _dest_pair(wk, wv)
-        if dw_kv is not None and not _claim(wk, wv):
-            dw_kv = None
-        r_kv = torch.empty(0, device=dev)
-        if dw_kv is None:
-            dw_kv = r_kv = torch.empty(2 * d, d, dtype=F32, device=dev)
-        # every gradient of the group goes to a (zero-filled) bucket slot?
-        all_dest = not any(r.numel() for r in (r_q, r_kv, r_o, r_f1, r_f2))
-    if same_qkv:   # both input gradients accumulate into dq: keep them ordered
-        _linear_bwd_x(bf16, dqp, _weight(bf16, wq), dq.view(-1, d), accumulate=True)
-        _linear_bwd_x(bf16, dkvp, _weight(bf16, wk, wv), dq.view(-1, d), accumulate=True)
-        dkv = torch.empty(0, device=dev)
-    else:
-        dkv = torch.empty(B, Lk, d, dtype=dt, device=dev)
-        _linear_bwd_x_group(bf16, [(dqp, _weight(bf16, wq), dq.view(-1, d), True),
-                                   (dkvp, _weight(bf16, wk, wv), dkv.view(-1, d), False)])
-    # the five weight gradients of the block: one grouped launch (each alone fills < 1/4 of the GPU)
-    _linear_bwd_w_group(bf16, [(df2.view(-1, d), f1.view(-1, dff), dw_f2),
-                               (df1.view(-1, dff), h1.view(-1, d), dw_f1),
-                               (dx.view(-1, d), o.view(-1, d), dw_o),
-                               (dqp.view(-1, d), q.view(-1, d), dw_q),
-                               (dkvp.view(-1, 2 * d), kv.view(-1, d), dw_kv)],
-                        zeroed=in_z or (grad_dest_zeroed and all_dest))
-    # (dc lives in zbuf; its output slot stays an empty placeholder — like the weight gradients
-    # when they live in zbuf or in a bucket slot)
-    ph = [torch.empty(0, device=dev) if r is None else r for r in (r_q, r_kv, r_o, r_f1, r_f2)]
-    # (a zbuf that is a bucket region is not returned either: custom ops must not return views of
-    # tensors they do not own; the autograd wrapper looks the region up again)
-    return [dq, dkv, ds_prev if ds_prev is not None else torch.empty(0, device=dev),
-            torch.empty(0, device=dev), ph[0], ph[1], ph[2],
-            torch.empty(0, device=dev) if in_bucket else zbuf, ph[3], ph[4]]
-
-
-def _block_full_setup(ctx, inputs, output):
-    q, kv, mask, s_prev, params, H, bf16, emit_s, same_qkv = inputs
-    h2, s = output[0], output[1]
-    ctx.save_for_backward(q, kv, mask, s_prev, s if s.numel() else None, *output[2:], *params)
-    ctx.cfg = (H, bf16, same_qkv, len(output) - 2)
-    ctx.set_materialize_grads(False)
-
-
-def _block_full_backward(ctx, grads):
-    dh2, ds_next = grads[0], grads[1]
-    H, bf16, same_qkv, nsaved = ctx.cfg
-    t = ctx.saved_tensors
-    q, kv, mask, s_prev, s = t[:5]
-    saved, params = t[5:5 + nsaved], t[5 + nsaved:]
-    if dh2 is None:
-        dh2 = torch.zeros_like(q)
-    d = q.shape[-1]
-    need_dsprev = s_prev is not None and ctx.needs_input_grad[3]
-    (dq, dkv, ds_prev, dc, dw_q, dw_kv, dw_o, zbuf, dw_f1,
-     dw_f2) = block_full_bwd_op(dh2, ds_next, q, kv, mask, s_prev, s, saved, params, H, bf16,
-                                same_qkv, need_dsprev)
-    # the small "+=" outputs share one zero-initialised buffer: [dp2 | dp1 | db_f2 | db_f1 | dc]
-    dff = params[8].shape[0]
-    if zbuf.numel() == 0:                 # the block's zero buffer is a data-parallel bucket region
-        zd = _zbuf_dest[params[0].data_ptr()]
-        zbuf = zd[0][zd[1]:zd[1] + zd[2]]
-    dp2, dp1 = zbuf[:1 + 2 * d], zbuf[1 + 2 * d:2 * (1 + 2 * d)]
-    zo = 2 * (1 + 2 * d)
-    db_f2, db_f1 = zbuf[zo:zo + d], zbuf[zo + d:zo + d + dff]
-    dc = zbuf[zo + d + dff:zo + d + dff + 1]
-    has_prev = s_prev is not None
-    # weight gradients written straight into DP bucket slots come back as empty placeholders
-    wq, wk, wv, wo, f1w, f2w = params[0], params[1], params[2], params[3], params[8], params[10]
-    if zbuf.numel() > _zbuf_layout(d, dff)[0]:        # weight gradients inside the zero buffer
-        dw_q, dw_kv, dw_o, dw_f1, dw_f2 = _zbuf_weights(zbuf, d, dff)
-    else:
-        dw_q = dw_q if dw_q.numel() else _dest(wq)
-        dw_o = dw_o if dw_o.numel() else _dest(wo)
-        dw_f1 = dw_f1 if dw_f1.numel() else _dest(f1w)
-        dw_f2 = dw_f2 if dw_f2.numel() else _dest(f2w)
-        if not dw_kv.numel():
-            dw_kv = _dest_pair(wk, wv)
-    pgrads = [dw_q, dw_kv[:d], dw_kv[d:], dw_o, dp1[1:1 + d], dp1[1 + d:], dp2[1:1 + d],
-              dp2[1 + d:], dw_f1, db_f1, dw_f2, db_f2, dp1[0:1], dp2[0:1],
-              dc if has_prev else None]
-    return (dq, None if same_qkv else dkv, None, ds_prev if need_dsprev else None, pgrads,
-            None, None, None, None)
-
-
-block_full_op.register_autograd(_block_full_backward, setup_context=_block_full_setup)
-
-
-# ------------------------------------------------------------------------------------------------
-# mmemo::block_lite — concat -> minus -> LN block  (cmu-mosei/run.py:236-262, Ren-MME/run.py:188-214)
-# params order: wo(proj) wm(minus, (d,2d)) nw nb c
-# ------------------------------------------------------------------------------------------------
-@torch.library.custom_op("mmemo::block_lite", mutates_args=())
-def block_lite_op(q: Tensor, kv: Tensor, mask: Optional[Tensor], s_prev: Optional[Tensor],
-                  params: Sequence[Tensor], n_heads: int, bf16: bool, emit_s: bool) -> List[Tensor]:
-    _need_cuda(q, kv)
-    wo, wm, nw, nb, gc = params
-    B, Lq, d = q.shape
-    dt, dev = _act_dtype(bf16), q.device
-    q, kv = q.contiguous(), kv.contiguous()
-    o, s, stat = _attn_fwd(bf16, q, kv, kv, mask, s_prev, gc, n_heads, emit_s)
-    x = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_fwd(bf16, o, _weight(bf16, wo), None, None, x.view(-1, d))
-    # y = [q | x] Wm^T as two accumulating GEMMs over the halves of Wm (no concat copy)
-    wms = _weight(bf16, wm)
-    y = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_fwd(bf16, q, wms, None, None, y.view(-1, d), ldw=2 * d, N=d, K=d)
-    _linear_fwd(bf16, x, wms[:, d:], None, None, y.view(-1, d), accumulate=True, ldw=2 * d, N=d, K=d)
-    out, st = _add_ln_fwd(bf16, None, y, None, nw, nb)
-    e = torch.empty(0, device=dev)
-    return [out, s if s is not None else e, o, stat, x, y, st]
-
-
-@torch.library.custom_op("mmemo::block_lite_bwd", mutates_args=())
-def block_lite_bwd_op(dout: Tensor, ds_next: Optional[Tensor], q: Tensor, kv: Tensor,
-                      mask: Optional[Tensor], s_prev: Optional[Tensor], s: Optional[Tensor],
-                      saved: Sequence[Tensor], params: Sequence[Tensor], n_heads: int, bf16: bool,
-                      need_dsprev: bool) -> List[Tensor]:
-    wo, wm, nw, nb, gc = params
-    o, stat, x, y, st = saved
-    B, Lq, d = q.shape
-    Lk = kv.shape[1]
-    dt, dev = _act_dtype(bf16), q.device
-    q, kv = q.contiguous(), kv.contiguous()
-    _, dy, dpn = _add_ln_bwd(bf16, dout.contiguous(), None, y, None, nw, None, st, False, False)
-    wms = _weight(bf16, wm)
-    # minus: dq = dy Wm[:, :d], dx = dy Wm[:, d:], dWm = dy^T [q | x]
-    dq = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    dx = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_bwd_x(bf16, dy, wms, dq.view(-1, d), ldw=2 * d, N=d, K=d)
-    _linear_bwd_x(bf16, dy, wms[:, d:], dx.view(-1, d), ldw=2 * d, N=d, K=d)
-    dwm = torch.empty(d, 2 * d, dtype=F32, device=dev)
-    _linear_bwd_w(bf16, dy.view(-1, d), q.view(-1, d), dwm)
-    _linear_bwd_w(bf16, dy.view(-1, d), x.view(-1, d), dwm[:, d:])
-    # proj
-    do = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    _linear_bwd_x(bf16, dx, _weight(bf16, wo), do.view(-1, d))
-    dwo = torch.empty(d, d, dtype=F32, device=dev)
-    _linear_bwd_w(bf16, dx.view(-1, d), o.view(-1, d), dwo)
-    # attention core (Q = q, K = V = kv): dk and dv both flow into kv
-    dqa = torch.empty(B, Lq, d, dtype=dt, device=dev)
-    dk = torch.empty(B, Lk, d, dtype=dt, device=dev)
-    dv = torch.empty(B, Lk, d, dtype=dt, device=dev)
-    ds_prev, dc = _attn_bwd(bf16, do, q, kv, kv, mask, s, s_prev, gc, ds_next, o, stat, n_heads,
-                            dqa, dk, dv, need_dsprev)
-    dq = dq + dqa
-    dkv = dk + dv
-    return [dq, dkv, ds_prev if ds_prev is not None else torch.empty(0, device=dev),
-            dc if dc is not None else torch.empty(0, device=dev), dwo, dwm, dpn]
-
-
-def _block_lite_setup(ctx, inputs, output):
-    q, kv, mask, s_prev, params, H, bf16, emit_s = inputs
-    s = output[1]
-    ctx.save_for_backward(q, kv, mask, s_prev, s if s.numel() else None, *output[2:], *params)
-    ctx.cfg = (H, bf16, len(output) - 2)
-    ctx.set_materialize_grads(False)
-
-
-def _block_lite_backward(ctx, grads):
-    dout, ds_next = grads[0], grads[1]
-    H, bf16, nsaved = ctx.cfg
-    t = ctx.saved_tensors
-    q, kv, mask, s_prev, s = t[:5]
-    saved, params = t[5:5 + nsaved], t[5 + nsaved:]
-    if dout is None:
-        dout = torch.zeros_like(q)
-    d = q.shape[-1]
-    need_dsprev = s_prev is not None and ctx.needs_input_grad[3]
-    dq, dkv, ds_prev, dc, dwo, dwm, dpn = block_lite_bwd_op(dout, ds_next, q, kv, mask, s_prev, s,
-                                                            saved, params, H, bf16, need_dsprev)
-    has_prev = s_prev is not None
-    pgrads = [dwo, dwm, dpn[1:1 + d], dpn[1 + d:], dc if has_prev else None]
-    return (dq, dkv, None, ds_prev if need_dsprev else None, pgrads, None, None, None)
-
-
-block_lite_op.register_autograd(_block_lite_backward, setup_context=_block_lite_setup)
 
 
 # ------------------------------------------------------------------------------------------------

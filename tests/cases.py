@@ -213,3 +213,32 @@ def rel_err(a: torch.Tensor, b: torch.Tensor) -> float:
 
 def golden_path(name: str) -> str:
     return os.path.join(GOLDEN_DIR, name + ".pt")
+
+
+# ------------------------------------------------------------------------------------------
+def trunk_per_block(towers, n_layers: int, keep_all: bool, pool: bool = True):
+    """``blocks.fusion_trunk_multi`` walked chain by chain through each block's own ``forward``
+    (a trunk group of one problem per call): the reference the grouped trunk is compared with."""
+    from mmemo_b200 import blocks, ops
+    segs = []
+    for blks, feats, masks in towers:
+        outs = {"l": [], "v": [], "a": []}
+        for ci, (qm, sm) in enumerate(blocks.CHAINS):
+            q, s, src = feats[qm], None, feats[sm]
+            for i in range(n_layers):
+                q, s = blks[n_layers * ci + i](q, src, src, masks[sm], s,
+                                               emit_scores=i + 1 < n_layers)
+                if keep_all or i + 1 == n_layers:
+                    outs[qm].append(q)
+        segs.append(outs["l"] + outs["a"] + outs["v"])
+    return [ops.pool(t, 3) for t in segs] if pool else segs
+
+
+def use_per_block_trunk(monkeypatch) -> None:
+    """Make every model family run its fusion trunks through ``trunk_per_block``."""
+    import mmemo_b200
+    for mod in (mmemo_b200.cmu_mosei, mmemo_b200.ren_mme, mmemo_b200.robot_demo):
+        monkeypatch.setattr(mod, "fusion_trunk_multi", trunk_per_block)
+    monkeypatch.setattr(mmemo_b200.realformer, "fusion_trunk",
+                        lambda blks, n_layers, feats, masks, keep_all:
+                        trunk_per_block([(blks, feats, masks)], n_layers, keep_all)[0])

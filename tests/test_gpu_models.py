@@ -395,26 +395,25 @@ def test_robot_demo_graphed_ensemble_equals_sequential_members(B):
 
 
 # ------------------------------------------------------------------------------------------------
-# grouped trunk (group_ops.py) vs the per-block path
+# grouped trunk (group_ops.py) vs the blocks one by one
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name", ["realformer_state_transfer", "mosei_concat_trans",
                                   "renmme_base_model", "robot_multi_class"])
 @pytest.mark.parametrize("mode", ["fp32", "bf16"])
-def test_grouped_trunk_equals_per_block_path(name, mode, monkeypatch):
-    """One grouped op per layer over all chains / towers must give what the chain-by-chain blocks
-    give: float32 to summation order (the same launchers run per problem), bf16 to bf16 noise
-    (different kernels: grouped mma.sync attention, grouped tcgen05 GEMMs), for logits AND every
-    parameter / input gradient - this pins the slot layout of the grouped weight-gradient buffer."""
-    from mmemo_b200 import blocks
+def test_grouped_trunk_equals_one_problem_groups(name, mode, monkeypatch):
+    """One grouped op per layer over all chains / towers (9 or 18 problems) must give what the
+    chain-by-chain blocks give (one-problem groups, ``cases.trunk_per_block``): float32 to
+    summation order (the same launchers run per problem), bf16 to bf16 noise (different kernels:
+    grouped mma.sync attention, grouped tcgen05 GEMMs), for logits AND every parameter / input
+    gradient - this pins the slot layout of the grouped weight-gradient buffer."""
     c = cases.CASES[name]
     g = torch.load(cases.golden_path(name))
     model = c.our_model(mmemo_b200).to(DEV).train()
     model.load_state_dict(g["state"])
     b = to_dev(g["batch"])
     with mmemo_b200.precision(mode):
-        monkeypatch.setattr(blocks, "GROUPED_TRUNK", True)
         lg_g, _, gr_g, ig_g = cases.run_module_with_grads(model, c, b, Loss)
-        monkeypatch.setattr(blocks, "GROUPED_TRUNK", False)
+        cases.use_per_block_trunk(monkeypatch)
         lg_b, _, gr_b, ig_b = cases.run_module_with_grads(model, c, b, Loss)
     tol = 2e-5 if mode == "fp32" else 4e-2
     assert rel_err(lg_g.float(), lg_b.float()) < tol

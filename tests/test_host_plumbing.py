@@ -83,37 +83,82 @@ def test_unfused_paths_when_k_is_not_v(stub):
     assert out.shape == (2, 5, 16)
 
 
-def test_trunk_skips_unused_score_writes(stub, monkeypatch):
+def test_trunk_and_single_blocks_skip_unused_score_writes(stub, monkeypatch):
     """The last layer of a chain must not write its scores (nothing consumes them) - in the grouped
-    trunk (one op per layer over the nine chains) and in the per-block path - and the drop-in blocks
-    themselves keep returning scores afterwards (emit_scores is a per-call argument, not module
-    state)."""
-    from mmemo_b200 import blocks, group_ops
-    emitted, groups = [], []
-    real, real_g = ops.block_lite_op, group_ops.trunk_lite_op
-
-    def spy(q, kv, mask, s_prev, params, H, bf16, emit_s):
-        emitted.append(emit_s)
-        return real(q, kv, mask, s_prev, params, H, bf16, emit_s)
+    trunk (one op per layer over the nine chains) and when the blocks are called one by one (one
+    problem per op) - and the drop-in blocks themselves keep returning scores afterwards
+    (emit_scores is a per-call argument, not module state)."""
+    from mmemo_b200 import group_ops
+    groups = []
+    real_g = group_ops.trunk_lite_op
 
     def spy_g(qs, kvs, masks, s_prevs, params, H, bf16, emit_s, drop_p, drop_seed):
         groups.append((len(qs), len(s_prevs), emit_s))
         return real_g(qs, kvs, masks, s_prevs, params, H, bf16, emit_s, drop_p, drop_seed)
 
-    monkeypatch.setattr(ops, "block_lite_op", spy)
     monkeypatch.setattr(group_ops, "trunk_lite_op", spy_g)
     m = mmemo_b200.cmu_mosei.Multi_ATTN(16, 4, 5, 6, 2, 2, 1, l_dim=8, v_dim=6, a_dim=7)
     args = (torch.randn(2, 4, 8), torch.randn(2, 5, 6), torch.randn(2, 6, 7), torch.ones(2, 4),
             torch.ones(2, 5), torch.ones(2, 6))
     out_g = m(*args)
-    assert groups == [(9, 0, True), (9, 9, False)] and emitted == []
-    monkeypatch.setattr(blocks, "GROUPED_TRUNK", False)
+    assert groups == [(9, 0, True), (9, 9, False)]
+    groups.clear()
+    cases.use_per_block_trunk(monkeypatch)
     out_b = m(*args)
-    assert emitted == [True, False] * 9 and out_b.shape == out_g.shape
+    assert groups == [(1, 0, True), (1, 1, False)] * 9 and out_b.shape == out_g.shape
     blk = m.multimodal_blocks[1]                  # a last-layer block, called directly
     x = torch.randn(2, 4, 16)
     out, s = blk(x, x, x, torch.ones(2, 4))
     assert s is not None and s.shape == (2, 2, 4, 4)
+
+
+def test_standalone_blocks_are_one_problem_trunk_groups(stub):
+    """A block called on K = V runs as a trunk group of one problem, on the per-problem attention
+    entry points: a ResidualEncoder forward + backward issues 66 library calls in fp32 and 52 in
+    bf16, and a bf16 lite block casts its two weights in one launch and computes its three weight
+    gradients in one grouped launch (12 calls)."""
+    from mmemo_b200 import synth
+    b = synth.encoder_batch(B=2, L=16, d=32)
+    for mode, n in (("fp32", 66), ("bf16", 52)):
+        stub.clear()
+        ops.clear_shadow_cache()
+        enc = mmemo_b200.ResidualEncoder(32, 4, 3)
+        with mmemo_b200.precision(mode):
+            enc(b["x"], b["mask"]).float().sum().backward()
+        assert len(stub) == n, (mode, stub)
+        assert not any(c.startswith("mmemo_resattn") and "grouped" in c for c in stub), stub
+    stub.clear()
+    blk = mmemo_b200.cmu_mosei.Attention_Block(16, 2, 1)
+    q, kv = torch.randn(2, 5, 16, requires_grad=True), torch.randn(2, 7, 16, requires_grad=True)
+    with mmemo_b200.precision("bf16"):
+        out, s = blk(q, kv, kv, torch.ones(2, 7))
+        out.float().sum().backward()
+    assert len(stub) == 12 and stub.count("mmemo_linear_bwd_w_grouped_bf16") == 1, stub
+    assert s.shape == (2, 2, 5, 7) and q.grad.shape == q.shape and kv.grad.shape == kv.shape
+
+
+@pytest.mark.parametrize("mode", ["fp32", "bf16"])
+def test_standalone_block_dropout_stays_on_the_trunk_op(stub, monkeypatch, mode):
+    """Training dropout of a block called on its own runs inside its trunk op (one op call per
+    forward, one grouped dropout launch per site and direction), not on the per-op path."""
+    from mmemo_b200 import blocks, group_ops
+    n_ops = []
+    for name in ("trunk_full_op", "trunk_lite_op"):
+        monkeypatch.setattr(group_ops, name,
+                            lambda *a, _op=getattr(group_ops, name): n_ops.append(1) or _op(*a))
+    x = torch.randn(2, 5, 16, requires_grad=True)
+    for blk in (blocks.FullAttentionBlock(16, 2, 2, drop=0.1),
+                blocks.LiteAttentionBlock(16, 2, 1, drop=0.1)):
+        blk.train()
+        stub.clear()
+        n_ops.clear()
+        with mmemo_b200.precision(mode):
+            out, _ = blk(x, x, x, torch.ones(2, 5))
+            out.float().sum().backward()
+        assert len(n_ops) == 1, type(blk)
+        sfx = "bf16" if mode == "bf16" else "f32"
+        assert stub.count(f"mmemo_dropout_multi_{sfx}") == 4, stub       # 2 sites x (fwd + bwd)
+        assert not any(c in ("mmemo_dropout_f32", "mmemo_dropout_bf16") for c in stub), stub
 
 
 def test_grouped_trunk_launch_count(stub):
@@ -225,17 +270,17 @@ def test_fused_adamw_host_logic(monkeypatch):
     assert mo.Adam([w1]).param_groups[0]["weight_decay"] == 0.0
 
 
-def test_block_gradient_regions_are_claimed_once_and_forgotten_with_their_reducer():
+def test_block_gradient_regions_are_claimed_once_and_dropped_with_their_reducer():
     """ops.claim_zbufs: the bucket regions of a GROUP of blocks are handed out all-or-nothing, once
-    per backward, only while the reducer has zero-filled them; unregister_grad_dests drops every
-    destination that lives in a removed reducer's buckets."""
+    per backward, only while the reducer has zero-filled them; unregister_zbuf_dests drops every
+    region that lives in a removed reducer's buckets and keeps those of other reducers."""
     k1, k2 = torch.nn.Parameter(torch.zeros(2, 2)), torch.nn.Parameter(torch.zeros(2, 2))
-    other = torch.nn.Parameter(torch.zeros(3))
+    k3, other = torch.nn.Parameter(torch.zeros(2, 2)), torch.nn.Parameter(torch.zeros(3))
     flat_a, flat_b = torch.zeros(256), torch.zeros(256)
     ops.clear_grad_dest()
     ops.register_zbuf_dest(k1, flat_a, 0, 100)
     ops.register_zbuf_dest(k2, flat_a, 128, 100)
-    ops.register_grad_dest(other, flat_b, 32)
+    ops.register_zbuf_dest(k3, flat_b, 32, 100)
     try:
         ops.grad_dest_enabled, ops.grad_dest_zeroed = True, False
         ops.begin_backward()
@@ -249,36 +294,15 @@ def test_block_gradient_regions_are_claimed_once_and_forgotten_with_their_reduce
         assert ops.claim_zbufs([k1, k2], 100) is None                  # second use in this backward
         ops.begin_backward()
         assert ops.claim_zbufs([k2], 100) is not None
-        ops.unregister_grad_dests([flat_a])
+        ops.unregister_zbuf_dests([flat_a])
         ops.begin_backward()
-        assert ops.claim_zbufs([k2], 100) is None and ops._dest(other) is not None
-        ops.unregister_grad_dests([flat_b])
-        assert ops._dest(other) is None
+        assert ops.claim_zbufs([k2], 100) is None
+        assert ops.claim_zbufs([k3], 100)[0].data_ptr() == flat_b[32:].data_ptr()
+        ops.unregister_zbuf_dests([flat_b])
+        ops.begin_backward()
+        assert ops.claim_zbufs([k3], 100) is None
     finally:
         ops.grad_dest_zeroed = False
-        ops.clear_grad_dest()
-        ops.begin_backward()
-
-
-def test_bucket_slot_is_written_once_per_backward():
-    """A weight that is used twice in one forward (shared module) must not have both gradients
-    written into the same data-parallel bucket slot: the second use gets a fresh buffer and
-    autograd sums the two."""
-    w = torch.nn.Parameter(torch.zeros(4, 3))
-    flat = torch.zeros(64)
-    ops.clear_grad_dest()
-    ops.register_grad_dest(w, flat, 16)
-    ops.grad_dest_enabled = True
-    try:
-        ops.begin_backward()
-        buf1, ret1 = ops._wgrad(w, 4, 3)
-        buf2, ret2 = ops._wgrad(w, 4, 3)
-        assert ret1.numel() == 0 and buf1.data_ptr() == flat[16:].data_ptr()      # the slot itself
-        assert ret2.numel() == 12 and buf2.data_ptr() != buf1.data_ptr()          # a fresh buffer
-        ops.begin_backward()                                                        # next step
-        buf3, ret3 = ops._wgrad(w, 4, 3)
-        assert ret3.numel() == 0 and buf3.data_ptr() == buf1.data_ptr()
-    finally:
         ops.clear_grad_dest()
         ops.begin_backward()
 
