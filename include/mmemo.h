@@ -475,32 +475,23 @@ int mmemo_allreduce_sum_f32(void* multicast_ptr, void* const* buffer_ptrs_dev,
  * pointers and element counts).  Replaces nn.utils.clip_grad_norm_(params, CLIP) +
  * optimizer.step(): others/realformer.py:314-315,342 (Adam), cmu-mosei/run.py:368-369,398,
  * Ren-MME/run.py:336-337,379, rencecps/run.py:175-176,202, robot_demo.py:471-472,502 (AdamW).
- *   grad_sqnorm : *sqnorm_out = sum_i |g_i|^2 (device scalar; zeroed by the call)
- *   clip_grads  : g_i *= min(1, max_norm / (sqrt(*sqnorm) + 1e-6))       [torch's formula]
- *   adam_step   : torch.optim.Adam (decoupled=0: g += wd*p) / AdamW (decoupled=1: p *= 1-lr*wd),
- *                 no amsgrad; `step` is the 1-based step count of this update.  With sqnorm != NULL
- *                 the clip coefficient above is applied to the gradients on the fly (grads are
- *                 not modified), so clip + step cost one pass.
- * ------------------------------------------------------------------------------------------- */
-int mmemo_grad_sqnorm_f32(int count, const float* const* grads, const int64_t* numel,
-                          float* sqnorm_out, mmemo_stream_t stream);
-int mmemo_clip_grads_f32(int count, float* const* grads, const int64_t* numel, const float* sqnorm,
-                         float max_norm, mmemo_stream_t stream);
-int mmemo_adam_step_f32(int count, float* const* params, const float* const* grads,
-                        float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
-                        float lr, float beta1, float beta2, float eps, float weight_decay,
-                        int decoupled, int64_t step, const float* sqnorm, float max_norm,
-                        mmemo_stream_t stream);
-/* Several optimizers at once (the k folds of a cross-validation, one model each), one launch per
- * 96 tensors whatever the number of optimizers:
+ * One call may serve several optimizers (the k folds of a cross-validation, one model each), with
+ * one launch per 96 tensors whatever their number; one optimizer is the case of a single slot 0.
  *   grad_sqnorm_multi : sqnorm_out[slot[i]] += |g_i|^2 (float32 device array, zero-initialised by
  *                       the caller): one squared norm per optimizer
- *   adam_step_multi   : adam_step with per-tensor lr[i], step[i] (1-based), weight_decay[i] and
- *                       clip coefficient from sqnorm[slot[i]] (sqnorm nullable: no clipping);
- *                       betas, eps, decoupled and max_norm are shared by the call.
- * All arrays are HOST arrays of length count. */
+ *   clip_grads        : g_i *= min(1, max_norm / (sqrt(*sqnorm) + 1e-6))       [torch's formula]
+ *   adam_step_multi   : torch.optim.Adam (decoupled=0: g += wd*p) / AdamW (decoupled=1:
+ *                       p *= 1-lr*wd), no amsgrad, with per-tensor lr[i], step[i] (the 1-based step
+ *                       count of this update) and weight_decay[i]; betas, eps, decoupled and
+ *                       max_norm are shared by the call.  With sqnorm != NULL the clip coefficient
+ *                       above, from sqnorm[slot[i]], is applied to the gradients on the fly (grads
+ *                       are not modified), so clip + step cost one pass.
+ * All arrays of pointers, counts and per-tensor values are HOST arrays of length count.
+ * ------------------------------------------------------------------------------------------- */
 int mmemo_grad_sqnorm_multi_f32(int count, const float* const* grads, const int64_t* numel,
                                 const int* slot, float* sqnorm_out, mmemo_stream_t stream);
+int mmemo_clip_grads_f32(int count, float* const* grads, const int64_t* numel, const float* sqnorm,
+                         float max_norm, mmemo_stream_t stream);
 int mmemo_adam_step_multi_f32(int count, float* const* params, const float* const* grads,
                               float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
                               const float* lr, const int64_t* step, const float* weight_decay,

@@ -107,10 +107,7 @@ SIGNATURES = {
     "mmemo_circle_loss_bwd": [_vp, _vp, _vp, _vp, _i64, _i64, _vp],
     "mmemo_rdrop_kl_fwd": [_vp, _vp, _i64, _i64, _vp],
     "mmemo_rdrop_kl_bwd": [_vp, _vp, _vp, _i64, _i64, _vp],
-    "mmemo_grad_sqnorm_f32": [_i32, _vp, _vp, _vp, _vp],
     "mmemo_clip_grads_f32": [_i32, _vp, _vp, _vp, _f32, _vp],
-    "mmemo_adam_step_f32": [_i32, _vp, _vp, _vp, _vp, _vp, _f32, _f32, _f32, _f32, _f32, _i32, _i64,
-                            _vp, _f32, _vp],
     "mmemo_grad_sqnorm_multi_f32": [_i32, _vp, _vp, _vp, _vp, _vp],
     "mmemo_adam_step_multi_f32": [_i32] + [_vp] * 9 + [_f32, _f32, _f32, _i32, _vp, _f32, _vp],
     "mmemo_assemble_batch_f32": [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _i32, _f32, _vp],

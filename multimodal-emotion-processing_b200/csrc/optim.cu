@@ -3,9 +3,10 @@
 //   others/realformer.py:314-315,342 (Adam)   cmu-mosei/run.py:368-369,398   Ren-MME/run.py:336-337,379
 //   rencecps/run.py:175-176,202   robot_demo.py:471-472,502 (AdamW)
 // which torch runs as ~5 multi-tensor launches for the norm/clip and ~10 for the update over
-// 100-280 small tensors.  Here: one launch for the global squared norm, one for the update (the
-// clip coefficient is computed on the device from the norm, so there is no host sync), per chunk
-// of 96 tensors.  HBM-bound: reads p, g, m, v and writes p, m, v once (28 B per parameter).
+// 100-280 small tensors.  Here, for one optimizer or for the k fold optimizers of a cross-validation
+// at once: one launch for the squared norms (one per optimizer), one for the update (the clip
+// coefficient is computed on the device from the norm, so there is no host sync), per chunk of 96
+// tensors.  HBM-bound: reads p, g, m, v and writes p, m, v once (28 B per parameter).
 #include "common.cuh"
 
 namespace {
@@ -137,13 +138,8 @@ __device__ __forceinline__ void adam_tensor(const AdamTable& t, int which, const
   }
 }
 
-__global__ void __launch_bounds__(256)
-adam_multi_kernel(AdamTable t, AdamHyper h, const float* __restrict__ sqnorm) {
-  adam_tensor(t, blockIdx.y, h, clip_coef(sqnorm, h.max_norm));
-}
-
-// Several optimizers (the k folds of a cross-validation) in one launch: each tensor carries its own
-// lr, weight decay, bias corrections (its own step count) and the norm slot of its optimizer.
+// Each tensor carries its own lr, weight decay, bias corrections (its own step count) and the norm
+// slot of its optimizer, so one launch serves any number of optimizers (e.g. the k folds).
 struct MemberHyper {
   float lr[OPT_MAXT], weight_decay[OPT_MAXT], step_size[OPT_MAXT], inv_bc2_sqrt[OPT_MAXT];
   int slot[OPT_MAXT];
@@ -169,27 +165,6 @@ unsigned grid_x(long long nmax) {
 }  // namespace
 
 extern "C" {
-
-int mmemo_grad_sqnorm_f32(int count, const float* const* grads, const int64_t* numel,
-                          float* sqnorm_out, mmemo_stream_t s) {
-  MM_REQUIRE(count >= 0 && sqnorm_out && (count == 0 || (grads && numel)));
-  cudaStream_t st = mm_stream(s);
-  MM_CUDA_OK(cudaMemsetAsync(sqnorm_out, 0, sizeof(float), st));
-  for (int base = 0; base < count; base += OPT_MAXT) {
-    NormTable t = {};
-    long long nmax = 0;
-    t.count = count - base < OPT_MAXT ? count - base : OPT_MAXT;
-    for (int i = 0; i < t.count; ++i) {
-      MM_REQUIRE(grads[base + i] && numel[base + i] >= 0);
-      t.g[i] = grads[base + i];
-      t.n[i] = numel[base + i];
-      nmax = t.n[i] > nmax ? t.n[i] : nmax;
-    }
-    sqnorm_multi_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, sqnorm_out);
-    MM_LAUNCH_OK();
-  }
-  return MMEMO_OK;
-}
 
 int mmemo_grad_sqnorm_multi_f32(int count, const float* const* grads, const int64_t* numel,
                                 const int* slot, float* sqnorm_out, mmemo_stream_t s) {
@@ -232,43 +207,6 @@ int mmemo_clip_grads_f32(int count, float* const* grads, const int64_t* numel, c
   return MMEMO_OK;
 }
 
-int mmemo_adam_step_f32(int count, float* const* params, const float* const* grads,
-                        float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
-                        float lr, float beta1, float beta2, float eps, float weight_decay,
-                        int decoupled, int64_t step, const float* sqnorm, float max_norm,
-                        mmemo_stream_t s) {
-  MM_REQUIRE(count >= 0 && step >= 1 && (count == 0 || (params && grads && exp_avg && exp_avg_sq && numel)));
-  MM_REQUIRE(!sqnorm || max_norm > 0.f);
-  cudaStream_t st = mm_stream(s);
-  AdamHyper h = {};
-  h.lr = lr; h.beta1 = beta1; h.beta2 = beta2; h.eps = eps; h.weight_decay = weight_decay;
-  // bias corrections in double like torch's Python scalars (1 - beta ** step)
-  const double bc1 = 1.0 - pow((double)beta1, (double)step);
-  const double bc2 = 1.0 - pow((double)beta2, (double)step);
-  h.step_size = (float)((double)lr / bc1);
-  h.inv_bc2_sqrt = (float)(1.0 / sqrt(bc2));
-  h.max_norm = max_norm;
-  h.decoupled = decoupled;
-  for (int base = 0; base < count; base += OPT_MAXT) {
-    AdamTable t = {};
-    long long nmax = 0;
-    t.count = count - base < OPT_MAXT ? count - base : OPT_MAXT;
-    for (int i = 0; i < t.count; ++i) {
-      const int j = base + i;
-      MM_REQUIRE(params[j] && grads[j] && exp_avg[j] && exp_avg_sq[j] && numel[j] >= 0);
-      t.p[i] = params[j];
-      t.g[i] = const_cast<float*>(grads[j]);
-      t.m[i] = exp_avg[j];
-      t.v[i] = exp_avg_sq[j];
-      t.n[i] = numel[j];
-      nmax = t.n[i] > nmax ? t.n[i] : nmax;
-    }
-    adam_multi_kernel<<<dim3(grid_x(nmax), (unsigned)t.count), 256, 0, st>>>(t, h, sqnorm);
-    MM_LAUNCH_OK();
-  }
-  return MMEMO_OK;
-}
-
 int mmemo_adam_step_multi_f32(int count, float* const* params, const float* const* grads,
                               float* const* exp_avg, float* const* exp_avg_sq, const int64_t* numel,
                               const float* lr, const int64_t* step, const float* weight_decay,
@@ -299,7 +237,7 @@ int mmemo_adam_step_multi_f32(int count, float* const* params, const float* cons
       t.v[i] = exp_avg_sq[j];
       t.n[i] = numel[j];
       nmax = t.n[i] > nmax ? t.n[i] : nmax;
-      // the same double-precision bias corrections as mmemo_adam_step_f32
+      // bias corrections in double like torch's Python scalars (1 - beta ** step)
       const double bc1 = 1.0 - pow((double)beta1, (double)step[j]);
       const double bc2 = 1.0 - pow((double)beta2, (double)step[j]);
       mh.lr[i] = lr[j];

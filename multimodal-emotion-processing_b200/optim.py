@@ -7,7 +7,8 @@ every reference training loop,
 ``Adam`` / ``AdamW`` keep torch.optim's constructor arguments, ``param_groups`` (so
 ``ReduceLROnPlateau`` keeps working, others/realformer.py:343) and ``state_dict`` layout
 (``step``, ``exp_avg``, ``exp_avg_sq``), and run the whole update as one libmmemo launch per 96
-tensors.  Two ways to clip:
+tensors.  ``step_group`` steps several of them (the k folds of a cross-validation) in the same
+launches; ``step()`` is ``step_group`` of one optimizer.  Two ways to clip:
 
 * drop-in: keep the reference's two calls, with ``clip_grad_norm_`` from this module (two launches:
   squared norm, scale; returns the total norm like torch's);
@@ -28,9 +29,6 @@ from torch import Tensor
 
 from . import ops
 
-_CHUNK = 96      # tensors per launch of the multi-tensor kernels (csrc/optim.cu OPT_MAXT)
-
-
 def _ptrs(ts: List[Tensor]):
     return (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
 
@@ -46,12 +44,16 @@ def _check(ts: Iterable[Tensor], what: str) -> None:
                                "(no CPU fallback)")
 
 
+def _arr(ctype, vals):
+    return (ctype * len(vals))(*vals)
+
+
 def grad_sqnorm(grads: List[Tensor]) -> Tensor:
     """Device scalar  sum_i |g_i|^2  in one launch (per 96 tensors)."""
     _check(grads, "gradients")
-    out = torch.empty(1, dtype=torch.float32, device=grads[0].device)
-    ops._call("mmemo_grad_sqnorm_f32", len(grads), _ptrs(grads), _ns(grads), out.data_ptr(),
-              ops._stream())
+    out = torch.zeros(1, dtype=torch.float32, device=grads[0].device)
+    ops._call("mmemo_grad_sqnorm_multi_f32", len(grads), _ptrs(grads), _ns(grads),
+              _arr(C.c_int, [0] * len(grads)), out.data_ptr(), ops._stream())
     return out
 
 
@@ -111,34 +113,7 @@ class _FusedAdam(torch.optim.Optimizer):
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
-        groups = self._collect()
-        if not groups:
-            return loss
-        sq = None
-        if self.max_grad_norm is not None:     # global norm over every group, like the reference
-            sq = grad_sqnorm([g for _, _, gs in groups for g in gs])
-        for group, ps, gs in groups:
-            # parameters that joined later (frozen before) carry their own step count
-            by_step = {}
-            for i, p in enumerate(ps):
-                by_step.setdefault(int(self.state[p]["step"]), []).append(i)
-            for t, sel in sorted(by_step.items()):
-                pp = [ps[i] for i in sel]
-                gg = [gs[i] for i in sel]
-                mm = [self.state[p]["exp_avg"] for p in pp]
-                vv = [self.state[p]["exp_avg_sq"] for p in pp]
-                b1, b2 = group["betas"]
-                ops._call("mmemo_adam_step_f32", len(pp), _ptrs(pp), _ptrs(gg), _ptrs(mm),
-                          _ptrs(vv), _ns(pp), float(group["lr"]), float(b1), float(b2),
-                          float(group["eps"]), float(group["weight_decay"]),
-                          int(self._decoupled), t + 1, None if sq is None else sq.data_ptr(),
-                          float(self.max_grad_norm or 0.0), ops._stream())
-                for p in pp:
-                    self.state[p]["step"] += 1
-                # the launch wrote the parameters through raw pointers: bump their version counters
-                # so that everything keyed on them (the bf16 weight shadows of ops.shadow_bf16,
-                # autograd's saved-tensor checks) sees the update like after an in-place torch op
-                torch._C._increment_version(pp)
+        step_group([self])
         return loss
 
 
@@ -158,21 +133,18 @@ class AdamW(_FusedAdam):
         super().__init__(params, lr, betas, eps, weight_decay, amsgrad, max_grad_norm)
 
 
-def _arr(ctype, vals):
-    return (ctype * len(vals))(*vals)
-
-
 @torch.no_grad()
 def step_group(optimizers) -> None:
-    """``for opt in optimizers: opt.step()`` for several ``Adam`` / ``AdamW`` instances (the k folds
-    of a cross-validation, one model each) in one launch per 96 tensors, whatever their number.
+    """``for opt in optimizers: opt.step()`` for one or several ``Adam`` / ``AdamW`` instances (the
+    k folds of a cross-validation, one model each) in one launch per 96 tensors, whatever their
+    number.  ``step()`` itself is ``step_group([self])``.
 
     Each optimizer keeps its own ``param_groups``, ``state`` and ``state_dict`` and ends up exactly
     as if it had been stepped alone: its own lr (e.g. set by its own ``ReduceLROnPlateau``), weight
-    decay and step counts, and with ``max_grad_norm`` its gradients clipped by the norm over its own
-    parameters (one squared norm per optimizer, computed first, one launch per 96 tensors).
-    Optimizers that differ in class, ``betas``, ``eps`` or ``max_grad_norm`` are updated by one call
-    per such combination."""
+    decay and per-tensor step counts (a parameter that starts receiving gradients later has its own
+    bias corrections), and with ``max_grad_norm`` its gradients clipped by the norm over all of its
+    param groups (one squared norm per optimizer, computed first).  That is one library call for the
+    norms and one update call per combination of class, ``betas``, ``eps`` and ``max_grad_norm``."""
     opts = list(optimizers)
     for o in opts:
         if not isinstance(o, _FusedAdam):
@@ -187,10 +159,8 @@ def step_group(optimizers) -> None:
                 norm_slot += [k] * len(gs)
     if norm_g:
         sq = torch.zeros(len(opts), dtype=torch.float32, device=norm_g[0].device)
-        for i in range(0, len(norm_g), _CHUNK):
-            gs, sl = norm_g[i:i + _CHUNK], norm_slot[i:i + _CHUNK]
-            ops._call("mmemo_grad_sqnorm_multi_f32", len(gs), _ptrs(gs), _ns(gs), _arr(C.c_int, sl),
-                      sq.data_ptr(), ops._stream())
+        ops._call("mmemo_grad_sqnorm_multi_f32", len(norm_g), _ptrs(norm_g), _ns(norm_g),
+                  _arr(C.c_int, norm_slot), sq.data_ptr(), ops._stream())
     # [(param, grad, optimizer index, param_group)] per combination of the shared hyper-parameters
     calls = {}
     for k, (o, groups) in enumerate(zip(opts, collected)):
@@ -198,20 +168,20 @@ def step_group(optimizers) -> None:
             key = (o._decoupled, tuple(group["betas"]), float(group["eps"]), o.max_grad_norm)
             calls.setdefault(key, []).extend((p, g, k, group) for p, g in zip(ps, gs))
     for (decoupled, (b1, b2), eps, max_norm), items in calls.items():
-        for i in range(0, len(items), _CHUNK):
-            part = items[i:i + _CHUNK]
-            pp = [it[0] for it in part]
-            st = [opts[it[2]].state[it[0]] for it in part]
-            ops._call("mmemo_adam_step_multi_f32", len(part), _ptrs(pp), _ptrs([it[1] for it in part]),
-                      _ptrs([s["exp_avg"] for s in st]), _ptrs([s["exp_avg_sq"] for s in st]),
-                      _ns(pp), _arr(C.c_float, [float(it[3]["lr"]) for it in part]),
-                      _arr(C.c_int64, [int(s["step"]) + 1 for s in st]),
-                      _arr(C.c_float, [float(it[3]["weight_decay"]) for it in part]),
-                      _arr(C.c_int, [it[2] for it in part]), float(b1), float(b2), eps,
-                      int(decoupled), None if sq is None or max_norm is None else sq.data_ptr(),
-                      float(max_norm or 0.0), ops._stream())
-        for p, _, k, _ in items:
-            opts[k].state[p]["step"] += 1
-        # (see _FusedAdam.step: the launch wrote the parameters through raw pointers)
-        torch._C._increment_version([it[0] for it in items])
+        pp = [it[0] for it in items]
+        st = [opts[it[2]].state[it[0]] for it in items]
+        ops._call("mmemo_adam_step_multi_f32", len(items), _ptrs(pp), _ptrs([it[1] for it in items]),
+                  _ptrs([s["exp_avg"] for s in st]), _ptrs([s["exp_avg_sq"] for s in st]),
+                  _ns(pp), _arr(C.c_float, [float(it[3]["lr"]) for it in items]),
+                  _arr(C.c_int64, [int(s["step"]) + 1 for s in st]),
+                  _arr(C.c_float, [float(it[3]["weight_decay"]) for it in items]),
+                  _arr(C.c_int, [it[2] for it in items]), float(b1), float(b2), eps,
+                  int(decoupled), None if sq is None or max_norm is None else sq.data_ptr(),
+                  float(max_norm or 0.0), ops._stream())
+        for s in st:
+            s["step"] += 1
+        # the launch wrote the parameters through raw pointers: bump their version counters so
+        # that everything keyed on them (the bf16 weight shadows of ops.shadow_bf16, autograd's
+        # saved-tensor checks) sees the update like after an in-place torch op
+        torch._C._increment_version(pp)
 

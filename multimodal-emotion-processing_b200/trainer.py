@@ -3,8 +3,8 @@ fixed for current torch:  ``run()`` = Adam/AdamW + ``ReduceLROnPlateau(factor=0.
 the validation loss + best-checkpoint saving + early stop after 4 epochs without a new best
 (others/realformer.py:338-363, cmu-mosei/run.py:394-419, Ren-MME/run.py:370-401,
 rencecps/run.py:198-223, robot_demo.py:498-523), and the contiguous k-fold split the scripts spell
-out by hand (others/realformer.py:365-389), which runs the folds one after the other;
-``fit_folds`` trains them together instead.
+out by hand (others/realformer.py:365-389).  The reference runs the folds one after the other;
+``fit_folds`` trains them together, and ``fit`` is ``fit_folds`` with one fold.
 
 Differences from the reference, all outside the hot path:
 * ``ReduceLROnPlateau(verbose=True)`` raises ``TypeError`` on torch >= 2.7; the lr changes are
@@ -39,35 +39,6 @@ def kfold_splits(names: Sequence, k: int = 5) -> List[Tuple[list, list]]:
         hi = int(n * ((i + 1) / k)) if i + 1 < k else n
         out.append((names[:lo] + names[hi:], names[lo:hi]))
     return out
-
-
-def train_epoch(model: torch.nn.Module, iterator: Iterable, optimizer: torch.optim.Optimizer,
-                train_step: Callable, clip: Optional[float] = 1.0) -> float:
-    """others/realformer.py:300-318: mean of the per-batch losses.  ``train_step(model, batch)``
-    returns the scalar loss tensor; ``clip=None`` when the optimizer clips itself."""
-    model.train()
-    total, count = 0.0, 0
-    for batch in iterator:
-        count += 1
-        optimizer.zero_grad()
-        loss = train_step(model, batch)
-        loss.backward()
-        if clip is not None:
-            torch.nn.utils.clip_grad_norm_(model.parameters(), clip)
-        optimizer.step()
-        total += loss.item()
-    return total / max(count, 1)
-
-
-def valid_epoch(model: torch.nn.Module, iterator: Iterable, valid_step: Callable) -> float:
-    """others/realformer.py:320-336."""
-    model.eval()
-    total, count = 0.0, 0
-    with torch.no_grad():
-        for batch in iterator:
-            count += 1
-            total += float(valid_step(model, batch))
-    return total / max(count, 1)
 
 
 def checkpoint_name(name: str, valid_loss: float) -> str:
@@ -128,16 +99,12 @@ def fit(model: torch.nn.Module, optimizer: torch.optim.Optimizer,
     """The reference's ``run()``.  Returns ``{"train": [...], "valid": [...], "best": path | None,
     "lrs": [...]}``.  A new iterator is built every epoch (the reference reshuffles in
     ``data_loader``).  ``sched_patience`` is 2 in realformer and 1 in the other scripts."""
-    valid_step = valid_step or (lambda m, b: train_step(m, b))
-    run = _Run(optimizer, name, log_dir, sched_patience, sched_factor, stop_after, writer, log)
-    for epoch in range(epochs):
-        log(f"Epoch: {epoch + 1}")
-        tr = train_epoch(model, make_train_iter(), optimizer, train_step, clip)
-        va = valid_epoch(model, make_valid_iter(), valid_step)
-        run.end_epoch(model, epoch, tr, va)
-        if run.done:
-            break
-    return run.hist
+    valid_step = valid_step or train_step
+    return fit_folds([model], [optimizer], [make_train_iter], [make_valid_iter],
+                     lambda ms, bs: [train_step(ms[0], bs[0])],
+                     lambda ms, bs: [valid_step(ms[0], bs[0])], epochs=epochs, names=[name],
+                     log_dir=log_dir, clip=clip, sched_patience=sched_patience,
+                     sched_factor=sched_factor, stop_after=stop_after, writer=writer, log=log)[0]
 
 
 def _lockstep(iterables: Dict[int, Iterable]):
@@ -168,7 +135,10 @@ def _train_epoch_group(models, optimizers, iterables, train_step_group, clip) ->
         if len(losses) != len(ks):
             raise ValueError(f"train_step_group returned {len(losses)} losses for {len(ks)} folds")
         # the folds share no parameters: each receives exactly the gradients of its own loss
-        sum(losses).backward()
+        total_loss = losses[0]
+        for loss in losses[1:]:
+            total_loss = total_loss + loss
+        total_loss.backward()
         if clip is not None:
             for k in ks:
                 torch.nn.utils.clip_grad_norm_(models[k].parameters(), clip)

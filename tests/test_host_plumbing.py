@@ -230,9 +230,10 @@ def test_grad_reducer_on_encoder_skips_undefined_grads(stub):
         dist.destroy_process_group()
 
 
-def test_fused_adamw_host_logic(monkeypatch):
-    """optim.AdamW: torch.optim-compatible param_groups / state layout, one launch per step-count
-    group, global norm over all groups, empty groups skipped (Ren-MME/run.py:376-379)."""
+def test_fused_adamw_makes_one_norm_and_one_update_call(monkeypatch):
+    """optim.AdamW: torch.optim-compatible param_groups / state layout, one norm and one update call
+    per step with per-tensor step counts, global norm over all groups, empty groups skipped
+    (Ren-MME/run.py:376-379)."""
     from mmemo_b200 import optim as mo
     calls = []
     monkeypatch.setattr(ops, "_call", lambda name, *a: calls.append((name, a)))
@@ -248,23 +249,27 @@ def test_fused_adamw_host_logic(monkeypatch):
     w1.grad, w2.grad = torch.ones_like(w1), torch.ones_like(w2)
     opt.step()
     names = [n for n, _ in calls]
-    assert names == ["mmemo_grad_sqnorm_f32", "mmemo_adam_step_f32"]
+    assert names == ["mmemo_grad_sqnorm_multi_f32", "mmemo_adam_step_multi_f32"]
+    assert calls[0][1][0] == 2 and list(calls[0][1][3]) == [0, 0]     # both norms into slot 0
     a = calls[1][1]
-    assert a[0] == 2 and a[11] == 1 and a[12] == 1        # two tensors, decoupled, step 1
-    assert a[13] is not None and a[14] == 1.0             # fused clipping
+    assert a[0] == 2 and a[13] == 1 and list(a[7]) == [1, 1]   # two tensors, decoupled, step 1
+    assert a[14] == calls[0][1][4] and a[15] == 1.0             # fused clipping by that norm
     assert set(opt.state[w1]) == {"step", "exp_avg", "exp_avg_sq"} and frozen not in opt.state
     # a parameter that starts receiving gradients later gets its own bias-correction step
     calls.clear()
     frozen.grad = torch.ones_like(frozen)
     opt.step()
-    steps = sorted(a[12] for n, a in calls if n == "mmemo_adam_step_f32")
-    assert steps == [1, 2]
+    names = [n for n, _ in calls]
+    assert names == ["mmemo_grad_sqnorm_multi_f32", "mmemo_adam_step_multi_f32"]
+    a = calls[1][1]
+    assert list(a[7])[:a[0]] == [2, 2, 1]
     assert float(opt.state[w1]["step"]) == 2 and float(opt.state[frozen]["step"]) == 1
     # ReduceLROnPlateau-style lr edits are picked up
     opt.param_groups[0]["lr"] = 5e-4
     calls.clear()
     opt.step()
-    assert all(abs(a[6] - 5e-4) < 1e-12 for n, a in calls if n == "mmemo_adam_step_f32")
+    a = calls[1][1]
+    assert a[0] == 3 and list(a[6])[:a[0]] == pytest.approx([5e-4] * 3)     # float32 per tensor
     with pytest.raises(ValueError):
         mo.Adam([w1], amsgrad=True)
     assert mo.Adam([w1]).param_groups[0]["weight_decay"] == 0.0

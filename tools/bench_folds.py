@@ -1,7 +1,8 @@
 """Not a test: the optimizer step of k-fold training on one GPU — K separate ``optimizer.step()``
 calls (the reference's folds, one after the other) against one ``optim.step_group`` over the K
 fold optimizers — for the models of cfg 1a, 1b and 4 (``benchlib.WORKLOADS``), K in {1, 2, 3, 5},
-fused AdamW with clipping (``max_grad_norm=1.0``) as in the reference loops.
+fused AdamW with clipping (``max_grad_norm=1.0``) as in the reference loops.  ``step()`` is
+``step_group`` of one optimizer, so the comparison is K library-call pairs against one.
 
 Device events around 50 steps after 10 warm-up steps; library calls per step from
 ``ops.launch_count``; CUDA kernels per step from ``torch.profiler`` in a separate untimed pass.
