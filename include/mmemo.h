@@ -45,7 +45,9 @@ const char* mmemo_last_error(void); /* host string describing the last MMEMO_ERR
 /* Per-stream launch settings.  Every entry point below looks them up by the `stream` argument of
  * the call (defaults for a stream that was never configured: no workspace, all SMs, PDL on).
  *  - workspace: scratch for split-K partial tiles of the tcgen05 GEMM when the output is bf16 or
- *    carries a bias (fp32 weight gradients are summed by TMA reduce-add and need none).  The
+ *    carries a bias (fp32 weight gradients are summed by TMA reduce-add and need none), and of the
+ *    SIMT GEMM (float32 outputs: the float32 parity mode and the float32 heads), which sums its
+ *    partial tiles in a fixed order, so its results do not depend on CTA scheduling.  The
  *    library never allocates: the host attaches one device buffer to each stream it launches on;
  *    launches of one stream are ordered, so they can share it, and two streams never share one.
  *    A GEMM that would need more than `bytes` simply does not split.
@@ -121,6 +123,25 @@ int mmemo_linear_bwd_w_grouped_bf16(int n, const void* const* dy, const int64_t*
                                     const void* const* x, const int64_t* ldx, float* const* dw,
                                     const int64_t* lddw, const int64_t* M, const int64_t* N,
                                     const int64_t* K, int accumulate, mmemo_stream_t stream);
+/* Grouped float32 variants: n >= 0 problems (the float32 head linears of k folds), one SIMT launch
+ * per 48 problems (more only when their split-K scratch exceeds the stream's workspace).  Each
+ * problem splits K exactly as mmemo_linear_*_f32 would split it alone, so y, dx and dw are the
+ * same bits as mmemo_linear_*_f32 on that problem.  bias / dbias (nullable arrays and
+ * entries): bias[i] (N) added; dbias[i] (N) = column sums of dy[i] (overwritten; the dbias problems
+ * are GEMMs of their own, so with n > 24 dbias entries bwd_w takes one launch more). */
+int mmemo_linear_fwd_grouped_f32(int n, const float* const* x, const int64_t* ldx,
+                                 const float* const* w, const int64_t* ldw,
+                                 const float* const* bias, float* const* y, const int64_t* ldy,
+                                 const int64_t* M, const int64_t* N, const int64_t* K,
+                                 mmemo_stream_t stream);
+int mmemo_linear_bwd_x_grouped_f32(int n, const float* const* dy, const int64_t* lddy,
+                                   const float* const* w, const int64_t* ldw, float* const* dx,
+                                   const int64_t* lddx, const int64_t* M, const int64_t* N,
+                                   const int64_t* K, mmemo_stream_t stream);
+int mmemo_linear_bwd_w_grouped_f32(int n, const float* const* dy, const int64_t* lddy,
+                                   const float* const* x, const int64_t* ldx, float* const* dw,
+                                   const int64_t* lddw, float* const* dbias, const int64_t* M,
+                                   const int64_t* N, const int64_t* K, mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Fused residual-attention core (kernel a / a').  Replaces
@@ -360,6 +381,27 @@ int mmemo_pool_fwd_multi_bf16(int n_towers, const void* const* seg_ptrs, const i
                               int n_groups, int n_slots, int64_t B, int64_t d, float* const* out,
                               mmemo_stream_t stream);
 
+/* Training form for the k folds of folds.py: n_towers towers with their OWN batch sizes B[t] (HOST
+ * array), and each tower's argmax (B[t], n_slots*d) int32 in argmax[t] (HOST array).  out[t] and
+ * argmax[t] are bitwise what mmemo_pool_fwd_* writes for tower t. */
+int mmemo_pool_fwd_multi_arg_f32(int n_towers, const void* const* seg_ptrs,
+                                 const int64_t* group_len, int n_groups, int n_slots,
+                                 const int64_t* B, int64_t d, float* const* out,
+                                 int32_t* const* argmax, mmemo_stream_t stream);
+int mmemo_pool_fwd_multi_arg_bf16(int n_towers, const void* const* seg_ptrs,
+                                  const int64_t* group_len, int n_groups, int n_slots,
+                                  const int64_t* B, int64_t d, float* const* out,
+                                  int32_t* const* argmax, mmemo_stream_t stream);
+/* mmemo_pool_bwd_* of every tower in one launch per 16 towers: dout[t], argmax[t] and the
+ * dseg_ptrs of tower t ([n_towers][n_groups * n_slots], HOST arrays) with batch size B[t].  Each
+ * tower's segment gradients are bitwise those of mmemo_pool_bwd_*. */
+int mmemo_pool_bwd_multi_f32(int n_towers, const float* const* dout, int32_t* const* argmax,
+                             void* const* dseg_ptrs, const int64_t* group_len, int n_groups,
+                             int n_slots, const int64_t* B, int64_t d, mmemo_stream_t stream);
+int mmemo_pool_bwd_multi_bf16(int n_towers, const float* const* dout, int32_t* const* argmax,
+                              void* const* dseg_ptrs, const int64_t* group_len, int n_groups,
+                              int n_slots, const int64_t* B, int64_t d, mmemo_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Heads and losses (float32 only; O(B*C) work).
  * state_transfer: others/realformer.py:274-286.  feats (B,P,2C) = [o | g]; out (B,P,C).
@@ -390,6 +432,50 @@ int mmemo_rdrop_kl_fwd(const float* logits, float* out, int64_t B, int64_t C,
                        mmemo_stream_t stream);
 int mmemo_rdrop_kl_bwd(const float* dout, const float* logits, float* dlogits, int64_t B, int64_t C,
                        mmemo_stream_t stream);
+
+/* The same heads and losses for n >= 0 members (the k folds trained together by folds.py), one
+ * launch per 32 members.  Every pointer argument is a HOST array with one device pointer per member
+ * (entries of dtrans / dgamma / dbeta / dw / dbias / weights may be null: not computed / no
+ * weights); B[i] / R[i] is member i's batch size / row count; P and C are shared.  Each member's
+ * forward output is bitwise that of the per-model entry point; parameter gradients are summed with
+ * float atomics within a member (as there) and never across members.
+ * circle_loss_fwd_multi: loss[i] (one float) = mean over the R[i] rows of circle_loss (times
+ *   weights[i][r] when given): (multi_circle_loss(logits, labels) [* weights]).mean().
+ * circle_loss_bwd_multi: its gradient for d loss[i] = dloss[i][0].
+ * rdrop_kl_*_multi: mmemo_rdrop_kl_* per member (B[i] even, >= 2). */
+int mmemo_state_transfer_fwd_multi(int n, const float* const* feats, const float* const* trans,
+                                   float* const* out, const int64_t* B, int64_t P, int64_t C,
+                                   mmemo_stream_t stream);
+int mmemo_state_transfer_bwd_multi(int n, const float* const* dout, const float* const* feats,
+                                   const float* const* trans, const float* const* out,
+                                   float* const* dfeats, float* const* dtrans, const int64_t* B,
+                                   int64_t P, int64_t C, mmemo_stream_t stream);
+int mmemo_bilinear_head_fwd_multi(int n, const float* const* this_feat,
+                                  const float* const* last_feat, const float* const* trans,
+                                  const float* const* gamma, const float* const* beta,
+                                  const float* const* w, const float* const* bias,
+                                  float* const* out, float* const* z, const int64_t* B, int64_t C,
+                                  float eps, mmemo_stream_t stream);
+int mmemo_bilinear_head_bwd_multi(int n, const float* const* dout, const float* const* this_feat,
+                                  const float* const* last_feat, const float* const* trans,
+                                  const float* const* gamma, const float* const* beta,
+                                  const float* const* w, const float* const* z,
+                                  float* const* dthis, float* const* dlast, float* const* dtrans,
+                                  float* const* dgamma, float* const* dbeta, float* const* dw,
+                                  float* const* dbias, const int64_t* B, int64_t C, float eps,
+                                  mmemo_stream_t stream);
+int mmemo_circle_loss_fwd_multi(int n, const float* const* logits, const float* const* labels,
+                                const float* const* weights, const int64_t* R, int64_t C,
+                                float* const* loss, mmemo_stream_t stream);
+int mmemo_circle_loss_bwd_multi(int n, const float* const* dloss, const float* const* logits,
+                                const float* const* labels, const float* const* weights,
+                                float* const* dlogits, const int64_t* R, int64_t C,
+                                mmemo_stream_t stream);
+int mmemo_rdrop_kl_fwd_multi(int n, const float* const* logits, const int64_t* B, int64_t C,
+                             float* const* out, mmemo_stream_t stream);
+int mmemo_rdrop_kl_bwd_multi(int n, const float* const* dout, const float* const* logits,
+                             float* const* dlogits, const int64_t* B, int64_t C,
+                             mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Ensemble head (inference, float32): y = (out_1 + ... + out_K) / K over K >= 1 members, summed as

@@ -10,4 +10,5 @@ __version__ = "0.1.0"
 
 from .blocks import get_precision, precision, set_precision  # noqa: E402,F401
 from . import batching, cmu_mosei, ensemble, optim, realformer, ren_mme, rencecps, robot_demo, synth, trainer  # noqa: E402,F401
+from . import folds  # noqa: E402,F401
 from .encoder import ResidualEncoder  # noqa: E402,F401

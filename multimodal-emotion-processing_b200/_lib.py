@@ -29,6 +29,8 @@ _ROWSUM = [_vp, _i64, _vp, _i64, _i64, _i64, _vp]
 _POOL_FWD = [_vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp, _vp]
 _POOL_BWD = [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _i64, _vp]
 _POOL_FWD_MULTI = [_i32, _vp, _vp, _i32, _i32, _i64, _i64, _vp, _vp]
+_POOL_MULTI_ARG = [_i32, _vp, _vp, _i32, _i32, _vp, _i64, _vp, _vp, _vp]
+_POOL_BWD_MULTI = [_i32, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i64, _vp]
 _DROPOUT = [_vp, _vp, _i64, _f32, _u64, _vp]
 _FOLD_UQ = [_vp, _i64, _i64, _i64] + [_vp] * 6 + [_vp]
 
@@ -66,6 +68,9 @@ SIGNATURES = {
     "mmemo_linear_fwd_grouped_bf16": [_i32] + [_vp] * 15 + [_vp],
     "mmemo_linear_bwd_x_grouped_bf16": [_i32] + [_vp] * 12 + [_vp],
     "mmemo_linear_bwd_w_grouped_bf16": [_i32] + [_vp] * 9 + [_i32, _vp],
+    "mmemo_linear_fwd_grouped_f32": [_i32] + [_vp] * 10 + [_vp],
+    "mmemo_linear_bwd_x_grouped_f32": [_i32] + [_vp] * 9 + [_vp],
+    "mmemo_linear_bwd_w_grouped_f32": [_i32] + [_vp] * 10 + [_vp],
     "mmemo_resattn_fwd_f32": _ATTN_FWD, "mmemo_resattn_fwd_bf16": _ATTN_FWD,
     "mmemo_resattn_bwd_f32": _ATTN_BWD, "mmemo_resattn_bwd_bf16": _ATTN_BWD,
     "mmemo_resattn_fwd_grouped_bf16": [_i32, _vp, _vp],
@@ -95,6 +100,8 @@ SIGNATURES = {
     "mmemo_pool_fwd_f32": _POOL_FWD, "mmemo_pool_fwd_bf16": _POOL_FWD,
     "mmemo_pool_bwd_f32": _POOL_BWD, "mmemo_pool_bwd_bf16": _POOL_BWD,
     "mmemo_pool_fwd_multi_f32": _POOL_FWD_MULTI, "mmemo_pool_fwd_multi_bf16": _POOL_FWD_MULTI,
+    "mmemo_pool_fwd_multi_arg_f32": _POOL_MULTI_ARG, "mmemo_pool_fwd_multi_arg_bf16": _POOL_MULTI_ARG,
+    "mmemo_pool_bwd_multi_f32": _POOL_BWD_MULTI, "mmemo_pool_bwd_multi_bf16": _POOL_BWD_MULTI,
     "mmemo_ensemble_head_fwd": [_i32, _i32, _vp, _i64, _i64, _i64, _i64, _i64, _f32, _vp, _vp],
     "mmemo_ensemble_head_fwd_members": [_i32, _i32, _vp, _i64, _i64, _i64, _i64, _i64, _f32, _vp,
                                         _vp, _vp],
@@ -107,6 +114,14 @@ SIGNATURES = {
     "mmemo_circle_loss_bwd": [_vp, _vp, _vp, _vp, _i64, _i64, _vp],
     "mmemo_rdrop_kl_fwd": [_vp, _vp, _i64, _i64, _vp],
     "mmemo_rdrop_kl_bwd": [_vp, _vp, _vp, _i64, _i64, _vp],
+    "mmemo_state_transfer_fwd_multi": [_i32, _vp, _vp, _vp, _vp, _i64, _i64, _vp],
+    "mmemo_state_transfer_bwd_multi": [_i32] + [_vp] * 7 + [_i64, _i64, _vp],
+    "mmemo_bilinear_head_fwd_multi": [_i32] + [_vp] * 10 + [_i64, _f32, _vp],
+    "mmemo_bilinear_head_bwd_multi": [_i32] + [_vp] * 16 + [_i64, _f32, _vp],
+    "mmemo_circle_loss_fwd_multi": [_i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
+    "mmemo_circle_loss_bwd_multi": [_i32] + [_vp] * 6 + [_i64, _vp],
+    "mmemo_rdrop_kl_fwd_multi": [_i32, _vp, _vp, _i64, _vp, _vp],
+    "mmemo_rdrop_kl_bwd_multi": [_i32, _vp, _vp, _vp, _vp, _i64, _vp],
     "mmemo_clip_grads_f32": [_i32, _vp, _vp, _vp, _f32, _vp],
     "mmemo_grad_sqnorm_multi_f32": [_i32, _vp, _vp, _vp, _vp, _vp],
     "mmemo_adam_step_multi_f32": [_i32] + [_vp] * 9 + [_f32, _f32, _f32, _i32, _vp, _f32, _vp],

@@ -1,6 +1,7 @@
 // Inference of an ensemble of k fold models (others/realformer.py:418-420, Ren-MME/run.py:560,
 // robot_demo.py:610-615: pred = mean of the members' logits).
-//   pool_fwd_multi    : the mean || max pooling of many fusion trunks (towers) in one launch
+//   pool_{fwd,bwd}_multi : the mean || max pooling of many fusion trunks (towers) in one launch,
+//                          with argmax and backward for the grouped training of k folds (folds.py)
 //   ensemble_head_fwd : every member's classifier linears + head, and the member mean, in one launch
 //                       (_members: each member's output as well, for fold_uncertainty)
 #include <cooperative_groups.h>
@@ -13,7 +14,8 @@ namespace cg = cooperative_groups;
 namespace {
 
 // ---------------------------------------------------------------------------------------------
-// Grouped pooling: pool_fwd_kernel (pool.cu) without argmax for several towers; blockIdx.z = tower.
+// Grouped pooling: pool_fwd_kernel / pool_bwd_kernel (pool.cu) for several towers with their own
+// batch sizes; blockIdx.z = tower (backward: tower * zsplit + part of the position axis).
 constexpr int POOL_MAX_GROUPS = 4;
 constexpr int POOL_MAX_SLOTS = 32;
 constexpr int POOL_MAX_PTRS = 256;    // segment pointers per launch
@@ -21,32 +23,57 @@ constexpr int POOL_MAX_TOWERS = 16;   // towers per launch (fewer when a tower h
 
 struct PoolMultiTable {
   const void* ptr[POOL_MAX_PTRS];     // [tower][group * n_slots + slot]
-  float* out[POOL_MAX_TOWERS];
+  float* out[POOL_MAX_TOWERS];        // forward: pooled output; backward: its gradient
+  int32_t* amax[POOL_MAX_TOWERS];     // training forward / backward only
+  int B[POOL_MAX_TOWERS];
   int len[POOL_MAX_GROUPS];
   int n_groups, n_slots, total_len;
 };
 
-template <typename T>
+template <typename T, bool WithArg>
 __global__ void __launch_bounds__(128)
 pool_fwd_multi_kernel(PoolMultiTable tb, int d) {
   const int F = tb.n_slots * d;
   const int f = blockIdx.x * 128 + threadIdx.x;
   const int64_t b = blockIdx.y;
   const int tower = blockIdx.z;
-  if (f >= F) return;
+  if (f >= F || b >= tb.B[tower]) return;
   const int slot = f / d, k = f - slot * d;
   float sum, mx;
-  pool_column<T, false>(tb.ptr + tower * tb.n_groups * tb.n_slots, tb.len, tb.n_groups, tb.n_slots,
-                        b, d, slot, k, sum, mx, nullptr);
+  int arg;
+  pool_column<T, WithArg>(tb.ptr + tower * tb.n_groups * tb.n_slots, tb.len, tb.n_groups,
+                          tb.n_slots, b, d, slot, k, sum, mx, &arg);
   float* out = tb.out[tower];
   out[b * 2 * F + f] = sum / (float)tb.total_len;
   out[b * 2 * F + F + f] = mx;
+  if (WithArg) tb.amax[tower][b * F + f] = arg;
 }
 
 template <typename T>
-int pool_fwd_multi(int n_towers, const void* const* ptrs, const int64_t* len, int n_groups,
-                   int n_slots, int64_t B, int64_t d, float* const* out, cudaStream_t st) {
-  MM_REQUIRE(n_towers >= 1 && ptrs && len && out && d > 0 && B >= 0);
+__global__ void __launch_bounds__(128)
+pool_bwd_multi_kernel(PoolMultiTable tb, int d, int zsplit) {
+  const int F = tb.n_slots * d;
+  const int f = blockIdx.x * 128 + threadIdx.x;
+  const int64_t b = blockIdx.y;
+  const int tower = blockIdx.z / zsplit, part = blockIdx.z - tower * zsplit;
+  if (f >= F || b >= tb.B[tower]) return;
+  const int slot = f / d, k = f - slot * d;
+  const float* dout = tb.out[tower];
+  const float dmean = dout[b * 2 * F + f] / (float)tb.total_len;
+  const float dmax = dout[b * 2 * F + F + f];
+  const int arg = tb.amax[tower][b * F + f];
+  const int per = (tb.total_len + zsplit - 1) / zsplit;
+  const int p_beg = part * per, p_end = min(tb.total_len, p_beg + per);
+  pool_column_bwd<T>(tb.ptr + tower * tb.n_groups * tb.n_slots, tb.len, tb.n_groups, tb.n_slots,
+                     b, d, slot, k, dmean, dmax, arg, p_beg, p_end);
+}
+
+// One table per POOL_MAX_TOWERS towers; `bwd` = the backward (out = dout, ptrs = dsegs).
+template <typename T>
+int pool_multi(bool bwd, int n_towers, const void* const* ptrs, const int64_t* len, int n_groups,
+               int n_slots, const int64_t* B, int64_t B_all, int64_t d, float* const* out,
+               int32_t* const* amax, cudaStream_t st) {
+  MM_REQUIRE(n_towers >= 1 && ptrs && len && out && d > 0);
   if (n_groups < 1 || n_groups > POOL_MAX_GROUPS || n_slots < 1 || n_slots > POOL_MAX_SLOTS)
     return MMEMO_ERR_SHAPE;
   PoolMultiTable tb;
@@ -61,19 +88,32 @@ int pool_fwd_multi(int n_towers, const void* const* ptrs, const int64_t* len, in
   MM_REQUIRE(tb.total_len > 0);
   const int segs = n_groups * n_slots;
   for (int t = 0; t < n_towers; ++t) {          // check every tower before the first launch
-    MM_REQUIRE(out[t]);
+    MM_REQUIRE(out[t] && (!amax || amax[t]) && (B ? B[t] : B_all) >= 0);
     for (int i = 0; i < segs; ++i) MM_REQUIRE(ptrs[(int64_t)t * segs + i]);
   }
-  if (B == 0) return MMEMO_OK;
   const int per = POOL_MAX_PTRS / segs < POOL_MAX_TOWERS ? POOL_MAX_PTRS / segs : POOL_MAX_TOWERS;
+  const unsigned gx = (unsigned)cdiv((int64_t)n_slots * d, 128);
   for (int t0 = 0; t0 < n_towers; t0 += per) {
     const int n = n_towers - t0 < per ? n_towers - t0 : per;
+    int64_t b_max = 0, b_sum = 0;
     for (int t = 0; t < n; ++t) {
       tb.out[t] = out[t0 + t];
+      tb.amax[t] = amax ? amax[t0 + t] : nullptr;
+      tb.B[t] = (int)(B ? B[t0 + t] : B_all);
+      b_max = tb.B[t] > b_max ? tb.B[t] : b_max;
+      b_sum += tb.B[t];
       for (int i = 0; i < segs; ++i) tb.ptr[t * segs + i] = ptrs[(int64_t)(t0 + t) * segs + i];
     }
-    dim3 grid((unsigned)cdiv((int64_t)n_slots * d, 128), (unsigned)B, (unsigned)n);
-    pool_fwd_multi_kernel<T><<<grid, 128, 0, st>>>(tb, (int)d);
+    if (b_max == 0) continue;
+    if (!bwd) {
+      dim3 grid(gx, (unsigned)b_max, (unsigned)n);
+      if (amax) pool_fwd_multi_kernel<T, true><<<grid, 128, 0, st>>>(tb, (int)d);
+      else pool_fwd_multi_kernel<T, false><<<grid, 128, 0, st>>>(tb, (int)d);
+    } else {
+      const int64_t zsplit = pool_bwd_zsplit((int64_t)gx * b_sum, tb.total_len);
+      dim3 grid(gx, (unsigned)b_max, (unsigned)(n * zsplit));
+      pool_bwd_multi_kernel<T><<<grid, 128, 0, st>>>(tb, (int)d, (int)zsplit);
+    }
     MM_LAUNCH_OK();
   }
   return MMEMO_OK;
@@ -306,14 +346,46 @@ extern "C" {
 int mmemo_pool_fwd_multi_f32(int n_towers, const void* const* seg_ptrs, const int64_t* group_len,
                              int n_groups, int n_slots, int64_t B, int64_t d, float* const* out,
                              mmemo_stream_t s) {
-  return pool_fwd_multi<float>(n_towers, seg_ptrs, group_len, n_groups, n_slots, B, d, out,
-                               mm_stream(s));
+  return pool_multi<float>(false, n_towers, seg_ptrs, group_len, n_groups, n_slots, nullptr, B, d,
+                           out, nullptr, mm_stream(s));
 }
 int mmemo_pool_fwd_multi_bf16(int n_towers, const void* const* seg_ptrs, const int64_t* group_len,
                               int n_groups, int n_slots, int64_t B, int64_t d, float* const* out,
                               mmemo_stream_t s) {
-  return pool_fwd_multi<bf16>(n_towers, seg_ptrs, group_len, n_groups, n_slots, B, d, out,
-                              mm_stream(s));
+  return pool_multi<bf16>(false, n_towers, seg_ptrs, group_len, n_groups, n_slots, nullptr, B, d,
+                          out, nullptr, mm_stream(s));
+}
+int mmemo_pool_fwd_multi_arg_f32(int n_towers, const void* const* seg_ptrs,
+                                 const int64_t* group_len, int n_groups, int n_slots,
+                                 const int64_t* B, int64_t d, float* const* out,
+                                 int32_t* const* argmax, mmemo_stream_t s) {
+  MM_REQUIRE(B && argmax);
+  return pool_multi<float>(false, n_towers, seg_ptrs, group_len, n_groups, n_slots, B, 0, d, out,
+                           argmax, mm_stream(s));
+}
+int mmemo_pool_fwd_multi_arg_bf16(int n_towers, const void* const* seg_ptrs,
+                                  const int64_t* group_len, int n_groups, int n_slots,
+                                  const int64_t* B, int64_t d, float* const* out,
+                                  int32_t* const* argmax, mmemo_stream_t s) {
+  MM_REQUIRE(B && argmax);
+  return pool_multi<bf16>(false, n_towers, seg_ptrs, group_len, n_groups, n_slots, B, 0, d, out,
+                          argmax, mm_stream(s));
+}
+int mmemo_pool_bwd_multi_f32(int n_towers, const float* const* dout, int32_t* const* argmax,
+                             void* const* dseg_ptrs, const int64_t* group_len, int n_groups,
+                             int n_slots, const int64_t* B, int64_t d, mmemo_stream_t s) {
+  MM_REQUIRE(B && argmax && dout);
+  return pool_multi<float>(true, n_towers, const_cast<const void* const*>(dseg_ptrs), group_len,
+                           n_groups, n_slots, B, 0, d, const_cast<float* const*>(dout), argmax,
+                           mm_stream(s));
+}
+int mmemo_pool_bwd_multi_bf16(int n_towers, const float* const* dout, int32_t* const* argmax,
+                              void* const* dseg_ptrs, const int64_t* group_len, int n_groups,
+                              int n_slots, const int64_t* B, int64_t d, mmemo_stream_t s) {
+  MM_REQUIRE(B && argmax && dout);
+  return pool_multi<bf16>(true, n_towers, const_cast<const void* const*>(dseg_ptrs), group_len,
+                          n_groups, n_slots, B, 0, d, const_cast<float* const*>(dout), argmax,
+                           mm_stream(s));
 }
 
 }  // extern "C"

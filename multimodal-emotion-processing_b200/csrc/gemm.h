@@ -22,7 +22,14 @@ struct GemmArgs {
   int c_zeroed;            // C is known to be all zero: the split-K reduce-add path skips its own fill
 };
 
+// Split-K (float32 C, linear epilogue, small output grid) uses the stream's workspace and sums the
+// partial tiles in a fixed order; without a workspace the GEMM does not split.
 int gemm_simt(const GemmArgs& g, int a_bf16, int b_bf16, int c_bf16, cudaStream_t st);
+// up to 48 independent float32 problems (no ReLU / position / accumulate epilogue) in one SIMT
+// launch (or a few, when their split-K scratch does not fit in the workspace at once); the bias
+// epilogue is kept.  Each problem gets gemm_simt's split factor: the same bits as gemm_simt.
+constexpr int GEMM_SIMT_MAX_GROUP = 48;
+int gemm_simt_grouped_f32(const GemmArgs* gs, int n, cudaStream_t st);
 
 // tcgen05/TMA path (bf16 operands, fp32 accumulate in TMEM).  c_bf16=0 -> float32 C.
 // Returns 1 if it accepts the shape/layout.

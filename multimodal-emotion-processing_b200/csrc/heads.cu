@@ -4,18 +4,11 @@
 //   bilinear_head  : cmu-mosei/run.py:332-339, Ren-MME/run.py:285-292, rencecps/run.py:141-148
 //   circle_loss    : others/realformer.py:289-298 (and its copies)
 //   rdrop_kl       : Ren-MME/run.py:332-334
-#include <math.h>
-
-#include "common.cuh"
+#include "heads.cuh"
 
 namespace {
 
-constexpr int CMAX = 16;
-
-__device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
-__device__ __forceinline__ float logsigmoidf_(float x) {
-  return fminf(x, 0.f) - log1pf(expf(-fabsf(x)));
-}
+constexpr int CMAX = HEAD_CMAX;
 
 // ---------------------------------------------------------------------------------------------
 // One WARP per sample: lane k owns class k; the (C x C) transfer matrix sits in shared memory and
@@ -28,28 +21,9 @@ state_transfer_fwd_kernel(const float* __restrict__ feats, const float* __restri
   __shared__ float T[CMAX * CMAX];
   for (int i = threadIdx.x; i < C * C; i += blockDim.x) T[i] = trans[i];
   __syncthreads();
-  const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (b >= B) return;
-  const bool on = lane < C;
-  float op = 0.f, gp = 0.f;
-  for (int i = 0; i < P; ++i) {
-    const float* f = feats + ((int64_t)b * P + i) * 2 * C;
-    float o = on ? f[lane] : 0.f;
-    const float g = on ? f[C + lane] : 0.f;
-    if (i > 0) {
-      float u = 0.f;
-      for (int j = 0; j < C; ++j) {
-        const float opj = __shfl_sync(0xffffffffu, op, j);
-        if (on) u = fmaf(opj, T[j * C + lane], u);
-      }
-      const float alpha = sigmoidf_(g + gp);
-      o = (1.0f - alpha) * o + alpha * tanhf(u);
-    }
-    if (on) out[((int64_t)b * P + i) * C + lane] = o;
-    op = o;
-    gp = g;
-  }
+  st_fwd_sample(feats, T, out, b, P, C, threadIdx.x & 31);
 }
 
 __global__ void __launch_bounds__(256)
@@ -60,59 +34,9 @@ state_transfer_bwd_kernel(const float* __restrict__ dout, const float* __restric
   __shared__ float T[CMAX * CMAX];
   for (int i = threadIdx.x; i < C * C; i += blockDim.x) T[i] = trans[i];
   __syncthreads();
-  const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (b >= B) return;
-  const bool on = lane < C;
-  float cdo = 0.f, cdg = 0.f;          // gradients carried from window i+1 into (o_i, g_i)
-  float dTr[CMAX];                     // column `lane` of dT, rows j
-#pragma unroll
-  for (int j = 0; j < CMAX; ++j) dTr[j] = 0.f;
-  for (int i = P - 1; i >= 0; --i) {
-    const float* f = feats + ((int64_t)b * P + i) * 2 * C;
-    float* df = dfeats + ((int64_t)b * P + i) * 2 * C;
-    const float dy = on ? dout[((int64_t)b * P + i) * C + lane] : 0.f;
-    const float dtot = dy + cdo;
-    if (i > 0) {
-      const float fo = on ? f[lane] : 0.f, fg = on ? f[C + lane] : 0.f;
-      const float gpv = on ? feats[((int64_t)b * P + i - 1) * 2 * C + C + lane] : 0.f;
-      const float op = on ? out[((int64_t)b * P + i - 1) * C + lane] : 0.f;
-      float u = 0.f;
-      for (int j = 0; j < C; ++j) {
-        const float opj = __shfl_sync(0xffffffffu, op, j);
-        if (on) u = fmaf(opj, T[j * C + lane], u);
-      }
-      const float a = sigmoidf_(fg + gpv);
-      const float t0 = tanhf(u);
-      const float dgs = dtot * (t0 - fo) * a * (1.0f - a);
-      const float du = on ? dtot * a * (1.0f - t0 * t0) : 0.f;
-      if (on) {
-        df[lane] = dtot * (1.0f - a);
-        df[C + lane] = dgs + cdg;
-      }
-      cdg = dgs;
-      // d o_{i-1}[j] = sum_k du[k] T[j][k]  (lane = j);  dT[j][k] += o_{i-1}[j] du[k]  (lane = k)
-      float ndo = 0.f;
-#pragma unroll
-      for (int k = 0; k < CMAX; ++k) {
-        if (k < C) {
-          const float duk = __shfl_sync(0xffffffffu, du, k);
-          const float opk = __shfl_sync(0xffffffffu, op, k);
-          if (on) ndo = fmaf(duk, T[lane * C + k], ndo);
-          dTr[k] = fmaf(opk, du, dTr[k]);
-        }
-      }
-      cdo = ndo;
-    } else if (on) {
-      df[lane] = dtot;
-      df[C + lane] = cdg;
-    }
-  }
-  if (dtrans && on) {
-#pragma unroll
-    for (int j = 0; j < CMAX; ++j)
-      if (j < C) atomicAdd(dtrans + j * C + lane, dTr[j]);
-  }
+  st_bwd_sample(dout, feats, T, out, dfeats, dtrans, b, P, C, threadIdx.x & 31);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -123,33 +47,9 @@ bilinear_fwd_kernel(const float* __restrict__ th, const float* __restrict__ la,
                     const float* __restrict__ beta, const float* __restrict__ W,
                     const float* __restrict__ bias, float* __restrict__ out,
                     float* __restrict__ zsave, int B, int C, float eps) {
-  const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (b >= B) return;
-  float z = 0.f;
-  if (lane < C)
-    for (int j = 0; j < C; ++j) {
-      const float tj = th[b * C + j];
-      for (int m = 0; m < C; ++m) z = fmaf(tj * la[b * C + m], T[(j * C + m) * C + lane], z);
-    }
-  const float mean = warp_sum(lane < C ? z : 0.f) / (float)C;
-  const float dlt = lane < C ? z - mean : 0.f;
-  const float rstd = rsqrtf(warp_sum(dlt * dlt) / (float)C + eps);
-  // cat[i]: i < C -> this[i]; else LN(z)[i-C]
-  float cat = 0.f;
-  if (lane < C) cat = th[b * C + lane];
-  const float ln = lane < C ? dlt * rstd * gamma[lane] + beta[lane] : 0.f;
-  const float ln_sh = __shfl_sync(0xffffffffu, ln, lane >= C ? lane - C : 0);
-  if (lane >= C && lane < 2 * C) cat = ln_sh;
-  float o = (lane < C) ? bias[lane] : 0.f;
-  for (int i = 0; i < 2 * C; ++i) {
-    const float ci = __shfl_sync(0xffffffffu, cat, i);
-    if (lane < C) o = fmaf(W[lane * 2 * C + i], ci, o);
-  }
-  if (lane < C) {
-    out[b * C + lane] = o;
-    zsave[b * C + lane] = z;
-  }
+  bilinear_fwd_sample(th, la, T, gamma, beta, W, bias, out, zsave, b, C, eps, threadIdx.x & 31);
 }
 
 __global__ void __launch_bounds__(256)
@@ -160,87 +60,9 @@ bilinear_bwd_kernel(const float* __restrict__ dout, const float* __restrict__ th
                     float* __restrict__ dla, float* __restrict__ dT, float* __restrict__ dgamma,
                     float* __restrict__ dbeta, float* __restrict__ dbias, int B, int C, float eps,
                     int copies) {
-  // [copies][C^3] dT | [C] dbias | [C] dgamma | [C] dbeta.  copies = 8 (one private dT per warp:
-  // plain += by the lane that owns class k, no shared-memory atomics - those are CAS loops and
-  // made this the longest kernel of the rencecps step) when it fits, else 1 (atomics).
   extern __shared__ float sm[];
-  const int C3 = C * C * C;
-  float* sT = sm;
-  float* sb = sT + copies * C3;
-  float* sg = sb + C;
-  float* sbe = sg + C;
-  const int nsm = copies * C3 + 3 * C;
-  for (int i = threadIdx.x; i < nsm; i += blockDim.x) sm[i] = 0.f;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float* myT = sT + (copies > 1 ? warp * C3 : 0);
-  for (int b = blockIdx.x * 8 + warp; b < B; b += gridDim.x * 8) {
-    const float z = lane < C ? zsave[b * C + lane] : 0.f;
-    const float mean = warp_sum(z) / (float)C;
-    const float dlt = lane < C ? z - mean : 0.f;
-    const float rstd = rsqrtf(warp_sum(dlt * dlt) / (float)C + eps);
-    const float zh = dlt * rstd;
-    const float dy = lane < C ? dout[b * C + lane] : 0.f;
-    const float thv = lane < C ? th[b * C + lane] : 0.f;
-    const float lav = lane < C ? la[b * C + lane] : 0.f;
-    // dcat[i] = sum_n dy[n] W[n][i]
-    float dcat = 0.f;
-    for (int n = 0; n < C; ++n) {
-      const float dyn = __shfl_sync(0xffffffffu, dy, n);
-      if (lane < 2 * C) dcat = fmaf(dyn, W[n * 2 * C + lane], dcat);
-    }
-    // LN backward on the second half of dcat
-    const float dln = __shfl_sync(0xffffffffu, dcat, lane < C ? lane + C : 0);
-    const float w = lane < C ? dln * gamma[lane] : 0.f;
-    const float m1 = warp_sum(w) / (float)C;
-    const float m2 = warp_sum(w * zh) / (float)C;
-    const float dz = lane < C ? rstd * (w - m1 - zh * m2) : 0.f;
-    if (lane < C) {
-      atomicAdd(&sg[lane], dln * zh);
-      atomicAdd(&sbe[lane], dln);
-      atomicAdd(&sb[lane], dy);
-    }
-    // d_this[j] = dcat[j] + sum_{m,k} last[m] T[j][m][k] dz[k];  d_last[m] = sum_{j,k} this[j] T dz
-    float dthis = (lane < C) ? dcat : 0.f, dlast = 0.f;
-    for (int k = 0; k < C; ++k) {
-      const float dzk = __shfl_sync(0xffffffffu, dz, k);
-      for (int o2 = 0; o2 < C; ++o2) {
-        const float l_o = __shfl_sync(0xffffffffu, lav, o2);
-        const float t_o = __shfl_sync(0xffffffffu, thv, o2);
-        if (lane < C) {
-          dthis = fmaf(l_o * dzk, T[(lane * C + o2) * C + k], dthis);  // j = lane, m = o2
-          dlast = fmaf(t_o * dzk, T[(o2 * C + lane) * C + k], dlast);  // j = o2, m = lane
-        }
-      }
-    }
-    if (lane < C) {
-      dth[b * C + lane] = dthis;
-      dla[b * C + lane] = dlast;
-    }
-    // dT[j][m][k] += this[j] last[m] dz[k]   (lane = k)
-    for (int j = 0; j < C; ++j) {
-      const float tj = __shfl_sync(0xffffffffu, thv, j);
-      for (int m = 0; m < C; ++m) {
-        const float lm = __shfl_sync(0xffffffffu, lav, m);
-        if (lane < C) {
-          if (copies > 1) myT[(j * C + m) * C + lane] += tj * lm * dz;
-          else atomicAdd(&sT[(j * C + m) * C + lane], tj * lm * dz);
-        }
-      }
-    }
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < C3; i += blockDim.x)
-    if (dT) {
-      float t = 0.f;
-      for (int c = 0; c < copies; ++c) t += sT[c * C3 + i];
-      atomicAdd(dT + i, t);
-    }
-  for (int i = threadIdx.x; i < C; i += blockDim.x) {
-    if (dgamma) atomicAdd(dgamma + i, sg[i]);
-    if (dbeta) atomicAdd(dbeta + i, sbe[i]);
-    if (dbias) atomicAdd(dbias + i, sb[i]);
-  }
+  bilinear_bwd_cta(sm, dout, th, la, T, gamma, W, zsave, dth, dla, dT, dgamma, dbeta, dbias, B, C,
+                   eps, copies, blockIdx.x, gridDim.x);
 }
 
 // dW[n][i] += sum_b dy[b][n] cat[b][i]: thread per (n, i); blockIdx.y splits the batch into strips
@@ -251,28 +73,8 @@ __global__ void bilinear_dw_kernel(const float* __restrict__ dout, const float* 
                                    int C, float eps) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= 2 * C * C) return;
-  const int n = idx / (2 * C), i = idx - n * 2 * C;
   const int b0 = blockIdx.y * 16, b1 = min(B, b0 + 16);
-  float acc = 0.f;
-  for (int b = b0; b < b1; ++b) {
-    float cat;
-    if (i < C) {
-      cat = th[b * C + i];
-    } else {
-      float mean = 0.f;
-      for (int k = 0; k < C; ++k) mean += zsave[b * C + k];
-      mean /= (float)C;
-      float var = 0.f;
-      for (int k = 0; k < C; ++k) {
-        const float t = zsave[b * C + k] - mean;
-        var = fmaf(t, t, var);
-      }
-      const float rstd = rsqrtf(var / (float)C + eps);
-      cat = (zsave[b * C + i - C] - mean) * rstd * gamma[i - C] + beta[i - C];
-    }
-    acc = fmaf(dout[b * C + n], cat, acc);
-  }
-  atomicAdd(dW + idx, acc);
+  bilinear_dw_strip(dout, th, zsave, gamma, beta, dW, idx, b0, b1, C, eps);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -280,21 +82,7 @@ __global__ void circle_loss_fwd_kernel(const float* __restrict__ s, const float*
                                        float* __restrict__ loss, int64_t R, int C) {
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= R) return;
-  float mn = 0.f, mp = 0.f;  // the appended zero
-  for (int i = 0; i < C; ++i) {
-    const float yi = y[r * C + i];
-    const float v = (1.0f - 2.0f * yi) * s[r * C + i];
-    mn = fmaxf(mn, v - yi * 1e12f);
-    mp = fmaxf(mp, v - (1.0f - yi) * 1e12f);
-  }
-  float sn = expf(0.f - mn), sp = expf(0.f - mp);
-  for (int i = 0; i < C; ++i) {
-    const float yi = y[r * C + i];
-    const float v = (1.0f - 2.0f * yi) * s[r * C + i];
-    sn += expf(v - yi * 1e12f - mn);
-    sp += expf(v - (1.0f - yi) * 1e12f - mp);
-  }
-  loss[r] = (mn + logf(sn)) + (mp + logf(sp));
+  loss[r] = circle_row_loss(s, y, r, C);
 }
 
 __global__ void circle_loss_bwd_kernel(const float* __restrict__ dloss, const float* __restrict__ s,
@@ -302,64 +90,20 @@ __global__ void circle_loss_bwd_kernel(const float* __restrict__ dloss, const fl
                                        int64_t R, int C) {
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= R) return;
-  float mn = 0.f, mp = 0.f;
-  for (int i = 0; i < C; ++i) {
-    const float yi = y[r * C + i];
-    const float v = (1.0f - 2.0f * yi) * s[r * C + i];
-    mn = fmaxf(mn, v - yi * 1e12f);
-    mp = fmaxf(mp, v - (1.0f - yi) * 1e12f);
-  }
-  float sn = expf(0.f - mn), sp = expf(0.f - mp);
-  for (int i = 0; i < C; ++i) {
-    const float yi = y[r * C + i];
-    const float v = (1.0f - 2.0f * yi) * s[r * C + i];
-    sn += expf(v - yi * 1e12f - mn);
-    sp += expf(v - (1.0f - yi) * 1e12f - mp);
-  }
-  const float g = dloss[r];
-  for (int i = 0; i < C; ++i) {
-    const float yi = y[r * C + i];
-    const float sg = 1.0f - 2.0f * yi;
-    const float v = sg * s[r * C + i];
-    const float pn = expf(v - yi * 1e12f - mn) / sn;
-    const float pp = expf(v - (1.0f - yi) * 1e12f - mp) / sp;
-    ds[r * C + i] = g * sg * (pn + pp);
-  }
+  circle_row_bwd(dloss[r], s, y, ds, r, C);
 }
 
 // single CTA: n = B/2 pairs x C classes
 __global__ void __launch_bounds__(256)
 rdrop_fwd_kernel(const float* __restrict__ s, float* __restrict__ out, int n, int C) {
-  __shared__ float red[8];
-  float acc = 0.f;
-  for (int e = threadIdx.x; e < n * C; e += 256) {
-    const int i = e / C, c = e - i * C;
-    const float a = s[(2 * i) * C + c], b = s[(2 * i + 1) * C + c];
-    const float la = logsigmoidf_(a), lb = logsigmoidf_(b);
-    acc += expf(lb) * (lb - la) + expf(la) * (la - lb);
-  }
-  acc = warp_sum(acc);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float t = 0.f;
-    for (int w = 0; w < 8; ++w) t += red[w];
-    out[0] = t / (float)n * 0.5f;
-  }
+  rdrop_kl_cta(s, out, n, C);
 }
 
 __global__ void rdrop_bwd_kernel(const float* __restrict__ dout, const float* __restrict__ s,
                                  float* __restrict__ ds, int n, int C) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n * C) return;
-  const int i = e / C, c = e - i * C;
-  const float a = s[(2 * i) * C + c], b = s[(2 * i + 1) * C + c];
-  const float la = logsigmoidf_(a), lb = logsigmoidf_(b);
-  const float sa = expf(la), sb = expf(lb);
-  const float g = dout[0] * 0.5f / (float)n;
-  // d/da [ sb*(lb-la) + sa*(la-lb) ] = -sb*(1-sa) + sa*(1-sa)*(la-lb) + sa*(1-sa)
-  ds[(2 * i) * C + c] = g * ((1.0f - sa) * (sa * (la - lb + 1.0f) - sb));
-  ds[(2 * i + 1) * C + c] = g * ((1.0f - sb) * (sb * (lb - la + 1.0f) - sa));
+  rdrop_kl_bwd_elem(dout, s, ds, e, n, C);
 }
 
 }  // namespace
@@ -406,10 +150,9 @@ int mmemo_bilinear_head_bwd(const float* dout, const float* this_feat, const flo
   if (B <= 0) return MMEMO_OK;
   MM_REQUIRE(dout && this_feat && last_feat && trans && gamma && beta && w && z && dthis && dlast);
   if (C < 1 || C > CMAX) return MMEMO_ERR_SHAPE;
-  const int copies = (C <= 10) ? 8 : 1;                    // 8 x C^3 floats <= 32 KB
-  const size_t smem = sizeof(float) * (copies * C * C * C + 3 * C);
-  int64_t blocks = cdiv(B, 8);
-  if (blocks > 32) blocks = 32;
+  const int copies = bilinear_bwd_copies(C);
+  const size_t smem = bilinear_bwd_smem(C);
+  const int64_t blocks = bilinear_bwd_ctas(B);
   bilinear_bwd_kernel<<<(unsigned)blocks, 256, smem, mm_stream(s)>>>(
       dout, this_feat, last_feat, trans, gamma, w, z, dthis, dlast, dtrans, dgamma, dbeta, dbias,
       (int)B, (int)C, eps, copies);

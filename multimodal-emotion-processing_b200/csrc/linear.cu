@@ -180,6 +180,104 @@ int mmemo_linear_bwd_w_grouped_bf16(int n, const void* const* dy, const int64_t*
   return MMEMO_OK;
 }
 
+// ---- grouped float32 variants: n independent problems, one SIMT launch per 48 (the head linears,
+// which run in float32 in both precision modes) ----
+int mmemo_linear_fwd_grouped_f32(int n, const float* const* x, const int64_t* ldx,
+                                 const float* const* w, const int64_t* ldw,
+                                 const float* const* bias, float* const* y, const int64_t* ldy,
+                                 const int64_t* M, const int64_t* N, const int64_t* K,
+                                 mmemo_stream_t s) {
+  MM_REQUIRE(n >= 0 && (n == 0 || (x && ldx && w && ldw && y && ldy && M && N && K)));
+  GemmArgs g[GEMM_SIMT_MAX_GROUP] = {};
+  for (int i0 = 0; i0 < n; i0 += GEMM_SIMT_MAX_GROUP) {
+    const int m = n - i0 < GEMM_SIMT_MAX_GROUP ? n - i0 : GEMM_SIMT_MAX_GROUP;
+    for (int j = 0; j < m; ++j) {
+      const int i = i0 + j;
+      MM_REQUIRE(x[i] && w[i] && y[i]);
+      g[j] = GemmArgs{};
+      g[j].A = x[i]; g[j].sAm = ldx[i]; g[j].sAk = 1;
+      g[j].B = w[i]; g[j].sBn = ldw[i]; g[j].sBk = 1;
+      g[j].C = y[i]; g[j].ldc = ldy[i];
+      g[j].M = M[i]; g[j].N = N[i]; g[j].K = K[i];
+      g[j].bias = bias ? bias[i] : nullptr; g[j].pos_period = 1;
+    }
+    const int rc = gemm_simt_grouped_f32(g, m, mm_stream(s));
+    if (rc) return rc;
+  }
+  return MMEMO_OK;
+}
+int mmemo_linear_bwd_x_grouped_f32(int n, const float* const* dy, const int64_t* lddy,
+                                   const float* const* w, const int64_t* ldw, float* const* dx,
+                                   const int64_t* lddx, const int64_t* M, const int64_t* N,
+                                   const int64_t* K, mmemo_stream_t s) {
+  MM_REQUIRE(n >= 0 && (n == 0 || (dy && lddy && w && ldw && dx && lddx && M && N && K)));
+  GemmArgs g[GEMM_SIMT_MAX_GROUP] = {};
+  for (int i0 = 0; i0 < n; i0 += GEMM_SIMT_MAX_GROUP) {
+    const int m = n - i0 < GEMM_SIMT_MAX_GROUP ? n - i0 : GEMM_SIMT_MAX_GROUP;
+    for (int j = 0; j < m; ++j) {
+      const int i = i0 + j;
+      MM_REQUIRE(dy[i] && w[i] && dx[i]);
+      g[j] = GemmArgs{};
+      g[j].A = dy[i]; g[j].sAm = lddy[i]; g[j].sAk = 1;
+      g[j].B = w[i]; g[j].sBn = 1; g[j].sBk = ldw[i];
+      g[j].C = dx[i]; g[j].ldc = lddx[i];
+      g[j].M = M[i]; g[j].N = K[i]; g[j].K = N[i];
+      g[j].pos_period = 1;
+    }
+    const int rc = gemm_simt_grouped_f32(g, m, mm_stream(s));
+    if (rc) return rc;
+  }
+  return MMEMO_OK;
+}
+
+namespace {
+__device__ const float g_one = 1.0f;     // the ones vector (stride 0) of the bias-gradient problems
+}
+
+int mmemo_linear_bwd_w_grouped_f32(int n, const float* const* dy, const int64_t* lddy,
+                                   const float* const* x, const int64_t* ldx, float* const* dw,
+                                   const int64_t* lddw, float* const* dbias, const int64_t* M,
+                                   const int64_t* N, const int64_t* K, mmemo_stream_t s) {
+  MM_REQUIRE(n >= 0 && (n == 0 || (dy && lddy && x && ldx && dw && lddw && M && N && K)));
+  const void* one = nullptr;
+  // problem list: every dW, then every dbias as the GEMM dy^T 1 (N x 1, K' = M)
+  GemmArgs all[2 * GEMM_SIMT_MAX_GROUP];
+  int n_all = 0;
+  for (int i0 = 0; i0 < n; i0 += GEMM_SIMT_MAX_GROUP) {
+    const int m = n - i0 < GEMM_SIMT_MAX_GROUP ? n - i0 : GEMM_SIMT_MAX_GROUP;
+    n_all = 0;
+    for (int j = 0; j < m; ++j) {
+      const int i = i0 + j;
+      MM_REQUIRE(dy[i] && x[i] && dw[i]);
+      GemmArgs& g = all[n_all++];
+      g = GemmArgs{};
+      g.A = dy[i]; g.sAm = 1; g.sAk = lddy[i];
+      g.B = x[i]; g.sBn = 1; g.sBk = ldx[i];
+      g.C = dw[i]; g.ldc = lddw[i];
+      g.M = N[i]; g.N = K[i]; g.K = M[i];
+      g.pos_period = 1;
+    }
+    for (int j = 0; dbias && j < m; ++j) {
+      const int i = i0 + j;
+      if (!dbias[i]) continue;
+      if (!one) MM_CUDA_OK(cudaGetSymbolAddress(const_cast<void**>(&one), g_one));
+      GemmArgs& g = all[n_all++];
+      g = GemmArgs{};
+      g.A = dy[i]; g.sAm = 1; g.sAk = lddy[i];
+      g.B = one; g.sBn = 0; g.sBk = 0;
+      g.C = dbias[i]; g.ldc = 1;
+      g.M = N[i]; g.N = 1; g.K = M[i];
+      g.pos_period = 1;
+    }
+    for (int a = 0; a < n_all; a += GEMM_SIMT_MAX_GROUP) {
+      const int rc = gemm_simt_grouped_f32(all + a, n_all - a < GEMM_SIMT_MAX_GROUP ?
+                                           n_all - a : GEMM_SIMT_MAX_GROUP, mm_stream(s));
+      if (rc) return rc;
+    }
+  }
+  return MMEMO_OK;
+}
+
 #define MM_LINEAR(SUF, BF)                                                                        \
   int mmemo_linear_fwd_##SUF(const void* x, int x_is_f32, int64_t ldx, const void* w, int64_t ldw, \
                              const float* bias, const float* pos, int64_t pos_period, void* y,    \

@@ -49,15 +49,8 @@ pool_bwd_kernel(SegTable tb, int64_t B, int d, const float* __restrict__ dout,
   // gridDim.z splits the position axis
   const int per = (tb.total_len + gridDim.z - 1) / gridDim.z;
   const int p_beg = blockIdx.z * per, p_end = min(tb.total_len, p_beg + per);
-  int pos0 = 0;
-  for (int g = 0; g < tb.n_groups; ++g) {
-    T* __restrict__ p = static_cast<T*>(const_cast<void*>(tb.ptr[g * tb.n_slots + slot])) +
-                        b * (int64_t)tb.len[g] * d + k;
-    const int lo = max(p_beg - pos0, 0), hi = min(p_end - pos0, tb.len[g]);
-    for (int t = lo; t < hi; ++t)
-      p[(int64_t)t * d] = from_f<T>(dmean + ((pos0 + t) == arg ? dmax : 0.f));
-    pos0 += tb.len[g];
-  }
+  pool_column_bwd<T>(tb.ptr, tb.len, tb.n_groups, tb.n_slots, b, d, slot, k, dmean, dmax, arg,
+                     p_beg, p_end);
 }
 
 int make_table(SegTable& tb, const void* const* ptrs, const int64_t* len, int n_groups, int n_slots) {
@@ -100,10 +93,7 @@ int pool_bwd(const float* dout, const int32_t* amax, void* const* ptrs, const in
   const int rc = make_table(tb, const_cast<const void* const*>(ptrs), len, n_groups, n_slots);
   if (rc) return rc;
   const int64_t base = cdiv((int64_t)n_slots * d, 128) * B;
-  int64_t zsplit = cdiv(148 * 8, base);
-  if (zsplit < 1) zsplit = 1;
-  if (zsplit > tb.total_len) zsplit = tb.total_len;
-  if (zsplit > 64) zsplit = 64;
+  const int64_t zsplit = pool_bwd_zsplit(base, tb.total_len);
   dim3 grid((unsigned)cdiv((int64_t)n_slots * d, 128), (unsigned)B, (unsigned)zsplit);
   pool_bwd_kernel<T><<<grid, 128, 0, st>>>(tb, B, (int)d, dout, amax);
   MM_LAUNCH_OK();
