@@ -112,6 +112,21 @@ int mmemo_linear_fwd_grouped_bf16(int n, const void* const* x, const int64_t* ld
                                   const int* relu, const int* accumulate,
                                   const float* const* pos, const int64_t* pos_period,
                                   const int64_t* ldpos, mmemo_stream_t stream);
+/* The grouped forward with a training dropout between the bias and the position table (the
+ * modality projections, robot_demo.py:302-311 then :392-394): y[i] = drop_i(x[i] w[i]^T + bias[i])
+ * + pos[i], one tensor-core launch.  The mask of problem i is the one mmemo_dropout_multi_* draws
+ * for a contiguous (M[i], N[i]) tensor with seeds[i] and the device step counter `step` (read when
+ * the kernel runs), whatever ldy[i] is; kept values are scaled by 1 / (1 - p).  p = 0 is the
+ * plain grouped forward.  No relu / accumulate; every problem must fit the tensor-core kernel
+ * (MMEMO_ERR_SHAPE otherwise: there is no other implementation of the mask). */
+int mmemo_linear_fwd_grouped_dropout_bf16(int n, const void* const* x, const int64_t* ldx,
+                                          const void* const* w, const int64_t* ldw,
+                                          const float* const* bias, void* const* y,
+                                          const int64_t* ldy, const int64_t* M, const int64_t* N,
+                                          const int64_t* K, const float* const* pos,
+                                          const int64_t* pos_period, const int64_t* ldpos,
+                                          const uint64_t* seeds, float p, const uint64_t* step,
+                                          mmemo_stream_t stream);
 int mmemo_linear_bwd_x_grouped_bf16(int n, const void* const* dy, const int64_t* lddy,
                                     const void* const* w, const int64_t* ldw, void* const* dx,
                                     const int64_t* lddx, const void* const* relu_src,
@@ -346,6 +361,17 @@ int mmemo_dropout_multi_f32(int n, const void* const* x, void* const* y, const i
 int mmemo_dropout_multi_bf16(int n, const void* const* x, void* const* y, const int64_t* numel,
                              const uint64_t* seeds, float p, const uint64_t* step,
                              mmemo_stream_t stream);
+/* Backward of mmemo_linear_fwd_grouped_dropout_bf16 for n >= 1 problems, one launch per 64: dym[i]
+ * (contiguous bf16 (M[i], N[i])) = mask_i * dy[i] / (1 - p), with dy[i] read at row stride
+ * lddy[i] (a column slice of a concatenated output) and the mask of that forward (same seeds, p,
+ * step); dbias[i] (nullable array and entries, float32 [N[i]]) += column sums of dym[i];
+ * dpos[i] (nullable, float32 (period[i], N[i]) at row stride ldpos[i]) += sums of the UNMASKED
+ * dy[i] rows m with m % period[i] = r into row r.  N[i] and lddy[i] even. */
+int mmemo_proj_dropout_bwd_bf16(int n, const void* const* dy, const int64_t* lddy,
+                                void* const* dym, const int64_t* M, const int64_t* N,
+                                const uint64_t* seeds, float p, const uint64_t* step,
+                                float* const* dbias, float* const* dpos, const int64_t* period,
+                                const int64_t* ldpos, mmemo_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Fusion pooling: concat on features, concat on positions (l, a, v), mean || max over ALL

@@ -66,6 +66,7 @@ SIGNATURES = {
     "mmemo_linear_bwd_x_f32": _LINEAR_BWD_X, "mmemo_linear_bwd_x_bf16": _LINEAR_BWD_X,
     "mmemo_linear_bwd_w_f32": _LINEAR_BWD_W, "mmemo_linear_bwd_w_bf16": _LINEAR_BWD_W,
     "mmemo_linear_fwd_grouped_bf16": [_i32] + [_vp] * 15 + [_vp],
+    "mmemo_linear_fwd_grouped_dropout_bf16": [_i32] + [_vp] * 14 + [_f32, _vp, _vp],
     "mmemo_linear_bwd_x_grouped_bf16": [_i32] + [_vp] * 12 + [_vp],
     "mmemo_linear_bwd_w_grouped_bf16": [_i32] + [_vp] * 9 + [_i32, _vp],
     "mmemo_linear_fwd_grouped_f32": [_i32] + [_vp] * 10 + [_vp],
@@ -97,6 +98,7 @@ SIGNATURES = {
     "mmemo_dropout_f32": _DROPOUT, "mmemo_dropout_bf16": _DROPOUT,
     "mmemo_dropout_multi_f32": [_i32, _vp, _vp, _vp, _vp, _f32, _vp, _vp],
     "mmemo_dropout_multi_bf16": [_i32, _vp, _vp, _vp, _vp, _f32, _vp, _vp],
+    "mmemo_proj_dropout_bwd_bf16": [_i32] + [_vp] * 6 + [_f32] + [_vp] * 6,
     "mmemo_pool_fwd_f32": _POOL_FWD, "mmemo_pool_fwd_bf16": _POOL_FWD,
     "mmemo_pool_bwd_f32": _POOL_BWD, "mmemo_pool_bwd_bf16": _POOL_BWD,
     "mmemo_pool_fwd_multi_f32": _POOL_FWD_MULTI, "mmemo_pool_fwd_multi_bf16": _POOL_FWD_MULTI,

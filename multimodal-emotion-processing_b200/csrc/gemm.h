@@ -20,6 +20,11 @@ struct GemmArgs {
   int relu;                // C = max(C, 0)
   int accumulate;          // C += result
   int c_zeroed;            // C is known to be all zero: the split-K reduce-add path skips its own fill
+  // dropout between bias and position table (forward family 3 only; drop_p = 0: none): the mask
+  // of a contiguous (M, N) tensor drawn from drop_seed + step[0] (dropout.cuh)
+  float drop_p;
+  uint64_t drop_seed;
+  const uint64_t* drop_step;
 };
 
 // Split-K (float32 C, linear epilogue, small output grid) uses the stream's workspace and sums the
@@ -34,7 +39,8 @@ int gemm_simt_grouped_f32(const GemmArgs* gs, int n, cudaStream_t st);
 // tcgen05/TMA path (bf16 operands, fp32 accumulate in TMEM).  c_bf16=0 -> float32 C.
 // Returns 1 if it accepts the shape/layout.
 bool gemm_tc_supported(const GemmArgs& g, int c_bf16, bool any_size = false);
-// family: 0 forward, 1 dX, 2 dW (only names the kernel instantiation)
+// family: 0 forward, 1 dX, 2 dW (only names the kernel instantiation), 3 forward with the dropout
+// epilogue (GemmArgs::drop_*)
 int gemm_tc(const GemmArgs& g, int c_bf16, int family, cudaStream_t st);
 // up to 48 independent problems in one persistent launch (every problem must be gemm_tc_supported)
 constexpr int GEMM_TC_MAX_GROUP = 48;

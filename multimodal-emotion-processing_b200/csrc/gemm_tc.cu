@@ -35,6 +35,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "dropout.cuh"
 #include "gemm.h"
 #include "tc_common.cuh"
 
@@ -65,6 +66,9 @@ struct TcArgs {
   int splits, kb_per, kb_total;
   int reduce_add;          // split-K slices are summed into the fp32 C by TMA reduce-add
   int tiles_m, tiles_n;    // in units of the (pair) tile: TM x BN
+  uint32_t drop_thr;       // family 3: dropout threshold round(p * 65536) (0: keep all) ...
+  float drop_scale;        //   ... and 1 / (1 - p)
+  unsigned long long drop_seed;
 };
 
 // One launch can serve up to MAXG independent GEMMs ("grouped"): the work items of all problems
@@ -73,8 +77,10 @@ struct TcArgs {
 // Two capacities of the same kernel: NG = 6 (the launches of one block: ~3.5 KB of kernel
 // parameters) and NG = 48 (the nine chains x five weight gradients of a fusion-trunk layer, both
 // towers' projections: ~29 KB, within the 32 764-byte parameter limit of CUDA >= 12.1).
-// FAM only names the instantiation after the Linear-layer pass it serves (0 fwd, 1 dX, 2 dW), so
-// that profiler launch lists can be read per family.
+// FAM names the instantiation after the Linear-layer pass it serves (0 fwd, 1 dX, 2 dW), so that
+// profiler launch lists can be read per family; FAM 3 is the forward with a dropout between the
+// bias and the position table (the training-mode modality projections), the only instantiation
+// that carries the mask code.
 constexpr int MAXG_SMALL = 6, MAXG = 48;
 template <int NG> struct TmapGroup { CUtensorMap a[NG], b[NG], c[NG], aux[NG]; };
 template <int NG> struct GroupArgs {
@@ -82,6 +88,7 @@ template <int NG> struct GroupArgs {
   int any_aux;             // some problem of the launch prefetches an aux tile (owns the second 32 KB)
   int streamk;             // 1: item_start counts K-BLOCKS (tiles x kb_total per problem) and every
   int kb_per_unit;         //    unit owns one contiguous range of kb_per_unit of them (see below)
+  const unsigned long long* drop_step;   // family 3: device step counter mixed into the seeds
   int item_start[NG + 1];
   TcArgs p[NG];
 };
@@ -349,6 +356,22 @@ gemm_tc_kernel(const __grid_constant__ TmapGroup<NG> TMS, const __grid_constant_
             for (int i = 0; i < 32; ++i)
               r[i] = __float_as_uint(__uint_as_float(r[i]) + sbias[ch * 32 + i]);
           }
+          if constexpr (FAM == 3) {
+            // y = drop(x W^T + b) + pos: the mask of element (m, c) of the contiguous (M, N)
+            // tensor, i = m*N + c, one hash per four consecutive i (dropout.cuh)
+            if (a.drop_thr) {
+              const uint64_t seed = drop_seed(a.drop_seed, G.drop_step);
+              const uint64_t i0 = (uint64_t)m * (uint64_t)a.N + (uint64_t)(nh + ch * 32);
+              uint64_t h = hash_bits(seed, i0 >> 2);
+#pragma unroll
+              for (int i = 0; i < 32; ++i) {
+                const uint64_t e = i0 + i;
+                if (i > 0 && (e & 3) == 0) h = hash_bits(seed, e >> 2);
+                r[i] = __float_as_uint(drop_keep(h, e, a.drop_thr)
+                                           ? __uint_as_float(r[i]) * a.drop_scale : 0.f);
+              }
+            }
+          }
           if (a.pos && m < a.M) {   // position table row of this output row (period = seq length)
             const float* prow = a.pos + (int64_t)pos_row * a.pos_ld + nh + ch * 32;
 #pragma unroll
@@ -611,7 +634,7 @@ int gemm_tc_grouped_t(const GemmArgs* gs, const int* c_bf16s, int n, cudaStream_
     tiles_sum += (int)(cdiv(g.M, TM) * cdiv(g.N, BN));
     const int kb = (int)cdiv(g.K, BK);
     kb_min = kb < kb_min ? kb : kb_min;
-    linear = linear && !g.relu && !g.relu_src && !g.pos;
+    linear = linear && !g.relu && !g.relu_src && !g.pos && !(g.drop_p > 0.f);
     all_reduce_add = all_reduce_add && !c_bf16s[i] && !g.bias;   // fp32 C summed by TMA reduce-add
   }
   int splits = 1;
@@ -715,6 +738,12 @@ int gemm_tc_grouped_t(const GemmArgs* gs, const int* c_bf16s, int n, cudaStream_
     a.splits = sp; a.kb_per = kb_per; a.kb_total = kb_total;
     a.reduce_add = reduce_add;
     a.tiles_m = tiles_m; a.tiles_n = tiles_n;
+    if (g.drop_p > 0.f) {
+      a.drop_thr = (uint32_t)(g.drop_p * 65536.0f + 0.5f);
+      a.drop_scale = 1.0f / (1.0f - g.drop_p);
+      a.drop_seed = g.drop_seed;
+      G.drop_step = reinterpret_cast<const unsigned long long*>(g.drop_step);
+    }
     G.item_start[i] = items;
     items += streamk ? tiles * kb_total : tiles * sp;
     if (reduce_add && !g.accumulate && !g.c_zeroed)   // the slices accumulate into C: start from zero
@@ -781,10 +810,12 @@ int gemm_tc_grouped(const GemmArgs* gs, const int* c_bf16s, int n, int family, c
   if (n <= MAXG_SMALL) {
     if (family == 0) return gemm_tc_grouped_t<MAXG_SMALL, 0>(gs, c_bf16s, n, st);
     if (family == 1) return gemm_tc_grouped_t<MAXG_SMALL, 1>(gs, c_bf16s, n, st);
+    if (family == 3) return gemm_tc_grouped_t<MAXG_SMALL, 3>(gs, c_bf16s, n, st);
     return gemm_tc_grouped_t<MAXG_SMALL, 2>(gs, c_bf16s, n, st);
   }
   if (family == 0) return gemm_tc_grouped_t<MAXG, 0>(gs, c_bf16s, n, st);
   if (family == 1) return gemm_tc_grouped_t<MAXG, 1>(gs, c_bf16s, n, st);
+  if (family == 3) return gemm_tc_grouped_t<MAXG, 3>(gs, c_bf16s, n, st);
   return gemm_tc_grouped_t<MAXG, 2>(gs, c_bf16s, n, st);
 }
 

@@ -122,6 +122,41 @@ int mmemo_linear_fwd_grouped_bf16(int n, const void* const* x, const int64_t* ld
   }
   return MMEMO_OK;
 }
+int mmemo_linear_fwd_grouped_dropout_bf16(int n, const void* const* x, const int64_t* ldx,
+                                          const void* const* w, const int64_t* ldw,
+                                          const float* const* bias, void* const* y,
+                                          const int64_t* ldy, const int64_t* M, const int64_t* N,
+                                          const int64_t* K, const float* const* pos,
+                                          const int64_t* pos_period, const int64_t* ldpos,
+                                          const uint64_t* seeds, float p, const uint64_t* step,
+                                          mmemo_stream_t s) {
+  if (n < 1 || n > GEMM_TC_MAX_GROUP) return MMEMO_ERR_ARG;
+  MM_REQUIRE(x && ldx && w && ldw && y && ldy && M && N && K && seeds && step);
+  MM_REQUIRE(p >= 0.f && p < 1.f);
+  GemmArgs g[GEMM_TC_MAX_GROUP] = {};
+  int cb[GEMM_TC_MAX_GROUP];
+  for (int i = 0; i < n; ++i) {
+    MM_REQUIRE(x[i] && w[i] && y[i]);
+    g[i].A = x[i]; g[i].sAm = ldx[i]; g[i].sAk = 1;
+    g[i].B = w[i]; g[i].sBn = ldw[i]; g[i].sBk = 1;
+    g[i].C = y[i]; g[i].ldc = ldy[i];
+    g[i].M = M[i]; g[i].N = N[i]; g[i].K = K[i];
+    g[i].bias = bias ? bias[i] : nullptr; g[i].pos_period = 1;
+    if (pos && pos[i]) {
+      MM_REQUIRE(pos_period && pos_period[i] > 0);
+      g[i].pos = pos[i]; g[i].pos_period = pos_period[i];
+      if (ldpos && ldpos[i]) {
+        MM_REQUIRE(ldpos[i] >= N[i]);
+        g[i].ldpos = ldpos[i];
+      }
+    }
+    g[i].drop_p = p; g[i].drop_seed = seeds[i]; g[i].drop_step = step;
+    cb[i] = 1;
+    // the mask exists only in the tensor-core epilogue: a problem it cannot take is an error
+    if (!gemm_tc_supported(g[i], 1, true)) return MMEMO_ERR_SHAPE;
+  }
+  return gemm_tc_grouped(g, cb, n, p > 0.f ? 3 : 0, mm_stream(s));
+}
 int mmemo_linear_bwd_x_grouped_bf16(int n, const void* const* dy, const int64_t* lddy,
                                     const void* const* w, const int64_t* ldw, void* const* dx,
                                     const int64_t* lddx, const void* const* relu_src,

@@ -1,6 +1,7 @@
 // Small bandwidth-bound helpers: periodic row-sum (bias / position-table gradients), dtype casts
 // (bf16 shadow weights) and counter-based dropout.
 #include "common.cuh"
+#include "dropout.cuh"
 
 namespace {
 
@@ -58,13 +59,7 @@ __global__ void cast_b2f_kernel(const bf16* __restrict__ s, float* __restrict__ 
   if (i < n) d[i] = __bfloat162float(s[i]);
 }
 
-// splitmix64-style hash of (seed, index) -> 64 well-mixed bits / a uniform in [0,1)
-__device__ __forceinline__ uint64_t hash_bits(uint64_t seed, uint64_t i) {
-  uint64_t z = seed + 0x9E3779B97F4A7C15ull * (i + 1);
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
+// a uniform in [0,1) from hash_bits (dropout.cuh)
 __device__ __forceinline__ float hash_uniform(uint64_t seed, uint64_t i) {
   return (float)(hash_bits(seed, i) >> 40) * (1.0f / 16777216.0f);
 }
@@ -122,6 +117,80 @@ dropout_multi_kernel(const __grid_constant__ DropTable t, float p, float scale,
         y[j] = from_f<T>(((uint32_t)(h >> (16 * (j & 3))) & 0xFFFFu) >= thr ? to_f(x[j]) * scale
                                                                              : 0.f);
       }
+    }
+  }
+}
+
+// Backward of the grouped projection's dropout epilogue, y_g = drop_g(x_g W_g^T + b_g) + pos_g
+// (gemm_tc.cu, family 3), for every problem of a group in ONE launch.  Problem g reads its dY
+// (M, N) once (ld = row stride: the column slices of a concatenated output are read in place),
+// regenerates the mask of the contiguous (M, N) tensor, writes m∘dY as a contiguous bf16 (M, N)
+// copy for the weight-gradient / input-gradient GEMMs and adds colsum(m∘dY) to dbias and the
+// period-row-sum of the UNMASKED dY (the table is added after the dropout) to dpos.
+// CTA = (problem, 64 columns, residue class r of the row period, strip of periods); lanes own
+// column pairs, the 8 warps split the strip's rows, partial sums meet in shared memory and reach
+// the zero-filled gradient buffer by one atomic add per column and CTA.
+constexpr int PDB_MAXP = 64;
+struct ProjDropBwdTable {
+  const bf16* dy[PDB_MAXP];
+  bf16* dym[PDB_MAXP];
+  float* dbias[PDB_MAXP];
+  float* dpos[PDB_MAXP];
+  long long lddy[PDB_MAXP], M[PDB_MAXP], ldpos[PDB_MAXP];
+  unsigned long long seed[PDB_MAXP];
+  int N[PDB_MAXP], period[PDB_MAXP], per_strip[PDB_MAXP];
+  int block_start[PDB_MAXP + 1];
+  int count;
+};
+__global__ void __launch_bounds__(256)
+proj_dropout_bwd_kernel(const __grid_constant__ ProjDropBwdTable t, uint32_t thr, float scale,
+                        const unsigned long long* __restrict__ step) {
+  __shared__ float red[8][4][33];
+  pdl_wait();
+  pdl_trigger();
+  int g = 0;
+  while (g + 1 < t.count && (int)blockIdx.x >= t.block_start[g + 1]) ++g;
+  const int lane = threadIdx.x & 31, wy = threadIdx.x >> 5;
+  const int N = t.N[g], P = t.period[g];
+  const int col_chunks = (N + 63) / 64;
+  int b = (int)blockIdx.x - t.block_start[g];
+  const int chunk = b % col_chunks;
+  b /= col_chunks;
+  const int r = b % P;                          // residue class of the row period
+  const int strip = b / P;
+  const long long M = t.M[g], lddy = t.lddy[g];
+  const int n = chunk * 64 + 2 * lane;          // lane owns columns n, n + 1 (N is even)
+  const uint64_t seed = drop_seed(t.seed[g], step);
+  const bf16* __restrict__ dy = t.dy[g];
+  bf16* __restrict__ dym = t.dym[g];
+  float db0 = 0.f, db1 = 0.f, dp0 = 0.f, dp1 = 0.f;
+  if (n < N) {
+    const long long n_per = (M - r + P - 1) / P;               // rows m = r + j*P, j < n_per
+    const long long j_end = min(n_per, (long long)(strip + 1) * t.per_strip[g]);
+    for (long long j = (long long)strip * t.per_strip[g] + wy; j < j_end; j += 8) {
+      const long long m = r + j * P;
+      const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(dy + m * lddy + n);
+      const float v0 = __low2float(v), v1 = __high2float(v);
+      const uint64_t i = (uint64_t)m * (uint64_t)N + (uint64_t)n;   // even: i, i+1 share a hash
+      const uint64_t h = hash_bits(seed, i >> 2);
+      const float m0 = drop_keep(h, i, thr) ? v0 * scale : 0.f;
+      const float m1 = drop_keep(h, i + 1, thr) ? v1 * scale : 0.f;
+      *reinterpret_cast<__nv_bfloat162*>(dym + m * N + n) = __floats2bfloat162_rn(m0, m1);
+      db0 += m0; db1 += m1;
+      dp0 += v0; dp1 += v1;
+    }
+  }
+  red[wy][0][lane] = db0; red[wy][1][lane] = db1;
+  red[wy][2][lane] = dp0; red[wy][3][lane] = dp1;
+  __syncthreads();
+  if (wy < 4) {
+    const int c = n + (wy & 1);
+    float* out = wy < 2 ? t.dbias[g] : t.dpos[g];
+    if (out && c < N) {
+      float s = 0.f;
+#pragma unroll
+      for (int w = 0; w < 8; ++w) s += red[w][wy][lane];
+      atomicAdd(wy < 2 ? out + c : out + (long long)r * t.ldpos[g] + c, s);
     }
   }
 }
@@ -507,6 +576,47 @@ int dropout_multi(int n, const void* const* x, void* const* y, const int64_t* nu
   return MMEMO_OK;
 }
 
+int proj_dropout_bwd_chunk(int n, const void* const* dy, const int64_t* lddy, void* const* dym,
+                           const int64_t* M, const int64_t* N, const uint64_t* seeds, float p,
+                           const uint64_t* step, float* const* dbias, float* const* dpos,
+                           const int64_t* period, const int64_t* ldpos, bool launch,
+                           cudaStream_t st) {
+  if (n < 1 || n > PDB_MAXP) return MMEMO_ERR_ARG;
+  MM_REQUIRE(dy && lddy && dym && M && N && seeds && p >= 0.f && p < 1.f);
+  static thread_local ProjDropBwdTable t;
+  t = ProjDropBwdTable{};
+  long long blocks = 0;
+  for (int i = 0; i < n; ++i) {
+    MM_REQUIRE(dy[i] && dym[i] && M[i] >= 0 && N[i] > 0 && N[i] % 2 == 0 && lddy[i] >= N[i]);
+    MM_REQUIRE(lddy[i] % 2 == 0 && ((reinterpret_cast<uintptr_t>(dy[i]) |
+                                     reinterpret_cast<uintptr_t>(dym[i])) & 3) == 0);
+    const float* dp = dpos ? dpos[i] : nullptr;
+    if (dp) MM_REQUIRE(period && period[i] >= 1 && period[i] <= 65535 && ldpos &&
+                       ldpos[i] >= N[i]);
+    const int P = dp ? (int)period[i] : 1;
+    const long long n_per = cdiv(M[i], (int64_t)P);
+    const int per_strip = 64;                       // rows of one residue class per CTA
+    const long long strips = n_per > 0 ? cdiv(n_per, (int64_t)per_strip) : 0;
+    t.dy[i] = static_cast<const bf16*>(dy[i]);
+    t.dym[i] = static_cast<bf16*>(dym[i]);
+    t.dbias[i] = dbias ? dbias[i] : nullptr;
+    t.dpos[i] = const_cast<float*>(dp);
+    t.lddy[i] = lddy[i]; t.M[i] = M[i]; t.ldpos[i] = dp ? ldpos[i] : 0;
+    t.seed[i] = seeds[i];
+    t.N[i] = (int)N[i]; t.period[i] = P; t.per_strip[i] = per_strip;
+    t.block_start[i] = (int)blocks;
+    blocks += cdiv(N[i], (int64_t)64) * P * strips;
+    if (blocks > (1ll << 30)) return MMEMO_ERR_SHAPE;
+  }
+  t.block_start[n] = (int)blocks;
+  t.count = n;
+  if (!launch || blocks == 0) return MMEMO_OK;
+  MM_CUDA_OK(mm_launch(proj_dropout_bwd_kernel, dim3((unsigned)blocks), dim3(256), 0, st, t,
+                       (uint32_t)(p * 65536.0f + 0.5f), 1.0f / (1.0f - p),
+                       reinterpret_cast<const unsigned long long*>(step)));
+  return MMEMO_OK;
+}
+
 int cast_multi_chunk(int count, const float* const* src, void* const* dst, const int64_t* n,
                      bool launch, cudaStream_t st) {
   if (count > CAST_MAXT) return MMEMO_ERR_ARG;
@@ -707,6 +817,22 @@ int mmemo_dropout_multi_bf16(int n, const void* const* x, void* const* y, const 
                              const uint64_t* seeds, float p, const uint64_t* step,
                              mmemo_stream_t s) {
   return dropout_multi<bf16>(n, x, y, numel, seeds, p, step, mm_stream(s));
+}
+int mmemo_proj_dropout_bwd_bf16(int n, const void* const* dy, const int64_t* lddy,
+                                void* const* dym, const int64_t* M, const int64_t* N,
+                                const uint64_t* seeds, float p, const uint64_t* step,
+                                float* const* dbias, float* const* dpos, const int64_t* period,
+                                const int64_t* ldpos, mmemo_stream_t s) {
+  if (n < 1) return MMEMO_ERR_ARG;
+  for (int pass = 0; pass < 2; ++pass)          // check every chunk, then launch them
+    for (int c = 0; c < n; c += PDB_MAXP) {
+      const int rc = proj_dropout_bwd_chunk(
+          n - c < PDB_MAXP ? n - c : PDB_MAXP, dy + c, lddy + c, dym + c, M + c, N + c, seeds + c,
+          p, step, dbias ? dbias + c : nullptr, dpos ? dpos + c : nullptr,
+          period ? period + c : nullptr, ldpos ? ldpos + c : nullptr, pass == 1, mm_stream(s));
+      if (rc) return rc;
+    }
+  return MMEMO_OK;
 }
 }
 

@@ -156,15 +156,18 @@ def _arch(m):
         return f.multimodal_blocks[0].n_heads, f.n_layers
     if isinstance(m, (Concat_Trans, Base_model)):
         return m.intensity.multimodal_blocks[0].n_heads, m.intensity.n_layers
+    if hasattr(m, "multimodal_blocks"):   # robot_demo.Multi_class (it imports this module)
+        return m.multimodal_blocks[0].n_heads, m.n_layers
     return None, None
 
 
-def _check_members(models) -> None:
+def _check_members(models, families=_FAMILIES) -> None:
+    """One class of ``families``, equal state_dict shapes and equal n_heads / n_layers."""
     if not models:
         raise ValueError("Ensemble needs at least one model")
     cls = type(models[0])
-    if cls not in _FAMILIES:
-        raise ValueError(f"Ensemble members must be one of {[c.__name__ for c in _FAMILIES]}, "
+    if cls not in families:
+        raise ValueError(f"Ensemble members must be one of {[c.__name__ for c in families]}, "
                          f"got {cls.__name__}")
     shapes0 = {k: tuple(v.shape) for k, v in models[0].state_dict().items()}
     for i, m in enumerate(models[1:], 1):

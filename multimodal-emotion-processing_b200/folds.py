@@ -3,12 +3,15 @@ for all folds' models instead of one per fold.
 
 ``forward(models, inputs)`` returns ``[models[k](*inputs[k]) for k]`` with autograd to each
 model's own parameters, for k models of ONE of ``realformer.State_Transfer``,
-``cmu_mosei.Concat_Trans``, ``ren_mme.Base_model`` or ``rencecps.Concat_Linear`` (equal
+``cmu_mosei.Concat_Trans``, ``ren_mme.Base_model``, ``rencecps.Concat_Linear`` or
+``robot_demo.Multi_class`` (equal
 state_dict shapes and ``n_heads`` / ``n_layers``, all in train or all in eval mode; ``ValueError``
 otherwise).  The folds' batch sizes may differ.  One call runs, for all folds together:
 
-- the modality projections as one grouped GEMM (bf16 mode; ``group_ops.proj_group_op``) and, for
-  ``Base_model``, the towers' shared LayerNorm as one grouped LayerNorm (``ln_group_op``);
+- the modality projections as one grouped GEMM (bf16 mode; ``group_ops.proj_group_op``, or with
+  the projections' own training dropout ``group_ops.proj_drop_group_op``, the mask drawn in the
+  GEMM epilogue; ``Multi_class``'s three visual projections write the column thirds of one stream)
+  and, for ``Base_model``, the towers' shared LayerNorm as one grouped LayerNorm (``ln_group_op``);
 - every tower of every fold through one ``fusion_trunk_multi``;
 - one grouped pooling (``mmemo_pool_fwd_multi_arg_*`` / ``mmemo_pool_bwd_multi_*``);
 - the float32 head linears as grouped SIMT GEMMs (``mmemo_linear_*_grouped_f32``), with the
@@ -21,6 +24,10 @@ backward.  A ``trainer.fit_folds`` step for Ren-MME is then::
     ls = folds.forward(ms, [b[:12] for b in bs])
     return [c + r for c, r in zip(folds.circle_losses(ls, [b[12] for b in bs]), folds.rdrop_kl(ls))]
 
+and for robot_demo's 4 folds (robot_demo.py:497-524; a batch is the 8 inputs then the labels)::
+
+    return folds.circle_losses(folds.forward(ms, [b[:8] for b in bs]), [b[8] for b in bs])
+
 Dropout.  The grouped trunk and head draw their masks from one seed per grouped call and a
 per-problem index (``ops.site_seeds``), so a fold trained in the group draws different masks from
 the ones it would draw alone.  Both are valid i.i.d. keep-(1-p) masks; with every dropout p = 0
@@ -30,8 +37,8 @@ sums the partial tiles in a fixed order), so the activation gradients the trunk 
 the same; parameter gradients summed with float atomics (head parameters, LayerNorm, scalar gates)
 agree to float rounding.
 
-Out of scope: ``robot_demo.Multi_class``, fp32 grouping of the trunk's GEMMs and attention (the
-float32 parity mode runs them per problem), and ``dp.GradReducer``.
+Out of scope: fp32 grouping of the trunk's GEMMs and attention (the float32 parity mode runs them
+per problem), and ``dp.GradReducer``.
 """
 from __future__ import annotations
 
@@ -45,11 +52,16 @@ from . import ops
 from .blocks import as_mask, fusion_trunk_multi, is_bf16
 from .cmu_mosei import Concat_Trans
 from .ensemble import _check_members
-from .group_ops import ln_bwd_group, ln_fwd_group, project
+from .group_ops import dropout_group_op, ln_bwd_group, ln_fwd_group, project, project_cat
 from .ops import BF, F32, LN_EPS, _arr, _p
 from .realformer import State_Transfer
 from .ren_mme import Base_model
 from .rencecps import Concat_Linear
+from .robot_demo import Multi_class
+
+# the families folds.forward groups (ensemble.Ensemble takes the first four; robot_demo.Ensemble
+# serves Multi_class)
+_FAMILIES = (State_Transfer, Concat_Trans, Base_model, Concat_Linear, Multi_class)
 
 
 def _call(name, *args):          # late-bound: tests stub ops._call / ops._stream
@@ -315,37 +327,6 @@ def ln_group(xs, gammas, betas, relu: bool = False) -> List[Tensor]:
 
 
 # ------------------------------------------------------------------------------------------------
-# grouped dropout with autograd (ops._dropout_group: the same seeds forward and backward)
-# ------------------------------------------------------------------------------------------------
-@torch.library.custom_op("mmemo::dropout_group", mutates_args=())
-def dropout_group_op(xs: Sequence[Tensor], p: float, seed: int) -> List[Tensor]:
-    ops._need_cuda(*xs)
-    xs = [x.contiguous() for x in xs]
-    ys = [torch.empty_like(x) for x in xs]
-    ops._dropout_group(xs, ys, p, ops.site_seeds(seed, len(xs), 0, 1))
-    return ys
-
-
-@dropout_group_op.register_fake
-def _(xs, p, seed):
-    return [torch.empty_like(x) for x in xs]
-
-
-def _dropout_group_setup(ctx, inputs, output):
-    ctx.p, ctx.seed = inputs[1], inputs[2]
-    ctx.shapes = [(x.shape, x.dtype, x.device) for x in inputs[0]]
-
-
-def _dropout_group_backward(ctx, grads):
-    dys = [g if g is not None else torch.zeros(s, dtype=dt, device=dv)
-           for g, (s, dt, dv) in zip(grads, ctx.shapes)]
-    return list(dropout_group_op(dys, ctx.p, ctx.seed)), None, None
-
-
-dropout_group_op.register_autograd(_dropout_group_backward, setup_context=_dropout_group_setup)
-
-
-# ------------------------------------------------------------------------------------------------
 # grouped heads
 # ------------------------------------------------------------------------------------------------
 @torch.library.custom_op("mmemo::bilinear_group", mutates_args=())
@@ -585,12 +566,14 @@ def forward(models: Sequence[torch.nn.Module], inputs: Sequence[Sequence]) -> Li
     models, inputs = list(models), [tuple(a) for a in inputs]
     if len(models) != len(inputs):
         raise ValueError(f"{len(models)} models but {len(inputs)} input tuples")
-    _check_members(models)
+    _check_members(models, _FAMILIES)
     if len({m.training for m in models}) > 1:
         raise ValueError("all models must be in the same train / eval mode")
     for args in inputs:
         ops._need_cuda(*[a for a in args if isinstance(a, Tensor)])
     m0 = models[0]
+    if isinstance(m0, Multi_class):
+        return _multi_class(models, inputs)
     if isinstance(m0, State_Transfer):
         return _state_transfer(models, inputs)
     if isinstance(m0, Concat_Linear):
@@ -602,9 +585,12 @@ def _unify(u, x3, poss=(None, None, None)):
     return [(x, c.weight, p) for x, c, p in zip(x3, (u.linguistic, u.visual, u.acoustic), poss)]
 
 
-def _project(probs):
+def _project(probs, drop_p=0.0):
+    """``drop_p`` > 0: the projections' own dropout (between the GEMM and the position add) in
+    the grouped GEMM's epilogue, one seed per call."""
     return project([x for x, _, _ in probs], [w for _, w, _ in probs], None,
-                   [p for _, _, p in probs], bf16=is_bf16())
+                   [p for _, _, p in probs], bf16=is_bf16(), drop_p=drop_p,
+                   seed=ops.next_dropout_seed() if drop_p > 0 else 0)
 
 
 def _heads(models, pooled_last, pooled_this, w_last, w_this, norms):
@@ -658,9 +644,7 @@ def _concat_linear(models, inputs):
 def _state_transfer(models, inputs):
     """others/realformer.py:266-286 for every fold: the B*P windows folded into the batch."""
     fs = [m.feature for m in models]
-    shapes, projected, masks = [], [], []
-    per_op = any(f.training and f.unify_dimension.drop.p > 0 for f in fs)
-    probs = []
+    shapes, masks, probs = [], [], []
     for f, args in zip(fs, inputs):
         l, v, a, lm, vm, am = args
         B, P = l.shape[0], l.shape[1]
@@ -668,11 +652,8 @@ def _state_transfer(models, inputs):
         fold = lambda t, B=B, P=P: t.reshape(B * P, *t.shape[2:])
         l, v, a = fold(l), fold(v), fold(a)
         masks.append({"l": as_mask(fold(lm)), "v": as_mask(fold(vm)), "a": as_mask(fold(am))})
-        if per_op:      # the projection's own dropout sits between the GEMM and the position add
-            projected += list(f.unify_dimension(l, v, a, f.positions(l, v, a)))
-        else:
-            probs += _unify(f.unify_dimension, (l, v, a), f.positions(l, v, a))
-    ys = projected if per_op else _project(probs)
+        probs += _unify(f.unify_dimension, (l, v, a), f.positions(l, v, a))
+    ys = _project(probs, float(fs[0].unify_dimension.drop.p) if fs[0].training else 0.0)
     trunk = [(f.multimodal_blocks, {"l": ys[3 * i], "v": ys[3 * i + 1], "a": ys[3 * i + 2]},
               masks[i]) for i, f in enumerate(fs)]
     pooled = pool_group(fusion_trunk_multi(trunk, fs[0].n_layers, keep_all=False, pool=False))
@@ -686,3 +667,34 @@ def _state_transfer(models, inputs):
     o = linear_group(h, [m.classifier.weight for m in models], [m.classifier.bias for m in models])
     return list(state_transfer_group_op([x.view(B, P, -1) for x, (B, P) in zip(o, shapes)],
                                         [m.trans for m in models]))
+
+
+def _multi_class(models, inputs):
+    """robot_demo.py:377-441 for every fold: five biased projections per fold (the three visual
+    ones write the column thirds of one (B, L, d) stream) with their dropout and position tables
+    as ONE grouped projection, every fold's trunk as one tower of ``fusion_trunk_multi``, one
+    grouped pooling and one grouped classifier linear."""
+    xs, ws, bs, poss, spans, masks = [], [], [], [], [], []
+    for m, args in zip(models, inputs):
+        if len(args) != 8:
+            raise ValueError(f"Multi_class takes 8 inputs per fold, got {len(args)}")
+        l, v_256, v_512, v_1024, a, l_mask, v_mask, a_mask = args
+        u = m.unify_dimension
+        for x, c in zip((l, v_256, v_512, v_1024, a),
+                        (u.linguistic, u.visual_256, u.visual_512, u.visual_1024, u.acoustic)):
+            xs.append(x)
+            ws.append(c.weight)
+            bs.append(c.bias)
+        spans += [1, 3, 1]
+        poss += [e.position_embeddings.weight for e in
+                 (m.linguistic_position, m.visual_position, m.acoustic_position)]
+        masks.append({"l": as_mask(l_mask), "v": as_mask(v_mask), "a": as_mask(a_mask)})
+    m0 = models[0]
+    p = float(m0.unify_dimension.drop.p) if m0.training else 0.0
+    ys = project_cat(xs, ws, bs, spans, poss, is_bf16(), p,
+                     ops.next_dropout_seed() if p > 0 else 0)
+    trunk = [(m.multimodal_blocks, {"l": ys[3 * i], "v": ys[3 * i + 1], "a": ys[3 * i + 2]},
+              masks[i]) for i, m in enumerate(models)]
+    pooled = pool_group(fusion_trunk_multi(trunk, m0.n_layers, keep_all=True, pool=False))
+    return linear_group(pooled, [m.classifier.weight for m in models],
+                        [m.classifier.bias for m in models])

@@ -744,6 +744,22 @@ def _padded_shadow(w: Tensor, todo: list) -> Tensor:
     return out
 
 
+def _cast_problems(xs, ws):
+    """The padded bf16 copies of every input and (cached) weight of a grouped projection, one cast
+    launch per 16 tensors; returns ([xb_g (M_g, Kp_g)], [wp_g (N_g, Kp_g)])."""
+    todo, xbs = [], []
+    for x in xs:
+        K = x.shape[-1]
+        x2 = x.reshape(-1, K)
+        x2 = x2 if x2.stride(1) == 1 else x2.contiguous()
+        xb = torch.empty(x2.shape[0], _pad8(K), dtype=BF, device=x.device)
+        todo.append((x2, xb))
+        xbs.append(xb)
+    wps = [_padded_shadow(w, todo) for w in ws]
+    _cast_pad(todo)
+    return xbs, wps
+
+
 @torch.library.custom_op("mmemo::proj_group", mutates_args=())
 def proj_group_op(xs: Sequence[Tensor], ws: Sequence[Tensor], biases: Sequence[Tensor],
                   poss: Sequence[Tensor]) -> List[Tensor]:
@@ -751,18 +767,8 @@ def proj_group_op(xs: Sequence[Tensor], ws: Sequence[Tensor], biases: Sequence[T
     weight gradient).  biases / poss entries with numel() == 0 mean "none"."""
     ops._need_cuda(*xs)
     G = len(xs)
-    todo, xbs, wps, ys, items = [], [], [], [], []
-    for g in range(G):
-        x = xs[g]
-        K = x.shape[-1]
-        x2 = x.reshape(-1, K)
-        x2 = x2 if x2.stride(1) == 1 else x2.contiguous()
-        xb = torch.empty(x2.shape[0], _pad8(K), dtype=BF, device=x.device)
-        todo.append((x2, xb))
-        xbs.append(xb)
-    for g in range(G):
-        wps.append(_padded_shadow(ws[g], todo))
-    _cast_pad(todo)
+    xbs, wps = _cast_problems(xs, ws)
+    ys, items = [], []
     for g in range(G):
         N = wps[g].shape[0]
         pos = _opt(poss[g])
@@ -776,15 +782,20 @@ def proj_group_op(xs: Sequence[Tensor], ws: Sequence[Tensor], biases: Sequence[T
     return ys + xbs
 
 
-def _proj_zlayout(Ns, Kps, has_bias, pos_lens):
-    """Offsets (floats, 256-byte aligned) of [dW_g (N, Kp) | dbias_g (N) | dpos_g (L, N)] per
-    problem inside the one zero-filled gradient buffer, and its total length."""
+def _zlayout(sizes):
+    """Offsets (floats, 256-byte aligned) of regions of the given sizes inside one zero-filled
+    gradient buffer, and its total length."""
     offs, tot = [], 0
-    for g in range(len(Ns)):
-        for n in (Ns[g] * Kps[g], Ns[g] if has_bias[g] else 0, pos_lens[g] * Ns[g]):
-            offs.append(tot)
-            tot += (n + 63) // 64 * 64
+    for n in sizes:
+        offs.append(tot)
+        tot += (n + 63) // 64 * 64
     return offs, tot
+
+
+def _proj_zlayout(Ns, Kps, has_bias, pos_lens):
+    """[dW_g (N, Kp) | dbias_g (N) | dpos_g (L, N)] per problem (``_zlayout``)."""
+    return _zlayout([n for g in range(len(Ns)) for n in
+                     (Ns[g] * Kps[g], Ns[g] if has_bias[g] else 0, pos_lens[g] * Ns[g])])
 
 
 @torch.library.custom_op("mmemo::proj_group_bwd", mutates_args=())
@@ -907,16 +918,260 @@ def project_into(xs, ws, biases, outs, poss=None) -> None:
     ops._linear_fwd_group(True, items)
 
 
-def project(xs, ws, biases=None, poss=None, bf16: bool = False) -> List[Tensor]:
-    """Modality projections of one or several towers.  bf16 mode with float32 inputs: the grouped
-    cast + tensor-core path above; otherwise the per-problem ``ops.linear`` (float32 parity mode,
-    or inputs that are already bf16)."""
+# ------------------------------------------------------------------------------------------------
+# mmemo::proj_drop_group — the training form of the modality projections (robot_demo.py:302-311
+#   then :392-394; others/realformer.py:133-143 without bias):
+#     out_s = cat_{g in span s}( drop_g(x_g W_g^T + b_g) ) + pos_s
+#   with the dropout in the tcgen05 epilogue (mmemo_linear_fwd_grouped_dropout_bf16) and the
+#   problems of a span writing column blocks of ONE output (the reference's visual concat) - no
+#   mask tensor, no concat copy, no position-add kernels.  The masks are those ops._dropout_group
+#   draws for the contiguous (M_g, N_g) projections with seeds ops.site_seeds(seed, G, 0, 1).
+#   Backward: ONE mmemo_proj_dropout_bwd_bf16 launch (masked dY copies, bias and position-table
+#   gradients) and one grouped weight-gradient GEMM.
+# ------------------------------------------------------------------------------------------------
+def _span_starts(spans):
+    starts, g = [], 0
+    for n in spans:
+        starts.append(g)
+        g += n
+    return starts
+
+
+def _drop_seeds(seed: int, G: int):
+    return ops.site_seeds(seed, G, 0, 1)
+
+
+@torch.library.custom_op("mmemo::proj_drop_group", mutates_args=())
+def proj_drop_group_op(xs: Sequence[Tensor], ws: Sequence[Tensor], biases: Sequence[Tensor],
+                       poss: Sequence[Tensor], spans: Sequence[int], drop_p: float,
+                       seed: int) -> List[Tensor]:
+    """Returns [out_0 .. out_{S-1}, xb_0 .. xb_{G-1}]; biases (per problem) and poss (per span,
+    (L, width of the span)) entries with numel() == 0 mean none."""
+    ops._need_cuda(*xs)
+    G = len(xs)
+    dev = xs[0].device
+    xbs, wps = _cast_problems(xs, ws)
+    outs, items = [], []
+    for s, (g0, n) in enumerate(zip(_span_starts(spans), spans)):
+        lead = tuple(xs[g0].shape[:-1])
+        width = sum(wps[g].shape[0] for g in range(g0, g0 + n))
+        y = torch.empty(*lead, width, dtype=BF, device=dev)
+        y2 = y.view(-1, width)
+        pos = _opt(poss[s])
+        if pos is not None:
+            assert xs[g0].dim() == 3 and tuple(pos.shape) == (lead[1], width), \
+                "position table must be (seq length, output width)"
+        c = 0
+        for g in range(g0, g0 + n):
+            assert tuple(xs[g].shape[:-1]) == lead, "problems of one span need equal leading shapes"
+            N = wps[g].shape[0]
+            items.append((xbs[g], wps[g], _opt(biases[g]), y2[:, c:c + N],
+                          None if pos is None else pos[:, c:c + N]))
+            c += N
+        outs.append(y)
+    seeds = _drop_seeds(seed, G)
+    step = ops.dropout_step(dev)
+    for i in range(0, G, ops.MAX_GEMM_GROUP):
+        part = items[i:i + ops.MAX_GEMM_GROUP]
+        _call("mmemo_linear_fwd_grouped_dropout_bf16", len(part),
+              _vpa([it[0] for it in part]), _i64s(it[0].stride(0) for it in part),
+              _vpa([it[1] for it in part]), _i64s(it[1].stride(0) for it in part),
+              _vpa([it[2] for it in part]), _vpa([it[3] for it in part]),
+              _i64s(it[3].stride(0) for it in part), _i64s(it[0].shape[0] for it in part),
+              _i64s(it[1].shape[0] for it in part), _i64s(it[1].shape[1] for it in part),
+              _vpa([it[4] for it in part]),
+              _i64s(0 if it[4] is None else it[4].shape[0] for it in part),
+              _i64s(0 if it[4] is None else it[4].stride(0) for it in part),
+              _arr(C.c_uint64, seeds[i:i + ops.MAX_GEMM_GROUP]), float(drop_p), step.data_ptr(),
+              _stream())
+    return outs + xbs
+
+
+def _i64s(vals):
+    return _arr(C.c_int64, [int(v) for v in vals])
+
+
+@proj_drop_group_op.register_fake
+def _(xs, ws, biases, poss, spans, drop_p, seed):
+    outs = []
+    for g0, n in zip(_span_starts(spans), spans):
+        width = sum(_w2d(ws[g]).shape[0] for g in range(g0, g0 + n))
+        outs.append(xs[g0].new_empty(*xs[g0].shape[:-1], width, dtype=BF))
+    return outs + [x.new_empty(x.numel() // x.shape[-1], _pad8(x.shape[-1]), dtype=BF) for x in xs]
+
+
+@torch.library.custom_op("mmemo::proj_drop_group_bwd", mutates_args=())
+def proj_drop_group_bwd_op(dys: Sequence[Tensor], xbs: Sequence[Tensor], ws: Sequence[Tensor],
+                           has_bias: Sequence[bool], pos_lens: Sequence[int],
+                           spans: Sequence[int], drop_p: float, seed: int,
+                           need_dx: Sequence[bool]) -> List[Tensor]:
+    """Returns [z] + [dx_g (float32 (M, K)) or empty]: z = ONE zero-initialised float32 buffer with
+    every parameter gradient of the group (``_drop_zlayout``)."""
+    G = len(xbs)
+    dev = dys[0].device
+    Ns = [_w2d(w).shape[0] for w in ws]
+    Ks = [_w2d(w).shape[1] for w in ws]
+    Kps = [_pad8(k) for k in Ks]
+    offs, tot = _drop_zlayout(Ns, Kps, has_bias, pos_lens, spans)
+    z = torch.zeros(tot, dtype=F32, device=dev)
+    dy_s, ld_s, dpos_s, ldpos_s, per_s = [], [], [], [], []
+    for s, (g0, n) in enumerate(zip(_span_starts(spans), spans)):
+        width = sum(Ns[g0:g0 + n])
+        dy2 = dys[s].contiguous().view(-1, width)
+        c = 0
+        for g in range(g0, g0 + n):
+            dy_s.append(dy2[:, c:c + Ns[g]])
+            dpos_s.append(z[offs[2 * G + s] + c:] if pos_lens[s] else None)
+            ldpos_s.append(width)
+            per_s.append(pos_lens[s])
+            c += Ns[g]
+    dyms = [torch.empty(d.shape, dtype=BF, device=dev) for d in dy_s]
+    _call("mmemo_proj_dropout_bwd_bf16", G, _vpa(dy_s), _i64s(d.stride(0) for d in dy_s),
+          _vpa(dyms), _i64s(d.shape[0] for d in dy_s), _i64s(Ns),
+          _arr(C.c_uint64, _drop_seeds(seed, G)), float(drop_p), ops.dropout_step(dev).data_ptr(),
+          _vpa([z[offs[2 * g + 1]:] if has_bias[g] else None for g in range(G)]), _vpa(dpos_s),
+          _i64s(per_s), _i64s(ldpos_s), _stream())
+    dwp = [z[offs[2 * g]:offs[2 * g] + Ns[g] * Kps[g]].view(Ns[g], Kps[g]) for g in range(G)]
+    ops._linear_bwd_w_group(True, [(dyms[g], xbs[g], dwp[g]) for g in range(G)], zeroed=True)
+    dxs = []
+    for g in range(G):
+        if need_dx[g]:
+            todo: list = []
+            wp = _padded_shadow(ws[g], todo)
+            _cast_pad(todo)
+            dxb = torch.empty(dyms[g].shape[0], Kps[g], dtype=BF, device=dev)
+            ops._linear_bwd_x(True, dyms[g], wp, dxb)
+            dxs.append(dxb[:, :Ks[g]].float())
+        else:
+            dxs.append(_e(dev))
+    return [z] + dxs
+
+
+def _drop_zlayout(Ns, Kps, has_bias, pos_lens, spans):
+    """[dW_g (N, Kp) | dbias_g (N)] per problem, then dpos_s (L, width of the span) per span."""
+    widths = [sum(Ns[g0:g0 + n]) for g0, n in zip(_span_starts(spans), spans)]
+    return _zlayout([n for g in range(len(Ns)) for n in
+                     (Ns[g] * Kps[g], Ns[g] if has_bias[g] else 0)] +
+                    [L * w for L, w in zip(pos_lens, widths)])
+
+
+def _proj_drop_setup(ctx, inputs, output):
+    xs, ws, biases, poss, spans, drop_p, seed = inputs
+    G = len(xs)
+    ctx.G, ctx.spans, ctx.drop = G, list(spans), (drop_p, seed)
+    ctx.has_bias = [b.numel() > 0 for b in biases]
+    ctx.pos_lens = [p.shape[0] if p.numel() else 0 for p in poss]
+    ctx.x_shapes = [tuple(x.shape) for x in xs]
+    ctx.out_shapes = [tuple(y.shape) for y in output[:len(spans)]]
+    ctx.save_for_backward(*output[len(spans):], *ws)
+    ctx.set_materialize_grads(False)
+
+
+def _proj_drop_backward(ctx, grads):
+    G, spans = ctx.G, ctx.spans
+    S = len(spans)
+    t = list(ctx.saved_tensors)
+    xbs, ws = t[:G], t[G:]
+    dev = xbs[0].device
+    need_dx = list(ctx.needs_input_grad[0])
+    Ns = [_w2d(w).shape[0] for w in ws]
+    Ks = [_w2d(w).shape[1] for w in ws]
+    Kps = [_pad8(k) for k in Ks]
+    dys = [g if g is not None else torch.zeros(sh, dtype=BF, device=dev)
+           for g, sh in zip(grads[:S], ctx.out_shapes)]
+    res = proj_drop_group_bwd_op(dys, xbs, ws, ctx.has_bias, ctx.pos_lens, spans, *ctx.drop,
+                                 need_dx)
+    z, dxs = res[0], res[1:]
+    offs, _ = _drop_zlayout(Ns, Kps, ctx.has_bias, ctx.pos_lens, spans)
+    dws, dbs, dps = [], [], []
+    for g in range(G):
+        dw = z[offs[2 * g]:offs[2 * g] + Ns[g] * Kps[g]].view(Ns[g], Kps[g])
+        if Kps[g] != Ks[g]:
+            dw = dw[:, :Ks[g]].contiguous()
+        dws.append(dw.view(ws[g].shape))
+        dbs.append(z[offs[2 * g + 1]:offs[2 * g + 1] + Ns[g]] if ctx.has_bias[g] else None)
+    for s, (g0, n) in enumerate(zip(_span_starts(spans), spans)):
+        L, w = ctx.pos_lens[s], sum(Ns[g0:g0 + n])
+        dps.append(z[offs[2 * G + s]:offs[2 * G + s] + L * w].view(L, w) if L else None)
+    return ([dxs[g].view(ctx.x_shapes[g]) if need_dx[g] else None for g in range(G)], dws, dbs,
+            dps, None, None, None)
+
+
+proj_drop_group_op.register_autograd(_proj_drop_backward, setup_context=_proj_drop_setup)
+
+
+# ------------------------------------------------------------------------------------------------
+# grouped dropout with autograd (ops._dropout_group: the same seeds forward and backward)
+# ------------------------------------------------------------------------------------------------
+@torch.library.custom_op("mmemo::dropout_group", mutates_args=())
+def dropout_group_op(xs: Sequence[Tensor], p: float, seed: int) -> List[Tensor]:
+    ops._need_cuda(*xs)
+    xs = [x.contiguous() for x in xs]
+    ys = [torch.empty_like(x) for x in xs]
+    ops._dropout_group(xs, ys, p, ops.site_seeds(seed, len(xs), 0, 1))
+    return ys
+
+
+@dropout_group_op.register_fake
+def _(xs, p, seed):
+    return [torch.empty_like(x) for x in xs]
+
+
+def _dropout_group_setup(ctx, inputs, output):
+    ctx.p, ctx.seed = inputs[1], inputs[2]
+    ctx.shapes = [(x.shape, x.dtype, x.device) for x in inputs[0]]
+
+
+def _dropout_group_backward(ctx, grads):
+    dys = [g if g is not None else torch.zeros(s, dtype=dt, device=dv)
+           for g, (s, dt, dv) in zip(grads, ctx.shapes)]
+    return list(dropout_group_op(dys, ctx.p, ctx.seed)), None, None
+
+
+dropout_group_op.register_autograd(_dropout_group_backward, setup_context=_dropout_group_setup)
+
+
+def project(xs, ws, biases=None, poss=None, bf16: bool = False, drop_p: float = 0.0,
+            seed: int = 0) -> List[Tensor]:
+    """Modality projections of one or several towers, y_g = drop(x_g w_g^T + b_g) + pos_g.  bf16
+    mode with float32 inputs: the grouped cast + tensor-core path above (``proj_group_op``, or with
+    ``drop_p`` > 0 ``proj_drop_group_op``); otherwise the per-problem ``ops.linear`` (float32
+    parity mode, or inputs that are already bf16), with the same masks (``project_cat``)."""
     G = len(xs)
     biases = biases if biases is not None else [None] * G
     poss = poss if poss is not None else [None] * G
+    if drop_p > 0:
+        return project_cat(xs, ws, biases, [1] * G, poss, bf16, drop_p, seed)
     if bf16 and all(x.dtype == F32 for x in xs):
         dev = xs[0].device
         ys = proj_group_op(list(xs), list(ws), [b if b is not None else _e(dev) for b in biases],
                            [p if p is not None else _e(dev) for p in poss])
         return list(ys[:G])
     return [ops.linear(x, w, b, p, bf16=bf16) for x, w, b, p in zip(xs, ws, biases, poss)]
+
+
+def project_cat(xs, ws, biases, spans, poss, bf16: bool = False, drop_p: float = 0.0,
+                seed: int = 0) -> List[Tensor]:
+    """One output per span of consecutive problems: ``cat_g(drop_g(x_g w_g^T + b_g)) + pos_s``
+    along the last dim (robot_demo.py:302-311 + :392-394: the three visual projections are one
+    span of the (B, L, d) visual stream), with autograd to inputs, weights, biases and tables.
+    bf16 mode with float32 inputs: ``proj_drop_group_op``.  Otherwise per-problem ``ops.linear``,
+    ONE ``dropout_group_op`` with the same site seeds (so both modes draw the same masks), then the
+    concat and the position add."""
+    G = len(xs)
+    assert sum(spans) == G and len(poss) == len(spans)
+    dev = xs[0].device
+    if bf16 and all(x.dtype == F32 for x in xs):
+        ys = proj_drop_group_op(list(xs), list(ws),
+                                [b if b is not None else _e(dev) for b in biases],
+                                [p if p is not None else _e(dev) for p in poss], list(spans),
+                                float(drop_p), int(seed))
+        return list(ys[:len(spans)])
+    ys = [ops.linear(x, w, b, bf16=bf16) for x, w, b in zip(xs, ws, biases)]
+    if drop_p > 0:
+        ys = list(dropout_group_op(ys, float(drop_p), int(seed)))
+    outs = []
+    for g0, n, pos in zip(_span_starts(spans), spans, poss):
+        y = ys[g0] if n == 1 else torch.cat(ys[g0:g0 + n], -1)
+        outs.append(y if pos is None else y + pos.to(y.dtype))
+    return outs

@@ -27,19 +27,13 @@ class Unify_Dimension_Conv1d(nn.Module):
         self.drop = nn.Dropout(DROP)
 
     def forward(self, l, v, a, pos=(None, None, None)):
-        bf = is_bf16()
+        from .group_ops import project
         convs = (self.linguistic, self.visual, self.acoustic)
-        if not (self.training and self.drop.p > 0):
-            # all three projections (+ fused position tables) as one group (group_ops.project)
-            from .group_ops import project
-            return tuple(project([l, v, a], [c.weight for c in convs], None, list(pos), bf16=bf))
-        out = []
-        for x, conv, p in zip((l, v, a), convs, pos):
-            y = ops.dropout(ops.linear(x, conv.weight, bf16=bf), self.drop.p, True)
-            if p is not None:           # reference order: drop(conv(x)) THEN + position
-                y = y + as_act(p)[None, : y.shape[1]]
-            out.append(y)
-        return tuple(out)
+        p = float(self.drop.p) if self.training else 0.0
+        # all three projections (+ fused position tables) as one group (group_ops.project); the
+        # reference order drop(conv(x)) THEN + position is kept in the GEMM epilogue
+        return tuple(project([l, v, a], [c.weight for c in convs], None, list(pos), bf16=is_bf16(),
+                             drop_p=p, seed=ops.next_dropout_seed() if p > 0 else 0))
 
 
 class Position_Embedding(nn.Module):

@@ -25,17 +25,13 @@ class Unify_Dimension_Conv1d(nn.Module):
         self.drop = nn.Dropout(DROP)
 
     def forward(self, l, v_256, v_512, v_1024, a):
-        bf = is_bf16()
+        from .group_ops import project
         convs = (self.linguistic, self.visual_256, self.visual_512, self.visual_1024, self.acoustic)
-        xs = (l, v_256, v_512, v_1024, a)
-        if not (self.training and self.drop.p > 0):
-            from .group_ops import project
-            yl, y256, y512, y1024, ya = project(list(xs), [c.weight for c in convs],
-                                                [c.bias for c in convs], bf16=bf)
-        else:
-            yl, y256, y512, y1024, ya = (
-                ops.dropout(ops.linear(x, c.weight, c.bias, bf16=bf), self.drop.p, True)
-                for x, c in zip(xs, convs))
+        p = float(self.drop.p) if self.training else 0.0
+        # all five projections, with their training dropout, as one group (group_ops.project)
+        yl, y256, y512, y1024, ya = project([l, v_256, v_512, v_1024, a], [c.weight for c in convs],
+                                            [c.bias for c in convs], bf16=is_bf16(), drop_p=p,
+                                            seed=ops.next_dropout_seed() if p > 0 else 0)
         return yl, torch.cat((y256, y512, y1024), 2), ya
 
 
